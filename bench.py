@@ -1,6 +1,6 @@
 """bench.py - CURIOUS training hot path on B200 (contract: see the repository prompt / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 metric   HER-relabelled transitions/s (BASELINE.json), Arm4-shaped synthetic replay:
          4 module buffers x 1e6 transitions (20 000 episodes x T=50, dimo=40, dimg=dimag=12, dimu=4, N=4).
@@ -17,6 +17,9 @@ Also on the line: update_us / updates_per_s (device-timed train()), get_actions 
 out), a rollout-inclusive cycle (50 x get_actions + store + 100 x train), the 19-worker-equivalent update, all of it
 again on the Arm8 shape (BASELINE config 4), and - several ranks - the bit-exact parity of the in-launch gradient
 exchange against an all-gather + rank-ordered sum (`exchange_parity`) and the per-rank scaling of the update.
+--dump-outputs DIR   after the timed steps, rank 0 writes the staged batch of the last step (o, g, u, td, o_2, r) as
+         DIR/<name>.npy, float32, the same seeded sample of DUMP_ROWS rows from every array (53 MB in all).  The inputs
+         are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -42,6 +45,9 @@ CP8 = [0.05, 0.2, 0.1, 0.0, 0.0, 0.0, 0.0, 0.0]
 EPS_TASK = 0.4
 N_BATCHES = 100                # config.py:72 - the SAME cycle in both arms: store_episode + N_BATCHES x train + polyak
 ROLLOUT_STEPS = T              # get_actions calls per rollout (rollout.py:217,226: one per env step)
+HER_OUTPUTS = ('o', 'g', 'u', 'td', 'o_2', 'r')   # the staged training batch one HER step produces
+DUMP_ROWS = 1 << 17            # --dump-outputs: rows sampled from the ROWS_PER_STEP of a step (x 101 floats x 4 B = 53 MB)
+DUMP_SEED = 0
 
 
 def workload_config():
@@ -345,7 +351,7 @@ def her_line(sampler, buffers, dims, n_modules, cp, torch, label):
     """One fused HER launch over ROWS_PER_STEP rows on this shape: transitions/s and fraction of the HBM roofline."""
     segs = her_step_segments(buffers, ROWS_PER_STEP, cp)
     out = {}
-    want = ('o', 'g', 'u', 'td', 'o_2', 'r')
+    want = HER_OUTPUTS
     ms = time_updates(lambda: sampler.sample_device(segs, ROWS_PER_STEP, clip_obs=200.0, want=want, out=out), 20, torch)
     bpt = algorithmic_bytes_per_transition(dims, n_modules)
     peak, _ = measured_peak_hbm()
@@ -354,6 +360,21 @@ def her_line(sampler, buffers, dims, n_modules, cp, torch, label):
     torch.cuda.empty_cache()
     return {'transitions_per_s': ROWS_PER_STEP / (ms * 1e-3), 'ms_per_launch': ms, 'algorithmic_bytes_per_transition': bpt,
             'achieved_gbs': achieved, 'frac_of_hbm_peak': achieved / peak, 'workload': label}
+
+
+def dump_outputs(out, directory):
+    """The arrays one HER step hands its caller (sample_device's dict of [ROWS_PER_STEP, dim] float32 device tensors),
+    as directory/<name>.npy: the rows of a fixed seeded sample, the same rows in every array."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    rows = np.sort(np.random.RandomState(DUMP_SEED).choice(ROWS_PER_STEP, DUMP_ROWS, replace=False))
+    sel = None
+    for name, t in out.items():
+        if name.startswith('_'):                          # references the launch keeps alive, not outputs
+            continue
+        if sel is None:
+            sel = torch.from_numpy(rows).to(t.device)
+        np.save(os.path.join(directory, name + '.npy'), t.index_select(0, sel).cpu().numpy().astype(np.float32))
 
 
 def build_cpu_workload(seed, episodes_per_buffer):
@@ -731,7 +752,7 @@ def run_ours(args):
     _lib.load()
     agent, sampler, buffers, dims, ag_ids, g_ids = build_gpu_workload(device, seed=1 + rank)
     segs = her_step_segments(buffers, ROWS_PER_STEP, CP)
-    want = ('o', 'g', 'u', 'td', 'o_2', 'r')
+    want = HER_OUTPUTS
     out = {}
 
     def her_step():
@@ -755,6 +776,8 @@ def run_ours(args):
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
     del out
     arm4 = measure_agent(agent, dims, N_MODULES, world, rank, barrier, torch, dist, device)
     clock_info = clocks.stop()
@@ -849,7 +872,13 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-sweep', action='store_true', help='skip the batch sweep / task_experts section')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write a seeded sample of the last timed step\'s outputs as DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     if args.impl == 'reference':
         run_reference_arm(args)
     else:

@@ -1,4 +1,5 @@
-"""The bench JSON line contract, checked on the committed records of the round (profiles/r01_bench_*.json) - CPU only."""
+"""The bench JSON line contract, checked on the committed records of the round (profiles/r01_bench_*.json), and the
+outputs bench.py --dump-outputs writes (on the host, and one run of the benchmark on the GPU)."""
 import glob
 import json
 import os
@@ -39,6 +40,66 @@ def test_committed_bench_record_keeps_the_contract(path):
         b = d['cpu_baseline']
         assert b['kind'] == 'port' and b['cores'] >= 1 and b['unit'] == d['unit'] and b['sample']
     assert isinstance(base, dict)
+
+
+def test_dump_outputs_writes_the_same_seeded_sample_of_every_output(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 DIR/<name>.npy per output of the HER step, the same rows of each (checked with small
+    host tensors standing in for the device ones), and the full-size dump stays under 64 MB."""
+    import numpy as np
+    import torch
+    import bench
+    arm, _, _ = bench.synth_dims()
+    cols = dict(arm, td=arm['task_descr'], o_2=arm['o'], r=1)           # sample_device's width of each output
+    dims = {k: cols[k] for k in bench.HER_OUTPUTS}
+    assert bench.DUMP_ROWS * sum(dims.values()) * 4 <= 64 << 20
+    monkeypatch.setattr(bench, 'ROWS_PER_STEP', 1000)
+    monkeypatch.setattr(bench, 'DUMP_ROWS', 100)
+    rows = torch.arange(1000, dtype=torch.float32)[:, None]
+    out = {k: rows * 100 + torch.arange(d, dtype=torch.float32) for k, d in dims.items()}
+    out['_keep'] = []
+    for d in ('a', 'b'):
+        bench.dump_outputs(out, str(tmp_path / d))
+    assert sorted(os.listdir(str(tmp_path / 'a'))) == sorted(k + '.npy' for k in dims)
+    picked = None
+    for k, d in dims.items():
+        x = np.load(str(tmp_path / 'a' / (k + '.npy')))
+        assert x.dtype == np.float32 and x.shape == (100, d)
+        assert np.array_equal(x, np.load(str(tmp_path / 'b' / (k + '.npy'))))
+        r = x[:, 0] / 100
+        assert picked is None or np.array_equal(r, picked)
+        picked = r
+    assert len(np.unique(picked)) == 100
+
+
+@pytest.mark.gpu
+def test_bench_dump_is_the_same_in_two_runs(tmp_path):
+    """Two runs of bench.py with the same arguments dump the same device outputs of their last timed step."""
+    import subprocess
+    import sys
+    import numpy as np
+    import bench
+    for d in ('a', 'b'):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--gpus', '1', '--steps', '1', '--warmup', '0',
+                            '--no-sweep', '--no-cpu-baseline', '--dump-outputs', str(tmp_path / d)],
+                           capture_output=True, timeout=1200)
+        assert p.returncode == 0, p.stderr.decode()[-2000:]
+    assert sorted(os.listdir(str(tmp_path / 'a'))) == sorted(k + '.npy' for k in bench.HER_OUTPUTS)
+    total = 0
+    for k in bench.HER_OUTPUTS:
+        x = np.load(str(tmp_path / 'a' / (k + '.npy')))
+        assert x.dtype == np.float32 and x.shape[0] == bench.DUMP_ROWS and np.isfinite(x).all(), k
+        assert np.array_equal(x, np.load(str(tmp_path / 'b' / (k + '.npy')))), k
+        total += x.nbytes
+    assert total <= 64 << 20
+    assert set(np.unique(np.load(str(tmp_path / 'a' / 'r.npy')))) <= {-1.0, 0.0}
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'td.npy')).sum(1), np.ones(bench.DUMP_ROWS, np.float32))
+
+
+def test_bench_rejects_a_run_without_timed_steps():
+    import subprocess
+    import sys
+    p = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '0'], capture_output=True)
+    assert p.returncode == 2 and b'--steps' in p.stderr
 
 
 def test_reference_arm_record_keeps_the_contract():

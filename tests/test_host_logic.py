@@ -256,12 +256,29 @@ def test_bench_roofline_arithmetic_matches_the_survey():
     assert set(line) >= {'sm_mhz', 'sm_max_mhz', 'reasons', 'samples', 'source'}
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/baselines/her'), reason='needs the reference checkout (build container)')
 def test_product_slot_policy_equals_the_live_reference():
     """ReplayBuffer._get_storage_idx of the drop-in (host logic, consumes the caller's np.random) against the unmodified
-    reference method on random sequences - no device needed: the object is built without its CUDA storage."""
+    reference method on random sequences - no device needed: the object is built without its CUDA storage.  Without a
+    reference checkout, against the slot sequences recorded from that method (tests/golden/storage_*.npz)."""
     import importlib.util
+    import json
     from curious_b200.replay_buffer import ReplayBuffer
+    from tests.ddpg_util import REFERENCE_ROOT
+    if not os.path.isdir(os.path.join(REFERENCE_ROOT, 'baselines', 'her')):
+        state = np.random.get_state()
+        try:
+            for name in ('storage_single', 'storage_batched'):
+                z = np.load(os.path.join(ROOT, 'tests', 'golden', name + '.npz'))
+                meta = json.loads(str(z['meta']))
+                mine = ReplayBuffer.__new__(ReplayBuffer)
+                mine.size, mine.T, mine.current_size, mine.n_transitions_stored = meta['size_ep'], meta['T'], 0, 0
+                np.random.seed(meta['seed'])
+                for k, inc in enumerate(meta['increments']):
+                    assert np.array_equal(np.atleast_1d(mine._get_storage_idx(inc)), z['idx_%d' % k]), (name, k)
+                    assert mine.current_size == z['sizes'][k], (name, k)
+        finally:
+            np.random.set_state(state)
+        return
     spec = importlib.util.spec_from_file_location('gen_golden', os.path.join(ROOT, 'oracle', 'gen_golden.py'))
     gen = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(gen)
