@@ -33,6 +33,7 @@
 //             per-CTA loss partials and bumps the device step counter beside the tiles.
 //
 // All arithmetic is FP32 FFMA (IEEE); see DESIGN.md section 4 for why tensor cores do not apply here.
+// The stream and action kernels are instantiated for hidden 64, 128 and 256 (Width<H>); the numbers above are for 256.
 #include <stdlib.h>
 
 #include "her_device.cuh"
@@ -43,7 +44,8 @@
 namespace cur {
 
 constexpr int S_ROWS = 4;                // batch rows per CTA
-constexpr int S_H = 256;                 // hidden units
+constexpr int S_H = 256;                 // hidden units of the widest instantiation (also 64 and 128, see Width)
+constexpr int S_KIN = 256;               // widest first-layer input (may exceed a narrow hidden width: Arm8 is 100)
 constexpr int S_CONSUMERS = 256;         // 8 consumer warps
 constexpr int S_THREADS = S_CONSUMERS + 32;   // + 1 producer warp
 constexpr int S_CK = 32;                 // k rows per weight chunk
@@ -59,9 +61,36 @@ constexpr int S_MISC = 2048;              // small per-CTA state + the staged HE
 constexpr int S_STAGE_OFF = 256;          // float offset of the HER stage inside misc
 constexpr size_t S_SMEM_BYTES = (size_t)(S_NSLOT * S_SLOT + 2 * S_XT + S_RED + S_MISC) * 4 + 128;   // + 9 mbarriers
 
+// The stream / action kernels at hidden width H in {64, 128, 256} (pad_hidden='native' runs a narrow net at its true
+// width).  A thread owns 4 output columns: H / 4 column groups, and the 256 consumer threads split a chunk's k rows into
+// KS = 1024 / H k-slices of RK rows each.  A chunk fills a 32 KB slot (32 rows at 256, 64 at 128); at 64 a hidden layer
+// has only 64 k rows, so its chunk is the whole 16 KB layer and a thread takes 4 of them instead of 8.  The KS partial
+// sums of a column are added in a fixed pairwise tree (TreeSum): the same bits on every run.
+template <int H>
+struct Width {
+  static_assert(H == 64 || H == 128 || H == 256, "instantiated widths");
+  static constexpr int CG = H / 4;                              // column groups
+  static constexpr int KS = S_CONSUMERS / CG;                   // k-slices
+  static constexpr int CK = (S_SLOT / H < H) ? S_SLOT / H : H;  // k rows per weight chunk
+  static constexpr int RK = CK / KS;                            // k rows of one thread per chunk
+  static_assert(KS * RK == CK && KS * 4 * H <= S_RED, "chunk split / partials fit");
+};
+static int chunk_rows(int H) { return H == 64 ? Width<64>::CK : H == 128 ? Width<128>::CK : Width<256>::CK; }
+
+template <int N>
+struct TreeSum {   // ((p[0] + p[s]) + (p[2s] + p[3s])) + ...: a fixed summation order of N partials
+  __device__ __forceinline__ static float run(const float* p, int s) {
+    return TreeSum<N / 2>::run(p, s) + TreeSum<N / 2>::run(p + (N / 2) * s, s);
+  }
+};
+template <>
+struct TreeSum<1> {
+  __device__ __forceinline__ static float run(const float* p, int) { return p[0]; }
+};
+
 struct SChunk {
-  const float* src;   // nrows x 256 floats, contiguous
-  int nrows;          // <= 32
+  const float* src;   // nrows x H floats, contiguous
+  int nrows;          // <= Width<H>::CK
   int k0;             // first k row of the layer this chunk covers
 };
 
@@ -79,7 +108,7 @@ struct StreamParams {
   const float* W0Q_act;      // main Q first-layer rows of the action inputs: [dimu][H]
   int ch0[2];                // chunks of a first layer: [0] pi nets, [1] Q nets
   float *Xp, *Xq;            // [n][KP] first-layer inputs of main.pi / main.Q(u)   (weight-gradient operands)
-  float *hp[S_MAXL], *hq[S_MAXL], *hqp[S_MAXL], *dc[S_MAXL], *dp[S_MAXL];   // row-major [n][256]
+  float *hp[S_MAXL], *hq[S_MAXL], *hqp[S_MAXL], *dc[S_MAXL], *dp[S_MAXL];   // row-major [n][H]
   float *dQ, *dy;            // [n], [n][lddy]
   int lddy;
   float* loss_part;          // [n / 4][4]
@@ -219,31 +248,33 @@ __device__ __forceinline__ void fma_row(float2 (&acc)[NR / 2][4], const float* _
 }
 
 // acc += sum over this thread's k rows of the next `nchunks` weight chunks of  xT[k][r] * W[k][4cg + c]
-template <int NR, class PT>
+template <int H, int NR, class PT>
 __device__ __forceinline__ void gemv_chunks(const PT& P, Ring& rg, int nchunks, const float* __restrict__ xT,
                                             float2 (&acc)[NR / 2][4]) {
-  const int cg = threadIdx.x & 63, ks = threadIdx.x >> 6;
+  using Wd = Width<H>;
+  constexpr int RK = Wd::RK;
+  const int cg = threadIdx.x % Wd::CG, ks = threadIdx.x / Wd::CG;
 #pragma unroll 1
   for (int c = 0; c < nchunks; ++c) {
     const int slot = rg.cons % S_NSLOT;
     const int nrows = rg.chunks[rg.cons].nrows, k0 = rg.chunks[rg.cons].k0;
     mbar_wait(rg.full + 8 * slot, (rg.cons / S_NSLOT) & 1);
     const float* ws = rg.slots + slot * S_SLOT + 4 * cg;
-    const float* xs = xT + (k0 + ks * 8) * NR;
+    const float* xs = xT + (k0 + ks * RK) * NR;
     if (P.dbg_skip_math) {
-    } else if (nrows == S_CK) {
-      // full chunk (all but the ragged first-layer blocks): no guards, so the LDS.128 of the thread's 8 k rows
+    } else if (nrows == Wd::CK) {
+      // full chunk (all but the ragged first-layer blocks): no guards, so the LDS.128 of the thread's RK k rows
       // are issued up front and the FFMA2s run back to back
-      float4 w[8];
+      float4 w[RK];
 #pragma unroll
-      for (int kk = 0; kk < 8; ++kk) w[kk] = *reinterpret_cast<const float4*>(ws + (ks * 8 + kk) * S_H);
+      for (int kk = 0; kk < RK; ++kk) w[kk] = *reinterpret_cast<const float4*>(ws + (ks * RK + kk) * H);
 #pragma unroll
-      for (int kk = 0; kk < 8; ++kk) fma_row<NR>(acc, xs + kk * NR, w[kk]);
+      for (int kk = 0; kk < RK; ++kk) fma_row<NR>(acc, xs + kk * NR, w[kk]);
     } else {
 #pragma unroll 1
-      for (int kk = 0; kk < 8; ++kk)
-        if (ks * 8 + kk < nrows)
-          fma_row<NR>(acc, xs + kk * NR, *reinterpret_cast<const float4*>(ws + (ks * 8 + kk) * S_H));
+      for (int kk = 0; kk < RK; ++kk)
+        if (ks * RK + kk < nrows)
+          fma_row<NR>(acc, xs + kk * NR, *reinterpret_cast<const float4*>(ws + (ks * RK + kk) * H));
     }
     __syncwarp();
     if ((threadIdx.x & 31) == 0) mbar_arrive(rg.empty + 8 * slot);
@@ -251,38 +282,47 @@ __device__ __forceinline__ void gemv_chunks(const PT& P, Ring& rg, int nchunks, 
   }
 }
 
+// A consumer thread that owns an output column: all of them at H = 256; below, threads H.. only take part in the
+// k-slices of the GEMV and in the barriers.
+template <int H>
+__device__ __forceinline__ bool owns_col(int col) { return H == S_CONSUMERS || col < H; }
+
 // One dense layer for NR rows: chunks -> split-K partials -> fixed-order sum.  Returns, for the thread's column
-// `col = tid`, the NR pre-activation sums in v[] (without bias).
-template <int NR, class PT>
+// `col = tid` (if owns_col), the NR pre-activation sums in v[] (without bias).
+template <int H, int NR, class PT>
 __device__ __forceinline__ void layer_gemv(const PT& P, Ring& rg, int nchunks, const float* xT, float* red,
                                            float (&v)[NR]) {
+  using Wd = Width<H>;
   float2 acc[NR / 2][4];
 #pragma unroll
   for (int p = 0; p < NR / 2; ++p)
 #pragma unroll
     for (int c = 0; c < 4; ++c) acc[p][c] = make_float2(0.f, 0.f);
-  gemv_chunks<NR>(P, rg, nchunks, xT, acc);
-  const int cg = threadIdx.x & 63, ks = threadIdx.x >> 6;
+  gemv_chunks<H, NR>(P, rg, nchunks, xT, acc);
+  const int cg = threadIdx.x % Wd::CG, ks = threadIdx.x / Wd::CG;
 #pragma unroll
   for (int p = 0; p < NR / 2; ++p) {
-    *reinterpret_cast<float4*>(red + (ks * NR + 2 * p) * S_H + 4 * cg) =
+    *reinterpret_cast<float4*>(red + (ks * NR + 2 * p) * H + 4 * cg) =
         make_float4(acc[p][0].x, acc[p][1].x, acc[p][2].x, acc[p][3].x);
-    *reinterpret_cast<float4*>(red + (ks * NR + 2 * p + 1) * S_H + 4 * cg) =
+    *reinterpret_cast<float4*>(red + (ks * NR + 2 * p + 1) * H + 4 * cg) =
         make_float4(acc[p][0].y, acc[p][1].y, acc[p][2].y, acc[p][3].y);
   }
   consumer_sync();
   const int col = threadIdx.x;
+  if (owns_col<H>(col)) {
 #pragma unroll
-  for (int r = 0; r < NR; ++r) {
-    const float* p = red + r * S_H + col;
-    v[r] = (p[0] + p[NR * S_H]) + (p[2 * NR * S_H] + p[3 * NR * S_H]);
+    for (int r = 0; r < NR; ++r) v[r] = TreeSum<Wd::KS>::run(red + r * H + col, NR * H);
+  } else {
+#pragma unroll
+    for (int r = 0; r < NR; ++r) v[r] = 0.f;
   }
 }
 
 // write the layer output: transposed into shared memory for the next layer, row-major to global for launch 2
-template <int NR>
+template <int H, int NR>
 __device__ __forceinline__ void put_xT(float* yT, const float (&v)[NR]) {
   const int col = threadIdx.x;
+  if (!owns_col<H>(col)) return;
 #pragma unroll
   for (int q = 0; q < NR / 4; ++q)
     *reinterpret_cast<float4*>(yT + col * NR + 4 * q) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
@@ -402,8 +442,9 @@ __device__ __forceinline__ void sample_rows(const StreamParams& P, int64_t row0,
   consumer_sync();
 }
 
-// y[r][j] = sum_k xT[k][r] * W[k * ldk + j * ldj] + bias[j]  for r < NR, j < nout (NR * nout <= 32), K = 256.
+// y[r][j] = sum_k xT[k][r] * W[k * ldk + j * ldj] + bias[j]  for r < NR, j < nout (NR * nout <= 32), K = H.
 // 8 k-parts per output (interleaved k), combined with a fixed shuffle tree; every thread must call it.
+template <int H>
 __device__ __noinline__ void small_out(const float* xT, int NR, int roff, int nr, const float* __restrict__ W, int ldk,
                                        int ldj, int nout, const float* bias, float* out /* [r][S_DU] */) {
   const int kp = threadIdx.x & 7, oj = threadIdx.x >> 3;
@@ -413,11 +454,11 @@ __device__ __noinline__ void small_out(const float* xT, int NR, int roff, int nr
   if (on) {
     // all 32 weight loads of the thread in flight at once: one exposed L2 round trip instead of four (the loop is on the
     // critical path of every net: nothing else runs in the CTA meanwhile)
-    float wv[S_H / 8];
+    float wv[H / 8];
 #pragma unroll
-    for (int kk = 0; kk < S_H / 8; ++kk) wv[kk] = __ldg(W + (int64_t)(kp + 8 * kk) * ldk + (int64_t)j * ldj);
+    for (int kk = 0; kk < H / 8; ++kk) wv[kk] = __ldg(W + (int64_t)(kp + 8 * kk) * ldk + (int64_t)j * ldj);
 #pragma unroll
-    for (int kk = 0; kk < S_H / 8; ++kk) acc = fmaf(xT[(kp + 8 * kk) * NR + roff + r], wv[kk], acc);
+    for (int kk = 0; kk < H / 8; ++kk) acc = fmaf(xT[(kp + 8 * kk) * NR + roff + r], wv[kk], acc);
   }
   acc += __shfl_xor_sync(0xffffffffu, acc, 1);
   acc += __shfl_xor_sync(0xffffffffu, acc, 2);
@@ -430,28 +471,29 @@ __device__ __forceinline__ float relu_mask(float v, float m) { return m > 0.f ? 
 // One forward net for NR rows: L hidden layers (bias + ReLU) from the first-layer input already in `xa`; optional
 // row-major copies of every hidden activation (rows 0-3 -> h_a, rows 4-7 -> h_b).  Returns the buffer that holds
 // the last hidden activations (transposed).
-template <int NR, class PT>
+template <int H, int NR, class PT>
 __device__ __forceinline__ float* forward_net(const PT& P, Ring& rg, int ch0, float* xa, float* xb, float* red,
                                               const float* const* bias, float* const* h_a, float* const* h_b,
                                               int64_t row0) {
   const int col = threadIdx.x;
+  const bool on = owns_col<H>(col);
   float* xin = xa;
   float* xout = xb;
   for (int l = 0; l < P.L; ++l) {
     float v[NR];
-    const float b = bias[l][col];                 // in flight during the layer (an exposed L2 round trip otherwise)
-    layer_gemv<NR>(P, rg, l == 0 ? ch0 : S_H / S_CK, xin, red, v);
+    const float b = on ? bias[l][col] : 0.f;      // in flight during the layer (an exposed L2 round trip otherwise)
+    layer_gemv<H, NR>(P, rg, l == 0 ? ch0 : H / Width<H>::CK, xin, red, v);
 #pragma unroll
     for (int r = 0; r < NR; ++r) v[r] = fmaxf(v[r] + b, 0.f);
-    if (h_a != nullptr) {
+    if (on && h_a != nullptr) {
 #pragma unroll
-      for (int r = 0; r < 4; ++r) h_a[l][(row0 + r) * S_H + col] = v[r];
+      for (int r = 0; r < 4; ++r) h_a[l][(row0 + r) * H + col] = v[r];
     }
-    if (NR == 8 && h_b != nullptr) {
+    if (on && NR == 8 && h_b != nullptr) {
 #pragma unroll
-      for (int r = 0; r < 4; ++r) h_b[l][(row0 + r) * S_H + col] = v[NR - 4 + r];
+      for (int r = 0; r < 4; ++r) h_b[l][(row0 + r) * H + col] = v[NR - 4 + r];
     }
-    put_xT<NR>(xout, v);
+    put_xT<H, NR>(xout, v);
     consumer_sync();
     float* t = xin; xin = xout; xout = t;
   }
@@ -464,6 +506,7 @@ __device__ __forceinline__ float* forward_net(const PT& P, Ring& rg, int ch0, fl
 // Each SM ingests 2.2-2.3 MB of weights for FOUR rows at a time (per-SM L2 -> shared bandwidth is what bounds this
 // kernel; the earlier main / target split streamed main.Q once for 8 stacked rows, which made those passes FFMA-bound
 // and left the target CTA idle for 40 % of the kernel).
+template <int H>
 __global__ void __launch_bounds__(S_THREADS, 1)
 ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -511,7 +554,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
       for (int i = 0; i < total; ++i) {
         const int slot = i % S_NSLOT, round = i / S_NSLOT;
         if (round > 0) mbar_wait(empty + 8 * slot, (round - 1) & 1);
-        const uint32_t bytes = (uint32_t)my_chunks[i].nrows * S_H * 4;
+        const uint32_t bytes = (uint32_t)my_chunks[i].nrows * H * 4;
         mbar_expect_tx(full + 8 * slot, bytes);
         bulk_g2s(ring_s + slot * S_SLOT * 4, my_chunks[i].src, bytes, full + 8 * slot);
       }
@@ -523,6 +566,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   Ring rg;
   rg.chunks = my_chunks; rg.slots = ringf; rg.full = full; rg.empty = empty; rg.cons = 0;
   const int col = tid;
+  const bool on = owns_col<H>(col);      // this thread owns an output column of the hidden layers
   const float inv_n = 1.0f / (float)P.grad_rows;      // scale of the backward seeds
   const float* stage = nullptr;
   if (P.fused_her) {
@@ -536,21 +580,21 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
     // main.Q(o, g, u), the TD loss and the critic's backward chain.  Nothing is exchanged with the actor CTA.
     build_x(P, xa, 4, 0, row0, true, 0, nullptr, nullptr, stage);
     consumer_sync();
-    float* xl = forward_net<4>(P, rg, P.ch0[0], xa, xb, red, P.bPT, nullptr, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutPT, d.dimu, 1, d.dimu, P.boutPT, s_th);
+    float* xl = forward_net<H, 4>(P, rg, P.ch0[0], xa, xb, red, P.bPT, nullptr, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutPT, d.dimu, 1, d.dimu, P.boutPT, s_th);
     consumer_sync();
     if (tid < S_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);
     consumer_sync();
     build_x(P, xa, 4, 0, row0, true, 2, s_th, nullptr, stage);
     consumer_sync();
-    xl = forward_net<4>(P, rg, P.ch0[1], xa, xb, red, P.bQT, nullptr, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutQT, 1, 1, 1, P.boutQT, s_qt);
+    xl = forward_net<H, 4>(P, rg, P.ch0[1], xa, xb, red, P.bQT, nullptr, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutQT, 1, 1, 1, P.boutQT, s_qt);
     consumer_sync();
     // main.Q(o, g, u)
     build_x(P, xa, 4, 0, row0, false, 1, nullptr, P.Xq, stage);
     consumer_sync();
-    xl = forward_net<4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, P.hq, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
+    xl = forward_net<H, 4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, P.hq, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
     consumer_sync();
     // critic loss (ddpg.py:436-439) and its backward seed
     if (tid < S_ROWS) {
@@ -570,29 +614,29 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
     }
     // backward through main.Q (critic chain): gradient at the last hidden layer is dQ * Wout^T (Wout is [H][1])
     float* xin = xa; float* xout = xb;
-    {
+    if (on) {
       const float wq = __ldg(P.WoutQ + col);
       float v[4];
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
-        v[r] = relu_mask(s_dq[r] * wq, __ldcg(P.hq[L - 1] + (row0 + r) * S_H + col));
-        P.dc[L - 1][(row0 + r) * S_H + col] = v[r];
+        v[r] = relu_mask(s_dq[r] * wq, __ldcg(P.hq[L - 1] + (row0 + r) * H + col));
+        P.dc[L - 1][(row0 + r) * H + col] = v[r];
       }
-      put_xT<4>(xin, v);
-      consumer_sync();
+      put_xT<H, 4>(xin, v);
     }
+    consumer_sync();
     for (int l = L - 1; l >= 1; --l) {
       float m[4];
 #pragma unroll
-      for (int r = 0; r < 4; ++r) m[r] = __ldcg(P.hq[l - 1] + (row0 + r) * S_H + col);   // ReLU masks of layer l-1
+      for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hq[l - 1] + (row0 + r) * H + col) : 0.f;   // ReLU masks of layer l-1
       float v[4];
-      layer_gemv<4>(P, rg, S_H / S_CK, xin, red, v);
+      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         v[r] = relu_mask(v[r], m[r]);
-        P.dc[l - 1][(row0 + r) * S_H + col] = v[r];
+        if (on) P.dc[l - 1][(row0 + r) * H + col] = v[r];
       }
-      put_xT<4>(xout, v);
+      put_xT<H, 4>(xout, v);
       consumer_sync();
       float* t = xin; xin = xout; xout = t;
     }
@@ -608,8 +652,8 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   consumer_sync();
   S_TL(1);
   {
-    float* xl = forward_net<4>(P, rg, P.ch0[0], xa, xb, red, P.bP, P.hp, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
+    float* xl = forward_net<H, 4>(P, rg, P.ch0[0], xa, xb, red, P.bP, P.hp, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
     consumer_sync();
     if (tid < S_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);   // actor_critic.py:89
     consumer_sync();
@@ -619,8 +663,8 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   build_x(P, xa, 4, 0, row0, false, 2, s_th, nullptr, stage);
   consumer_sync();
   {
-    float* xl = forward_net<4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, P.hqp, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
+    float* xl = forward_net<H, 4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, P.hqp, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
     consumer_sync();
   }
   S_TL(4);
@@ -643,29 +687,29 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   // ===== backward through main.Q, actor-through-critic chain =====
   {
     float* xin = xa; float* xout = xb;
-    {
+    if (on) {
       const float wq = __ldg(P.WoutQ + col);
       float v[4];
 #pragma unroll
-      for (int r = 0; r < 4; ++r) v[r] = relu_mask(s_dq[r] * wq, __ldcg(P.hqp[L - 1] + (row0 + r) * S_H + col));
-      put_xT<4>(xin, v);
-      consumer_sync();
+      for (int r = 0; r < 4; ++r) v[r] = relu_mask(s_dq[r] * wq, __ldcg(P.hqp[L - 1] + (row0 + r) * H + col));
+      put_xT<H, 4>(xin, v);
     }
+    consumer_sync();
     for (int l = L - 1; l >= 1; --l) {
       float m[4];
 #pragma unroll
-      for (int r = 0; r < 4; ++r) m[r] = __ldcg(P.hqp[l - 1] + (row0 + r) * S_H + col);
+      for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hqp[l - 1] + (row0 + r) * H + col) : 0.f;
       float v[4];
-      layer_gemv<4>(P, rg, S_H / S_CK, xin, red, v);
+      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) v[r] = relu_mask(v[r], m[r]);
-      put_xT<4>(xout, v);
+      put_xT<H, 4>(xout, v);
       consumer_sync();
       float* t = xin; xin = xout; xout = t;
     }
     // gradient wrt the action inputs of main.Q, then through tanh and the action penalty (ddpg.py:440-441):
     // d pi_loss/d(pre-tanh) = (dL/d(pi/max_u) + action_l2*2/(B*dimu)*th) * (1 - th^2)
-    small_out(xin, 4, 0, 4, P.W0Q_act, 1, S_H, d.dimu, nullptr, s_dy);
+    small_out<H>(xin, 4, 0, 4, P.W0Q_act, 1, H, d.dimu, nullptr, s_dy);
     consumer_sync();
     if (tid < S_ROWS * S_DU) {
       const int r = tid >> 3, j = tid & (S_DU - 1);
@@ -684,7 +728,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   // ===== backward through main.pi =====
   {
     float* xin = xa; float* xout = xb;
-    {
+    if (on) {
       float v[4];
 #pragma unroll
       for (int r = 0; r < 4; ++r) v[r] = 0.f;
@@ -695,24 +739,24 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
       }
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
-        v[r] = relu_mask(v[r], __ldcg(P.hp[L - 1] + (row0 + r) * S_H + col));
-        P.dp[L - 1][(row0 + r) * S_H + col] = v[r];
+        v[r] = relu_mask(v[r], __ldcg(P.hp[L - 1] + (row0 + r) * H + col));
+        P.dp[L - 1][(row0 + r) * H + col] = v[r];
       }
-      put_xT<4>(xin, v);
-      consumer_sync();
+      put_xT<H, 4>(xin, v);
     }
+    consumer_sync();
     for (int l = L - 1; l >= 1; --l) {
       float m[4];
 #pragma unroll
-      for (int r = 0; r < 4; ++r) m[r] = __ldcg(P.hp[l - 1] + (row0 + r) * S_H + col);
+      for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hp[l - 1] + (row0 + r) * H + col) : 0.f;
       float v[4];
-      layer_gemv<4>(P, rg, S_H / S_CK, xin, red, v);
+      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         v[r] = relu_mask(v[r], m[r]);
-        P.dp[l - 1][(row0 + r) * S_H + col] = v[r];
+        if (on) P.dp[l - 1][(row0 + r) * H + col] = v[r];
       }
-      put_xT<4>(xout, v);
+      put_xT<H, 4>(xout, v);
       consumer_sync();
       float* t = xin; xin = xout; xout = t;
     }
@@ -989,7 +1033,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
     consumer_sync();
     float* xl = pair_forward_net(P, rg, X, PP.pch0[0], L, gc0, xa, xb, red, P.bPT, nullptr, row0);
     X.wait();
-    small_out(xl, PR_ROWS, 0, PR_ROWS, P.WoutPT, d.dimu, 1, d.dimu, P.boutPT, s_th);
+    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutPT, d.dimu, 1, d.dimu, P.boutPT, s_th);
     consumer_sync();
     if (tid < PR_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);
     X.sync();
@@ -998,7 +1042,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
     consumer_sync();
     xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQT, nullptr, row0);
     X.wait();
-    small_out(xl, PR_ROWS, 0, PR_ROWS, P.WoutQT, 1, 1, 1, P.boutQT, s_qt);
+    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQT, 1, 1, 1, P.boutQT, s_qt);
     X.sync();
     consumer_sync();
     // main.Q(o, g, u)
@@ -1006,7 +1050,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
     consumer_sync();
     xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQ, P.hq, row0);
     X.wait();
-    small_out(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
+    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
     consumer_sync();
     // critic loss (ddpg.py:436-439) and its backward seed
     if (tid < PR_ROWS) {
@@ -1053,7 +1097,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
     float* xl = pair_forward_net(P, rg, X, PP.pch0[0], L, gc0, xa, xb, red, P.bP, P.hp, row0);
     X.wait();
     X.dbg = nullptr;
-    small_out(xl, PR_ROWS, 0, PR_ROWS, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
+    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
     consumer_sync();
     if (tid < PR_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);   // actor_critic.py:89
     X.sync();
@@ -1066,7 +1110,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
   {
     float* xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQ, P.hqp, row0);
     X.wait();
-    small_out(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
+    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
     consumer_sync();
   }
   PR_TL(4);
@@ -1102,7 +1146,7 @@ __device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf
     X.wait();
     // gradient wrt the action inputs of main.Q, then through tanh and the action penalty (ddpg.py:440-441):
     // d pi_loss/d(pre-tanh) = (dL/d(pi/max_u) + action_l2*2/(B*dimu)*th) * (1 - th^2)
-    small_out(xin, PR_ROWS, 0, PR_ROWS, P.W0Q_act, 1, S_H, d.dimu, nullptr, s_dy);
+    small_out<S_H>(xin, PR_ROWS, 0, PR_ROWS, P.W0Q_act, 1, S_H, d.dimu, nullptr, s_dy);
     consumer_sync();
     if (tid < PR_ROWS * S_DU) {
       const int r = tid >> 3, j = tid & (S_DU - 1);
@@ -1252,6 +1296,7 @@ __device__ __forceinline__ void put_out(void* base, int64_t i, float v, uint32_t
   else st_ll(reinterpret_cast<unsigned long long*>(base) + i, v, seq);
 }
 
+template <int H>
 __global__ void __launch_bounds__(S_THREADS, 1)
 actions_stream_kernel(const __grid_constant__ ActParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1281,7 +1326,7 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
       for (int i = 0; i < P.nchunks; ++i) {
         const int slot = i % S_NSLOT, round = i / S_NSLOT;
         if (round > 0) mbar_wait(empty + 8 * slot, (round - 1) & 1);
-        const uint32_t bytes = (uint32_t)P.chunks[i].nrows * S_H * 4;
+        const uint32_t bytes = (uint32_t)P.chunks[i].nrows * H * 4;
         mbar_expect_tx(full + 8 * slot, bytes);
         bulk_g2s(ring_s + slot * S_SLOT * 4, P.chunks[i].src, bytes, full + 8 * slot);
       }
@@ -1305,8 +1350,8 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
   build(0);
   consumer_sync();
   A_TL(1);
-  float* xl = forward_net<4>(P, rg, P.ch0[0], xa, xb, red, P.bP, nullptr, nullptr, row0);
-  small_out(xl, 4, 0, 4, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
+  float* xl = forward_net<H, 4>(P, rg, P.ch0[0], xa, xb, red, P.bP, nullptr, nullptr, row0);
+  small_out<H>(xl, 4, 0, 4, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
   consumer_sync();
   A_TL(2);
   if (tid < S_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) {
@@ -1319,8 +1364,8 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
   if (P.q != nullptr) {
     build(2);                                                          // Q(o, g, pi / max_u): the noise-free action
     consumer_sync();
-    xl = forward_net<4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, nullptr, nullptr, row0);
-    small_out(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
+    xl = forward_net<H, 4>(P, rg, P.ch0[1], xa, xb, red, P.bQ, nullptr, nullptr, row0);
+    small_out<H>(xl, 4, 0, 4, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
     consumer_sync();
     if (tid < nr) put_out(P.q, row0 + tid, s_q[tid * S_DU], P.seq);
   }
@@ -1328,12 +1373,13 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
 #undef A_TL
 }
 
-// W^T of the hidden layers (operands of the backward streams): dst[m][j][i] = src_m[i][j], 256 x 256 each
+// W^T of the hidden layers (operands of the backward streams): dst[m][j][i] = src_m[i][j], H x H each
 struct TransposeParams {
   const float* src[2 * S_MAXL];
   float* dst[2 * S_MAXL];
 };
 
+template <int H>
 __global__ void __launch_bounds__(256) transpose_kernel(const __grid_constant__ TransposeParams T) {
   __shared__ float tile[32][33];
   const float* src = T.src[blockIdx.z];
@@ -1341,10 +1387,17 @@ __global__ void __launch_bounds__(256) transpose_kernel(const __grid_constant__ 
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   const int i0 = blockIdx.y * 32, j0 = blockIdx.x * 32;
 #pragma unroll
-  for (int q = 0; q < 4; ++q) tile[ty + 8 * q][tx] = src[(int64_t)(i0 + ty + 8 * q) * S_H + j0 + tx];
+  for (int q = 0; q < 4; ++q) tile[ty + 8 * q][tx] = src[(int64_t)(i0 + ty + 8 * q) * H + j0 + tx];
   __syncthreads();
 #pragma unroll
-  for (int q = 0; q < 4; ++q) dst[(int64_t)(j0 + ty + 8 * q) * S_H + i0 + tx] = tile[tx][ty + 8 * q];
+  for (int q = 0; q < 4; ++q) dst[(int64_t)(j0 + ty + 8 * q) * H + i0 + tx] = tile[tx][ty + 8 * q];
+}
+
+static void launch_transposes(const TransposeParams& TP, int m, int H, cudaStream_t s) {
+  const dim3 grid(H / 32, H / 32, m);
+  if (H == 64) transpose_kernel<64><<<grid, 256, 0, s>>>(TP);
+  else if (H == 128) transpose_kernel<128><<<grid, 256, 0, s>>>(TP);
+  else transpose_kernel<256><<<grid, 256, 0, s>>>(TP);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1942,8 +1995,8 @@ struct RowsWorkspace {
   unsigned int* ticket;
   float* loss_part;
   float *Xp, *Xq;
-  float *hp[S_MAXL], *hq[S_MAXL], *hqp[S_MAXL], *dc[S_MAXL], *dp[S_MAXL];   // row-major [n][256]
-  float *TQ[S_MAXL], *TP[S_MAXL];                                            // W_l^T, l = 1..L-1
+  float *hp[S_MAXL], *hq[S_MAXL], *hqp[S_MAXL], *dc[S_MAXL], *dp[S_MAXL];   // row-major [n][H]
+  float *TQ[S_MAXL], *TP[S_MAXL];                                            // W_l^T [H][H], l = 1..L-1
   float *dQ, *dy;
   int KP, lddy;
   int64_t total;
@@ -1955,6 +2008,7 @@ static RowsWorkspace carve_rows(const cur_net_desc& d, int64_t n, float* base) {
   const int K0q = q.in_s + q.in_g;
   w.KP = (int)r4(K0q);
   w.lddy = (int)r4(d.dimu);
+  const int64_t H = d.hidden;
   int64_t o = 0;
   auto take = [&](int64_t floats) {
     float* ptr = base ? base + o : nullptr;
@@ -1966,10 +2020,10 @@ static RowsWorkspace carve_rows(const cur_net_desc& d, int64_t n, float* base) {
   w.Xp = take(n * w.KP);
   w.Xq = take(n * w.KP);
   for (int l = 0; l < d.layers; ++l) {
-    w.hp[l] = take(n * S_H); w.hq[l] = take(n * S_H); w.hqp[l] = take(n * S_H);
-    w.dc[l] = take(n * S_H); w.dp[l] = take(n * S_H);
-    w.TQ[l] = (l >= 1) ? take((int64_t)S_H * S_H) : nullptr;
-    w.TP[l] = (l >= 1) ? take((int64_t)S_H * S_H) : nullptr;
+    w.hp[l] = take(n * H); w.hq[l] = take(n * H); w.hqp[l] = take(n * H);
+    w.dc[l] = take(n * H); w.dp[l] = take(n * H);
+    w.TQ[l] = (l >= 1) ? take(H * H) : nullptr;
+    w.TP[l] = (l >= 1) ? take(H * H) : nullptr;
   }
   w.dQ = take(n);
   w.dy = take(n * w.lddy);
@@ -1983,10 +2037,11 @@ constexpr int64_t ROWS_MAX_BATCH = 1024;
 
 static bool rows_supported(const cur_net_desc* d, int64_t n) {
   if (check_desc(d) != CUR_OK) return false;
-  if (d->hidden != S_H || d->layers < 1 || d->layers > S_MAXL) return false;
+  // hidden 256, and 64 / 128 for networks run at their true width (pad_hidden='native'; the CTA-pair kernel is 256 only)
+  if ((d->hidden != 64 && d->hidden != 128 && d->hidden != S_H) || d->layers < 1 || d->layers > S_MAXL) return false;
   if (d->dimu > S_DU || n <= 0 || (n % S_ROWS) != 0 || n > ROWS_MAX_BATCH) return false;
   const NetLayout q = net_layout(*d, 0), p = net_layout(*d, 1);
-  if (q.in_s + q.in_g > S_H) return false;
+  if (q.in_s + q.in_g > S_KIN) return false;        // the transposed first-layer input buffer, not the hidden width
   // operands of the first-layer weight gradients must be 16-byte aligned column blocks of X
   if ((q.in_s % 4) != 0 || (p.in_s % 4) != 0 || (q.in_g % 4) != 0) return false;
   if (d->dimu > 4 && (d->dimu % 4) != 0) return false;
@@ -2015,6 +2070,30 @@ static void build_dw_batch(GemmBatch& G, const NetLayout& LQ, const NetLayout& L
   };
   net_grads(LQ, gQ, w.Xq, w.hq, w.dc, w.dQ, 1);
   net_grads(LP, gP, w.Xp, w.hp, w.dp, w.dy, w.lddy);
+}
+
+template <int H>
+static int launch_stream(cudaLaunchConfig_t& cfg, const StreamParams& P) {
+  static bool configured = false;
+  if (!configured) {
+    CUR_CUDA_TRY(cudaFuncSetAttribute(ddpg_stream_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)S_SMEM_BYTES));
+    configured = true;
+  }
+  CUR_CUDA_TRY(cudaLaunchKernelEx(&cfg, ddpg_stream_kernel<H>, P));
+  return CUR_OK;
+}
+
+template <int H>
+static int launch_actions(unsigned blocks, cudaStream_t s, const ActParams& P) {
+  static bool configured = false;
+  if (!configured) {
+    CUR_CUDA_TRY(cudaFuncSetAttribute(actions_stream_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)S_SMEM_BYTES));
+    configured = true;
+  }
+  actions_stream_kernel<H><<<blocks, S_THREADS, S_SMEM_BYTES, s>>>(P);
+  return CUR_OK;
 }
 
 // launch configuration; CUR_PDL=1 adds programmatic stream serialisation (measured: batch 256 60.2 us with, 58.3 us
@@ -2138,13 +2217,6 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
   const RowsWorkspace w = carve_rows(*d, n, workspace);
   const int L = d->layers, H = d->hidden;
 
-  static bool configured = false;
-  if (!configured) {
-    CUR_CUDA_TRY(cudaFuncSetAttribute(ddpg_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)S_SMEM_BYTES));
-    configured = true;
-  }
-
   // ---- launch 0: W_l^T of the hidden layers of main.Q and main.pi.  With the fused optimiser the weight-gradient
   // epilogue of the previous call already left the transposes of the stepped weights in the workspace; the caller says
   // so with adam->transposes_valid (and refreshes them with cur_ddpg_rows_refresh after any other change of theta).
@@ -2157,7 +2229,7 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
       TP.src[m] = mQ + LQ.off_W[l]; TP.dst[m++] = w.TQ[l];
       TP.src[m] = mP + LP.off_W[l]; TP.dst[m++] = w.TP[l];
     }
-    transpose_kernel<<<dim3(H / 32, H / 32, m), 256, 0, s>>>(TP);
+    launch_transposes(TP, m, H, s);
     CUR_CHECK_LAUNCH();
   }
 
@@ -2201,10 +2273,11 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
   // ---- weight chunks in consumption order
   int nc = 0;
   SChunk* list = P.chunks;
-  auto rows_of = [&](const float* src, int nrows, int k0) {      // a row block as chunks of <= 32 rows
-    for (int r = 0; r < nrows; r += S_CK) {
+  const int CK = chunk_rows(H);
+  auto rows_of = [&](const float* src, int nrows, int k0) {      // a row block as chunks of <= CK rows
+    for (int r = 0; r < nrows; r += CK) {
       SChunk& C = list[nc++];
-      C.src = src + (int64_t)r * H; C.nrows = (nrows - r < S_CK) ? nrows - r : S_CK; C.k0 = k0 + r;
+      C.src = src + (int64_t)r * H; C.nrows = (nrows - r < CK) ? nrows - r : CK; C.k0 = k0 + r;
     }
   };
   auto forward_net = [&](const float* th, const NetLayout& NL) {
@@ -2249,7 +2322,7 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
   const unsigned int n_ctas = (unsigned int)(n / S_ROWS);
   // CTA-pair form (column split over a 2-CTA cluster, 8 rows per pair): half the weight bytes per SM
   static const int pair_mode = getenv("CUR_ROWS_PAIR") ? atoi(getenv("CUR_ROWS_PAIR")) : 0;   // measured slower, see profiles/README.md
-  const bool use_pair = pair_mode != 0 && (n % PR_ROWS) == 0 && d->dimu <= 4 &&
+  const bool use_pair = pair_mode != 0 && H == S_H && (n % PR_ROWS) == 0 && d->dimu <= 4 &&
                         (her == nullptr || PR_ROWS * P.plan.stage_stride <= PR_MISC - PR_STAGE_OFF);
   if (use_pair) {
     static bool pair_configured = false;
@@ -2339,7 +2412,9 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
     cudaLaunchConfig_t cfg;
     cudaLaunchAttribute at[1];
     pdl_config(cfg, at, 2 * n_ctas, S_THREADS, S_SMEM_BYTES, s);
-    CUR_CUDA_TRY(cudaLaunchKernelEx(&cfg, ddpg_stream_kernel, P));       // (actor, critic) CTA pairs
+    if (H == 64) CUR_TRY(launch_stream<64>(cfg, P));                     // (actor, critic) CTA pairs
+    else if (H == 128) CUR_TRY(launch_stream<128>(cfg, P));
+    else CUR_TRY(launch_stream<256>(cfg, P));
   }
   CUR_CHECK_LAUNCH();
   if (tl_on && ++tl_calls == 40) {          // debug only: one warmed-up timeline of CTA 0
@@ -2482,7 +2557,7 @@ extern "C" int cur_ddpg_rows_refresh(void* stream, const cur_net_desc* d, const 
     TP.src[m] = mQ + LQ.off_W[l]; TP.dst[m++] = w.TQ[l];
     TP.src[m] = mP + LP.off_W[l]; TP.dst[m++] = w.TP[l];
   }
-  transpose_kernel<<<dim3(H / 32, H / 32, m), 256, 0, (cudaStream_t)stream>>>(TP);
+  launch_transposes(TP, m, H, (cudaStream_t)stream);
   CUR_CHECK_LAUNCH();
   return CUR_OK;
 }
@@ -2520,14 +2595,7 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
   const NetLayout LQ = net_layout(*d, 0), LP = net_layout(*d, 1);
   const float *thQ = theta, *thP = theta + r4(LQ.total);
   const int L = d->layers, H = d->hidden;
-  static bool configured = false;
-  static bool tl_on = false;
-  if (!configured) {
-    CUR_CUDA_TRY(cudaFuncSetAttribute(actions_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)S_SMEM_BYTES));
-    tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
-    configured = true;
-  }
+  static const bool tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
   ActParams P;
   P.d = *d;
   P.in_sp = LP.in_s; P.in_g = LQ.in_g; P.L = L;
@@ -2545,10 +2613,11 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
   P.WoutQ = thQ + LQ.off_Wout; P.boutQ = thQ + LQ.off_bout;
   P.pi = out_pi; P.q = out_q;
   int nc = 0;
+  const int CK = chunk_rows(H);
   auto rows_of = [&](const float* src, int nrows, int k0) {
-    for (int r = 0; r < nrows; r += S_CK) {
+    for (int r = 0; r < nrows; r += CK) {
       SChunk& C = P.chunks[nc++];
-      C.src = src + (int64_t)r * H; C.nrows = (nrows - r < S_CK) ? nrows - r : S_CK; C.k0 = k0 + r;
+      C.src = src + (int64_t)r * H; C.nrows = (nrows - r < CK) ? nrows - r : CK; C.k0 = k0 + r;
     }
   };
   auto forward_net = [&](const float* th, const NetLayout& NL) {
@@ -2559,7 +2628,7 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
     for (int l = 1; l < L; ++l) rows_of(th + NL.off_W[l], H, 0);
     return first;
   };
-  CUR_REQUIRE((out_q ? 2 : 1) * (4 + (L - 1) * (H / S_CK)) <= A_MAXCHUNK, "too many weight chunks");
+  CUR_REQUIRE((out_q ? 2 : 1) * (4 + (L - 1) * (H / CK)) <= A_MAXCHUNK, "too many weight chunks");
   P.ch0[0] = forward_net(thP, LP);
   P.ch0[1] = out_q != nullptr ? forward_net(thQ, LQ) : 0;
   P.nchunks = nc;
@@ -2571,7 +2640,9 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
   }
   P.tl = tl_on ? tl_dev : nullptr;
   const unsigned blocks = (unsigned)((n + S_ROWS - 1) / S_ROWS);
-  actions_stream_kernel<<<blocks, S_THREADS, S_SMEM_BYTES, (cudaStream_t)stream>>>(P);
+  if (H == 64) CUR_TRY(launch_actions<64>(blocks, (cudaStream_t)stream, P));
+  else if (H == 128) CUR_TRY(launch_actions<128>(blocks, (cudaStream_t)stream, P));
+  else CUR_TRY(launch_actions<256>(blocks, (cudaStream_t)stream, P));
   CUR_CHECK_LAUNCH();
   if (tl_on && ++tl_calls == 100) {          // debug only: one warmed-up timeline of CTA 0 (%globaltimer, ns)
     long long t[8];

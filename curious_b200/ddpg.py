@@ -68,10 +68,19 @@ class DDPG(object):
         # level) or 'auto' (rows whenever the shape is supported)
         self.update_schedule = kwargs.get('update_schedule', 'auto')
         self.fuse_her = kwargs.get('fuse_her', True)      # rows schedule: sample inside the update kernel
-        # hidden widths below 256 (config.py:25 is a user parameter): 'auto' = run zero-padded to 256 on the hand-written
-        # row / chain / action kernels whenever they take the padded shape (actor_critic._NetSpec; same results, 59 instead
-        # of 140 us per batch-256 update), True = always, False = never (dependency-level kernels at the true width)
+        # hidden widths below 256 (config.py:25 is a user parameter), four values:
+        #   'auto'    run zero-padded to 256 on the hand-written row / chain / action kernels whenever they take the padded
+        #             shape (actor_critic._NetSpec; same results, 59 instead of 140 us per batch-256 update)
+        #   True      always zero-padded to 256
+        #   False     never: dependency-level kernels at the true width
+        #   'native'  hidden 64 / 128 at the true width on the row kernels (train() up to 1024 rows, with the CUDA graph,
+        #             fused HER and fused Adam / the tile exchange) and the one-launch action kernel (get_actions up to 512
+        #             rows, compute_Q included).  Above 1024 rows the tcgen05 chain kernel needs 256 columns, so such a
+        #             batch runs the dependency-level kernels at the true width, like False.  Hidden 256 runs as always;
+        #             any other width raises ValueError.
         self.pad_hidden = kwargs.get('pad_hidden', 'auto')
+        if self.pad_hidden == 'native' and self.hidden not in self.NATIVE_HIDDEN:
+            raise ValueError("pad_hidden='native' needs hidden in %s, not %r" % (self.NATIVE_HIDDEN, self.hidden))
         # several ranks: 'tile' = the gradient tiles are exchanged over NVLink peer memory INSIDE the weight-gradient
         # launch, Adam and W^T stay in its epilogue (csrc/ddpg_rows.cu, parallel.TileGradExchange: 2 launches per update
         # like one rank), 'p2p' = one exchange + Adam kernel after the weight-gradient launch (csrc/p2p.cu: every rank
@@ -151,7 +160,8 @@ class DDPG(object):
                                                  normalize_obs=self.normalize_obs, norm_clip=self.norm_clip,
                                                  kernel_hidden=kh)
         self.net = mk(None)
-        if self.pad_hidden and self.hidden < self.KERNEL_HIDDEN and self.update_schedule != 'levels':
+        if (self.pad_hidden and self.pad_hidden != 'native' and self.hidden < self.KERNEL_HIDDEN and
+                self.update_schedule != 'levels'):
             wide = mk(self.KERNEL_HIDDEN)
             rows = self.batch_size * max(1, int(getattr(self, 'workers_per_rank', 1)))
             if self.pad_hidden is True or _lib.load().cur_ddpg_rows_supported(C.byref(wide.desc), min(rows, 256)):
@@ -225,6 +235,7 @@ class DDPG(object):
             self.set_flat(which, np.concatenate(chunks))
 
     KERNEL_HIDDEN = 256        # width of the hand-written row / chain / action kernels
+    NATIVE_HIDDEN = (64, 128, 256)   # widths the row / action kernels are instantiated for (pad_hidden='native')
 
     def ref_flat(self, arena, which):
         """The `which` net of an arena-shaped tensor (parameters, gradients, Adam moments) as a device vector in the
@@ -252,11 +263,18 @@ class DDPG(object):
             self._ws[n] = torch.zeros(floats, dtype=torch.float32, device=self.device)     # holds a ticket: zeroed
         return self._ws[n]
 
+    def _rows_shape_ok(self, n):
+        """cur_ddpg_rows_supported for this agent's net and n rows.  The library also takes hidden 64 / 128; an agent
+        runs a net of any width but 256 on the row / action kernels only when it was built with pad_hidden='native'."""
+        if int(self.net.desc.hidden) != self.KERNEL_HIDDEN and self.pad_hidden != 'native':
+            return False
+        return bool(_lib.load().cur_ddpg_rows_supported(C.byref(self.net.desc), n))
+
     def _use_rows(self, n):
         if self.update_schedule == 'levels':
             return False
         lib = _lib.load()
-        ok = bool(lib.cur_ddpg_rows_supported(C.byref(self.net.desc), n))
+        ok = self._rows_shape_ok(n)
         if self.update_schedule == 'rows':
             if not ok:
                 raise ValueError('update_schedule="rows" does not support this network / batch shape')
@@ -461,8 +479,7 @@ class DDPG(object):
 
     def _action_rows_ok(self):
         if self._action_rows is None:
-            self._action_rows = bool(self.action_path != 'levels' and
-                                     _lib.load().cur_ddpg_rows_supported(C.byref(self.net.desc), 4))
+            self._action_rows = bool(self.action_path != 'levels' and self._rows_shape_ok(4))
         return self._action_rows
 
     def _draw_action_noise(self, n, random_eps):
@@ -716,7 +733,7 @@ class DDPG(object):
         lib = _lib.load()
         wide_rows = k * self.batch_size
         self._wide = bool(k > 1 and self.workers_mode != 'micro' and (
-            (self.update_schedule != 'levels' and lib.cur_ddpg_rows_supported(C.byref(self.net.desc), wide_rows)) or
+            (self.update_schedule != 'levels' and self._rows_shape_ok(wide_rows)) or
             lib.cur_ddpg_uses_tensor_cores(C.byref(self.net.desc), wide_rows)))
         self._graph_rows = self.batch_size * (k if self._wide else 1)
         self._micro = 1 if self._wide else k

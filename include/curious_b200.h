@@ -274,7 +274,8 @@ int cur_ddpg_actions(void* stream, const cur_net_desc* d, const float* theta,
                      float* out_pi, float* out_q /* or NULL */);
 
 /* The same forward as ONE launch for the rollout's per-step call (rollout.py:217,226: n = rollout_batch_size rows, 50
- * calls per episode; hidden 256, see cur_ddpg_rows_supported): one CTA per 4 rows streams the net through shared memory.
+ * calls per episode; hidden 64, 128 or 256, see cur_ddpg_rows_supported): one CTA per 4 rows streams the net through
+ * shared memory.
  * Every data pointer may address MAPPED PINNED HOST memory (cur_host_alloc) - inputs are then read and actions written
  * over PCIe by the kernel itself.  seq == 0: out_pi / out_q are float32 arrays.  seq != 0: they are arrays of 8-byte words
  * {float32 bits | seq << 32}; an aligned 64-bit store is single-copy atomic, so a caller that owns the (host-visible)
@@ -375,8 +376,9 @@ int cur_ddpg_grads_group(void* stream, const cur_net_desc* d, int n_experts, con
  * optionally, both MpiAdam.update calls of DDPG._update (ddpg.py:246-248, mpi_adam.py:30-35) in
  * TWO launches: a thread-block-cluster kernel that runs the whole forward / backward data path for
  * 16-row groups of the batch, then one grouped weight-gradient GEMM over the full batch that
- * applies Adam in its epilogue.  Supported shapes: hidden == 256, layers <= 4, dimu <= 8,
- * first-layer fan-in <= 256, batch a multiple of 16 (cur_ddpg_rows_supported); anything else
+ * applies Adam in its epilogue.  Supported shapes: hidden 64, 128 or 256 (the kernels are instantiated
+ * for each; the optional CTA-pair form is 256 only), layers <= 4, dimu <= 8, first-layer fan-in <= 256
+ * whatever the hidden width, batch a multiple of 4 up to 1024 (cur_ddpg_rows_supported); anything else
  * uses cur_ddpg_grads.  Same outputs as cur_ddpg_grads.
  *
  * `workspace` must be ZERO-INITIALISED once by the caller (it holds a completion ticket).
