@@ -34,7 +34,8 @@ struct Workspace {
   float *dcl[CUR_MAX_LAYERS], *dpl[CUR_MAX_LAYERS];   // chain schedule (tc_chain.cu): one delta buffer per layer
   float* chain_loss;                                   // ... and its per-tile loss partials [n / 128][4]
   float* chain_wsplit;                                 // ... the parameters of both arenas as 3xTF32 halves (4 x arena)
-  uint32_t *chain_mp, *chain_mq, *chain_mqp;           // ... ReLU mask words [layers][8][n] (main.pi, main.Q(u), main.Q(pi))
+  uint32_t *chain_mp, *chain_mq, *chain_mqp;           // ... ReLU mask words [layers][H / 32][n] (main.pi, main.Q(u), main.Q(pi))
+  float* chain_dwpart;                                 // ... hidden < 256: K-slice partials of the FFMA weight gradients
   // tensor-core path (large batch only): split-K partial tiles / partial row reductions, TC_SLOTS problems per level
   float *tc_part, *tc_rowpart;
   int64_t tc_part_stride, tc_rowpart_stride;
@@ -71,15 +72,33 @@ static bool use_tc(const cur_net_desc& d, int64_t n) {
 // The fused chain kernel (tc_chain.cu) replaces the forward / loss / dX levels whenever the tensor-core path is on and the
 // shape fits; CUR_DDPG_CHAIN=0 or cur_ddpg_set_chain(0) keeps the level-by-level schedule (A/B measurements, tests).
 static int g_chain_mode = -1;
-static bool use_chain(const cur_net_desc& d, int64_t n) {
-  if (!use_tc(d, n) || !tc_chain_supported(d, n)) return false;
+static bool chain_enabled() {
   if (g_chain_mode >= 0) return g_chain_mode == 1;
   static int v = -1;
   if (v < 0) { const char* e = getenv("CUR_DDPG_CHAIN"); v = (e && e[0] == '0') ? 0 : 1; }
   return v == 1;
 }
+static bool use_chain(const cur_net_desc& d, int64_t n) {
+  if (!use_tc(d, n) || !tc_chain_supported(d, n)) return false;
+  return chain_enabled();
+}
+// Hidden 64 / 128 on the chain kernel (cur_ddpg_chain_grads): the weight gradients are too narrow for the 128 x 256 tile
+// of tc_gemm_kernel and run on the FFMA grouped GEMM, K split into at most this many slices of the batch
+constexpr int CH_DW_MAX_SPLITS = 8;
+static bool narrow_chain_ok(const cur_net_desc& d, int64_t n) {
+  return d.hidden < 256 && tc_chain_width_supported(d, n) && chain_enabled();
+}
+static int64_t chain_dw_floats(const cur_net_desc& d) {     // sum of M x N over the weight gradients of both nets
+  int64_t f = 0;
+  for (int which = 0; which < 2; ++which) {
+    const NetLayout q = net_layout(d, which);
+    f += (int64_t)(d.layers - 1) * d.hidden * d.hidden + (int64_t)(q.in_s + q.in_g) * d.hidden;
+  }
+  return f;
+}
 
-static Workspace carve(const cur_net_desc& d, int64_t n, float* base) {
+// narrow_chain: also carve the chain buffers of a net narrower than 256 (cur_ddpg_chain_workspace_floats)
+static Workspace carve(const cur_net_desc& d, int64_t n, float* base, bool narrow_chain = false) {
   Workspace w;
   const NetLayout q = net_layout(d, 0), p = net_layout(d, 1);
   w.ld_spi = (int)r4(p.in_s);
@@ -124,14 +143,17 @@ static Workspace carve(const cur_net_desc& d, int64_t n, float* base) {
   w.chain_loss = nullptr;
   w.chain_mp = w.chain_mq = w.chain_mqp = nullptr;
   w.chain_wsplit = nullptr;
-  if (tc_chain_supported(d, n)) {
+  w.chain_dwpart = nullptr;
+  const bool narrow = narrow_chain && d.hidden < 256 && tc_chain_width_supported(d, n);
+  if (tc_chain_supported(d, n) || narrow) {
     for (int l = 0; l < d.layers; ++l) { w.dcl[l] = take(n * w.H); w.dpl[l] = take(n * w.H); }
     w.chain_loss = take((n / 128) * 4);
     w.chain_wsplit = take(4 * (r4(q.total) + r4(p.total)));
-    w.chain_mp = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * 8 * n));
-    w.chain_mq = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * 8 * n));
-    w.chain_mqp = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * 8 * n));
+    w.chain_mp = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * (w.H / 32) * n));
+    w.chain_mq = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * (w.H / 32) * n));
+    w.chain_mqp = reinterpret_cast<uint32_t*>(take((int64_t)d.layers * (w.H / 32) * n));
   }
+  if (narrow) w.chain_dwpart = take(CH_DW_MAX_SPLITS * chain_dw_floats(d));
   if (tc_shape_ok(d, n)) {      // carved whenever the shape is eligible: the workspace size does not depend on the toggle
     GemmProb dwp = zero_prob();
     dwp.M = w.H; dwp.N = w.H; dwp.K = (int)n; dwp.a_trans = 1;
@@ -422,6 +444,79 @@ static int grid_prep(int64_t work) {
   return (int)(b < 1 ? 1 : (b > cap ? cap : b));
 }
 
+// ------------------------------------------------------------------------------------------------
+// Weight gradients of the chain schedule at hidden 64 / 128: dW = X^T dY (K = batch) as FFMA grouped-GEMM tiles over K
+// slices of the batch, each slice into its own partial block, then the slices summed in slice order (deterministic).
+// Without the split the few 32 x 32 tiles of H-wide gradients (4 per hidden layer at H = 64) occupy a handful of SMs for
+// the whole batch.
+// ------------------------------------------------------------------------------------------------
+struct DwSliceSum {
+  const float* part;        // [splits][count]
+  float* out;               // [count]
+  int64_t count;
+  int splits;
+};
+struct DwSliceSumBatch {
+  DwSliceSum p[2 * (CUR_MAX_LAYERS + 1)];
+  int n;
+};
+__global__ void __launch_bounds__(256) dw_slice_sum_kernel(const __grid_constant__ DwSliceSumBatch R) {
+  for (int i = 0; i < R.n; ++i) {
+    const DwSliceSum& P = R.p[i];
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < P.count; e += (int64_t)gridDim.x * blockDim.x) {
+      float v = P.part[e];
+      for (int s = 1; s < P.splits; ++s) v += P.part[(int64_t)s * P.count + e];
+      P.out[e] = v;
+    }
+  }
+}
+
+// probs: dW problems with contiguous outputs (ldc == N), K = n, B K-major [N][n]; A K-major [M][n] (a_trans 0) or the
+// input matrix [n][lda] (a_trans 1).  part: CH_DW_MAX_SPLITS x (sum of M x N) floats.
+static int chain_dw_ffma(cudaStream_t s, const GemmProb* probs, int np, int64_t n, float* part) {
+  CUR_REQUIRE(np <= 2 * (CUR_MAX_LAYERS + 1) && part != nullptr, "bad weight-gradient list");
+  int tiles = 0;
+  for (int i = 0; i < np; ++i) tiles += ((probs[i].M + GT - 1) / GT) * ((probs[i].N + GT - 1) / GT);
+  // enough slices for two CTAs per SM (the grouped GEMM's occupancy), each at least 256 rows, in whole GK chunks
+  int splits = (2 * sm_count() + tiles - 1) / (tiles > 0 ? tiles : 1);
+  if (splits > CH_DW_MAX_SPLITS) splits = CH_DW_MAX_SPLITS;
+  if (splits > n / 256) splits = (int)(n / 256);
+  if (splits < 1) splits = 1;
+  const int64_t ks = ((n + splits - 1) / splits + GK - 1) / GK * GK;
+  splits = (int)((n + ks - 1) / ks);
+  GemmBatch G;
+  G.n = 0; G.total_tiles = 0;
+  DwSliceSumBatch R;
+  R.n = 0;
+  float* pp = part;
+  for (int i = 0; i < np; ++i) {
+    const GemmProb& q = probs[i];
+    CUR_REQUIRE(q.ldc == q.N && q.b_trans == 1 && q.K == n, "bad weight-gradient problem");
+    const int64_t count = (int64_t)q.M * q.N;
+    for (int sl = 0; sl < splits; ++sl) {
+      const int64_t k0 = sl * ks;
+      GemmProb p = q;
+      p.split_k = 0;
+      p.K = (int)(k0 + ks <= n ? ks : n - k0);
+      p.A = q.a_trans ? q.A + k0 * q.lda : q.A + k0;
+      p.B = q.B + k0;
+      p.C = pp + sl * count;
+      G.p[G.n++] = p;
+      if (G.n == GEMM_MAX_PROBS) {
+        CUR_TRY(launch_gemm_batch(G, s));
+        G.n = 0;
+      }
+    }
+    DwSliceSum& r = R.p[R.n++];
+    r.part = pp; r.out = q.C; r.count = count; r.splits = splits;
+    pp += splits * count;
+  }
+  if (G.n > 0) CUR_TRY(launch_gemm_batch(G, s));
+  dw_slice_sum_kernel<<<2 * sm_count(), 256, 0, s>>>(R);
+  CUR_CHECK_LAUNCH();
+  return CUR_OK;
+}
+
 }  // namespace cur
 
 using namespace cur;
@@ -562,11 +657,13 @@ struct GroupBatcher {
 
 // DDPG._grads for n_e experts of identical shape: every dependency level is ONE launch (per kernel kind) over all
 // experts - the grouped-GEMM form of structure='task_experts' (train.py:287-289 builds one DDPG per module).
-static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_e, int64_t n) {
+// narrow_chain: one agent of hidden 64 / 128 on the chain schedule (cur_ddpg_chain_grads)
+static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_e, int64_t n, bool narrow_chain = false) {
   const NetLayout LQ = net_layout(*d, 0), LP = net_layout(*d, 1);
   const int L = d->layers, H = d->hidden;
+  const bool chain = narrow_chain || use_chain(*d, n);
   // ---- chain schedule, one agent: the 3xTF32 weight halves are split on a side stream beside the input preparation
-  if (n_e == 1 && use_chain(*d, n))
+  if (n_e == 1 && chain)
     CUR_TRY(tc_chain_presplit_async(s, E[0].mQ, E[0].tQ, E[0].w.chain_wsplit, r4(LQ.total) + r4(LP.total)));
   // ---- inputs
   for (int i = 0; i < n_e; ++i) {
@@ -587,9 +684,14 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
   GroupBatcher B(s, use_tc(*d, n), E, n_e);
 #define FOR_EXPERTS for (int i = 0; i < n_e; ++i)
 #define ADD(prob) CUR_TRY(B.add(i, (prob)))
-  if (use_chain(*d, n)) {
+  if (chain) {
     // ---- chain schedule (tc_chain.cu): forward nets, losses and the data-gradient chains of a 128-row tile in one
     // CTA per chain, then every weight / bias gradient as split-K tensor-core GEMMs + row reductions, one level per net
+    // (hidden 64 / 128: the weight gradients as K-sliced FFMA GEMMs, chain_dw_ffma)
+    CUR_REQUIRE(!narrow_chain || n_e == 1, "the narrow chain schedule runs one agent");
+    GemmProb dw_ffma[2 * (CUR_MAX_LAYERS + 1)];
+    int n_dw_ffma = 0;
+#define ADD_DW(prob) do { if (narrow_chain) dw_ffma[n_dw_ffma++] = (prob); else ADD(prob); } while (0)
     if (n_e > 1) CUR_TRY(tc_chain_lanes_fork(s));
     FOR_EXPERTS {
       Expert& x = E[i]; const Workspace& w = x.w;
@@ -599,7 +701,7 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
       io.mQ = x.mQ; io.mP = x.mP; io.tQ = x.tQ; io.tP = x.tP;
       io.Xpi = w.Xpi; io.Xg = w.Xg; io.XQu = w.XQu; io.Xpi_t = w.Xpi_t; io.Xg_t = w.Xg_t; io.XQpi = w.XQpi; io.XQ_t = w.XQ_t;
       io.ld_spi = w.ld_spi; io.ld_sq = w.ld_sq; io.ld_g = w.ld_g; io.lddy = (int)r4(d->dimu);
-      // (the chain keeps hp / hq / dcl / dpl TRANSPOSED, [256][n]: K-major operands of the weight-gradient GEMMs)
+      // (the chain keeps hp / hq / dcl / dpl TRANSPOSED, [H][n]: K-major operands of the weight-gradient GEMMs)
       for (int l = 0; l < L; ++l) { io.hp[l] = w.hp[l]; io.hq[l] = w.hq[l]; io.dc[l] = w.dcl[l]; io.dp[l] = w.dpl[l]; }
       io.mp = w.chain_mp; io.mq = w.chain_mq; io.mqp = w.chain_mqp; io.wsplit = w.chain_wsplit;
       io.Q = w.Q; io.Qt = w.Qt; io.dQ = w.dQ; io.dy = w.dy; io.q_pi = x.q_pi; io.r = x.batch->r;
@@ -613,7 +715,7 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
     }
     if (n_e > 1) CUR_TRY(tc_chain_lanes_join(s));
     const int lddy = (int)r4(d->dimu);
-    // dW = X^T dY with both operands K-major (K = batch): A = hT [256][n], B = dT [256][n]; first layers: A = X [n][in]
+    // dW = X^T dY with both operands K-major (K = batch): A = hT [H][n], B = dT [H][n]; first layers: A = X [n][in]
     auto dw_t = [&](const float* XT, int m_rows, const float* DT, float* dW) {
       GemmProb p = zero_prob();
       p.A = XT; p.lda = (int)n; p.a_trans = 0; p.K = (int)n; p.split_k = 2;
@@ -640,24 +742,26 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
       rowsum(w.hq[L - 1], H, w.dQ, 1, 1, x.gQ + LQ.off_Wout);                  // dWout = h^T dQ
       rowsum(nullptr, 1, w.dQ, 1, 1, x.gQ + LQ.off_bout);                      // dbout = sum dQ
       for (int l = L - 1; l >= 1; --l) {
-        ADD(dw_t(w.hq[l - 1], H, w.dcl[l], x.gQ + LQ.off_W[l]));
+        ADD_DW(dw_t(w.hq[l - 1], H, w.dcl[l], x.gQ + LQ.off_W[l]));
         rowsum(w.dcl[l], H, nullptr, 0, 1, x.gQ + LQ.off_b[l]);
       }
-      ADD(dw_x(w.XQu, w.ld_sq, LQ.in_s, w.dcl[0], x.gQ + LQ.off_W0));
+      ADD_DW(dw_x(w.XQu, w.ld_sq, LQ.in_s, w.dcl[0], x.gQ + LQ.off_W0));
       rowsum(w.dcl[0], H, nullptr, 0, 1, x.gQ + LQ.off_b0);
-      if (LQ.in_g > 0) ADD(dw_x(w.Xg, w.ld_g, LQ.in_g, w.dcl[0], x.gQ + LQ.off_W0g));
+      if (LQ.in_g > 0) ADD_DW(dw_x(w.Xg, w.ld_g, LQ.in_g, w.dcl[0], x.gQ + LQ.off_W0g));
       // main.pi from the actor chain
       rowsum(w.hp[L - 1], H, w.dy, lddy, d->dimu, x.gP + LP.off_Wout);
       rowsum(nullptr, 1, w.dy, lddy, d->dimu, x.gP + LP.off_bout);
       for (int l = L - 1; l >= 1; --l) {
-        ADD(dw_t(w.hp[l - 1], H, w.dpl[l], x.gP + LP.off_W[l]));
+        ADD_DW(dw_t(w.hp[l - 1], H, w.dpl[l], x.gP + LP.off_W[l]));
         rowsum(w.dpl[l], H, nullptr, 0, 1, x.gP + LP.off_b[l]);
       }
-      ADD(dw_x(w.Xpi, w.ld_spi, LP.in_s, w.dpl[0], x.gP + LP.off_W0));
+      ADD_DW(dw_x(w.Xpi, w.ld_spi, LP.in_s, w.dpl[0], x.gP + LP.off_W0));
       rowsum(w.dpl[0], H, nullptr, 0, 1, x.gP + LP.off_b0);
-      if (LP.in_g > 0) ADD(dw_x(w.Xg, w.ld_g, LP.in_g, w.dpl[0], x.gP + LP.off_W0g));
+      if (LP.in_g > 0) ADD_DW(dw_x(w.Xg, w.ld_g, LP.in_g, w.dpl[0], x.gP + LP.off_W0g));
       CUR_TRY(tc_chain_rowsums(s, RS));             // side stream: next to the GEMM launches
     }
+#undef ADD_DW
+    if (narrow_chain) CUR_TRY(chain_dw_ffma(s, dw_ffma, n_dw_ffma, n, E[0].w.chain_dwpart));
     CUR_TRY(B.flush());                             // (the batcher also flushes whenever a launch is full)
     CUR_TRY(B.B.T.finish(s));
     CUR_TRY(tc_chain_join(s));
@@ -799,7 +903,7 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
 
 static int fill_expert(Expert& x, const cur_net_desc* d, const float* theta_main, const float* theta_target,
                        const cur_norm_stats* stats, const cur_batch* batch, const cur_ddpg_hyper* h, float* workspace,
-                       float* grads, float* q_loss, float* pi_loss, float* q_pi) {
+                       float* grads, float* q_loss, float* pi_loss, float* q_pi, bool narrow_chain = false) {
   CUR_REQUIRE(theta_main && theta_target && batch && h && workspace && grads && q_pi, "NULL argument");
   CUR_REQUIRE(batch->o && batch->g && batch->u && batch->o_2 && batch->g_2 && batch->r, "NULL batch array");
   CUR_REQUIRE(!d->modular || batch->td, "task_descr required for a modular net");
@@ -807,7 +911,7 @@ static int fill_expert(Expert& x, const cur_net_desc* d, const float* theta_main
   if (d->normalize_obs)
     CUR_REQUIRE(stats && stats->o_mean && stats->o_std && stats->g_mean && stats->g_std, "normalizer stats required");
   const int64_t offP = r4(net_layout(*d, 0).total);
-  x.w = carve(*d, batch->n, workspace);
+  x.w = carve(*d, batch->n, workspace, narrow_chain);
   x.mQ = theta_main; x.mP = theta_main + offP; x.tQ = theta_target; x.tP = theta_target + offP;
   x.gQ = grads; x.gP = grads + offP;
   x.batch = batch; x.stats = stats; x.h = h; x.q_loss = q_loss; x.pi_loss = pi_loss; x.q_pi = q_pi;
@@ -836,4 +940,26 @@ extern "C" int cur_ddpg_grads_group(void* stream, const cur_net_desc* d, int n_e
                         a.workspace, a.grads, a.q_loss, a.pi_loss, a.q_pi));
   }
   return grads_levels((cudaStream_t)stream, d, E, n_experts, experts[0].batch.n);
+}
+
+extern "C" int cur_ddpg_chain_supported(const cur_net_desc* d, int64_t batch) {
+  if (check_desc(d) != CUR_OK || batch <= 0) return 0;
+  if (d->hidden == 256) return use_chain(*d, batch) ? 1 : 0;
+  return narrow_chain_ok(*d, batch) ? 1 : 0;
+}
+
+extern "C" int64_t cur_ddpg_chain_workspace_floats(const cur_net_desc* d, int64_t batch) {
+  if (check_desc(d) != CUR_OK || batch <= 0) return -1;
+  return carve(*d, batch, nullptr, true).total;
+}
+
+extern "C" int cur_ddpg_chain_grads(void* stream, const cur_net_desc* d, const float* theta_main,
+                                    const float* theta_target, const cur_norm_stats* stats, const cur_batch* batch,
+                                    const cur_ddpg_hyper* h, float* workspace, float* grads, float* q_loss,
+                                    float* pi_loss, float* q_pi) {
+  CUR_TRY(check_desc(d));
+  CUR_REQUIRE(batch != nullptr && cur_ddpg_chain_supported(d, batch->n), "shape not taken by the chain schedule");
+  Expert x;
+  CUR_TRY(fill_expert(x, d, theta_main, theta_target, stats, batch, h, workspace, grads, q_loss, pi_loss, q_pi, true));
+  return grads_levels((cudaStream_t)stream, d, &x, 1, batch->n, d->hidden < 256);
 }

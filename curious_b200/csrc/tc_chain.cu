@@ -7,7 +7,8 @@
 //   baselines/her/actor_critic.py:5-98, util.py:56-107   networks (forward)
 //   baselines/her/ddpg.py:412-449                        losses + the data-gradient half of tf.gradients
 // The weight gradients (dW = X^T dY, K = batch) follow as split-K tcgen05 GEMMs (tc_gemm.cu) on the activations /
-// deltas this kernel leaves in the workspace.
+// deltas this kernel leaves in the workspace; at hidden 64 / 128 (the kernel is a template on the width H, every `256`
+// below reads H) as K-sliced FFMA grouped GEMMs (ddpg.cu: chain_dw_ffma).
 //
 // Why: rows of the batch are independent until dW (the insight behind the rows schedule, ddpg_rows.cu), but that
 // schedule re-streams all weights per 4 rows (cost grows linearly with the rows), and the dependency-level schedule
@@ -46,19 +47,25 @@
 
 namespace cur {
 
-constexpr int CH_BM = 128, CH_BN = 256, CH_BK = 32;
+// The hidden width H (64, 128 or 256) is the N of every tcgen05.mma and a template parameter of the kernel and of the
+// feeder helpers; everything else (128 rows per CTA, the rings, the warp roles, 3xTF32) is the same at every width.
+constexpr int CH_BM = 128, CH_BK = 32;
 constexpr int CH_A_HALF = CH_BM * CH_BK * 4;              // 16 KB: one k-block of the A operand (hi or lo)
-constexpr int CH_B_HALF = CH_BN * CH_BK * 4;              // 32 KB
 constexpr int CH_A_STAGE = 2 * CH_A_HALF;                 // hi | lo
-constexpr int CH_B_STAGE = 2 * CH_B_HALF;                 // hi | lo
-constexpr int CH_NA = 2, CH_NB = 2;                       // ring depths: 64 KB + 128 KB (A: one stage per feeder parity)
+constexpr int CH_NA = 2, CH_NB = 2;                       // ring depths: 64 KB + 2 x 2 x 16 H bytes (A: one stage per feeder parity)
 constexpr int CH_MNBLK = 32 * 128;                        // bytes of one 32-wide N block of an MN-major weight tile
 constexpr int CH_WARP_FEED0 = 2, CH_FEED_WARPS = 8;
 constexpr int CH_THREADS = (CH_WARP_FEED0 + CH_FEED_WARPS) * 32;     // 320
-constexpr size_t CH_SMEM_BYTES = (size_t)CH_NA * CH_A_STAGE + (size_t)CH_NB * CH_B_STAGE + 1024 /* alignment */ + 256;
 constexpr int CH_MAX_GEMM = 16, CH_MAX_MAPS = 40;         // (hi, lo) map pairs
-constexpr int CH_NCH = CH_BN / 32;                        // 32-column chunks of a layer output
-constexpr int CH_VEC_FLOATS = 3 * 4 * CH_BN + 2 * 4 * CH_BN + 2 * CH_BN;   // 3 nets x <= 4 biases, 2 x [256][4], 2 x [256]
+template <int H>
+struct ChW {
+  static_assert(H == 64 || H == 128 || H == 256, "hidden widths of the chain kernel");
+  static constexpr int B_HALF = H * CH_BK * 4;            // one k-block of the B operand (hi or lo): 32 x H
+  static constexpr int B_STAGE = 2 * B_HALF;              // hi | lo
+  static constexpr size_t SMEM_BYTES = (size_t)CH_NA * CH_A_STAGE + (size_t)CH_NB * B_STAGE + 1024 /* alignment */ + 256;
+  static constexpr int NCH = H / 32;                      // 32-column chunks of a layer output
+  static constexpr int VEC_FLOATS = 3 * 4 * H + 2 * 4 * H + 2 * H;   // 3 nets x <= 4 biases, 2 x [H][4], 2 x [H]
+};
 
 struct ChGemm {
   int map1, nkb1, map2, nkb2;     // weight tensor maps (hi; lo = + 1) of the (up to two) K segments, their k-block counts
@@ -78,10 +85,10 @@ struct __align__(64) ChainParams {
   const float *Xpi, *Xg, *XQu, *XQpi, *Xpi_t, *Xg_t, *XQ_t;
   const float *bP[CUR_MAX_LAYERS], *bPT[CUR_MAX_LAYERS], *bQ[CUR_MAX_LAYERS], *bQT[CUR_MAX_LAYERS];
   const float *WoutP, *boutP, *WoutPT, *boutPT, *WoutQ, *boutQ, *WoutQT, *boutQT;
-  const float* W0Q_act;           // main.Q first-layer rows of the action inputs: [dimu][256]
-  // transposed copies [256][n] for the weight-gradient GEMMs: activations (hp, hq) and deltas (dc, dp)
+  const float* W0Q_act;           // main.Q first-layer rows of the action inputs: [dimu][H]
+  // transposed copies [H][n] for the weight-gradient GEMMs: activations (hp, hq) and deltas (dc, dp)
   float *hp[CUR_MAX_LAYERS], *hq[CUR_MAX_LAYERS], *dc[CUR_MAX_LAYERS], *dp[CUR_MAX_LAYERS];
-  // ReLU masks [layer][chunk][n], bit i of a word = unit 32 chunk + i is active
+  // ReLU masks [layer][chunk][n] (H / 32 chunks), bit i of a word = unit 32 chunk + i is active
   uint32_t *mp, *mq, *mqp;
   float *Q, *Qt, *dQ, *dy, *q_pi;
   const float* r;
@@ -111,10 +118,11 @@ struct Feeder {
     tc_bar_wait(acc_full + 8 * (g & 1), (uint32_t)(g >> 1) & 1u);
     tc_fence_after();
   }
-  // 32 accumulator columns of GEMM g, chunk c, for this thread's row
+  // 32 accumulator columns of GEMM g, chunk c, for this thread's row (accumulators g & 1 = 0 / 1 at columns 0 / H)
+  template <int H>
   __device__ __forceinline__ void ld_chunk(int g, int c, float (&v)[32]) const {
     uint32_t x[32];
-    tc_ld32(tmem_lane + (uint32_t)((g & 1) * CH_BN + c * 32), x);
+    tc_ld32(tmem_lane + (uint32_t)((g & 1) * H + c * 32), x);
     tc_ld_wait();
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(x[i]);
@@ -208,15 +216,16 @@ __device__ __forceinline__ void ch_feed_x(Feeder& F, const float* X, int ld, int
 }
 
 // Forward hidden layer boundary: h = relu(acc(g) + bias) -> mask word, optional transposed copy -> A operand of the next GEMM
+template <int H>
 __device__ __forceinline__ void ch_feed_relu(Feeder& F, int g, const float* bias, float* HT, uint32_t* mask,
                                              int64_t n) {
   F.wait_acc(g);
 #pragma unroll 1
-  for (int c = 0; c < CH_NCH; ++c) {
+  for (int c = 0; c < ChW<H>::NCH; ++c) {
     if (!F.mine()) { ++F.a_cnt; continue; }
     float v[32], b[32];
     ch_load32(bias + 32 * c, b);
-    F.ld_chunk(g, c, v);
+    F.ld_chunk<H>(g, c, v);
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i] + b[i], 0.f);
     if (mask) mask[(int64_t)c * n + F.row] = ch_mask_word(v);
@@ -227,17 +236,17 @@ __device__ __forceinline__ void ch_feed_relu(Feeder& F, int g, const float* bias
 
 // Output layer on the last hidden activation: h = relu(acc(g) + bias) (mask word, optional transposed copy),
 // out[j] = sum_c h[c] Wout[c][j] (the chunks of this warp's parity, then combined over the warp pair)
-template <int NJMAX>
+template <int H, int NJMAX>
 __device__ __forceinline__ void ch_out_layer(Feeder& F, int g, const float* bias, float* HT, uint32_t* mask,
                                              int64_t n, const float* Wout, int nj, float (&out)[NJMAX]) {
 #pragma unroll
   for (int j = 0; j < NJMAX; ++j) out[j] = 0.f;
   F.wait_acc(g);
 #pragma unroll 1
-  for (int c = F.par; c < CH_NCH; c += 2) {
+  for (int c = F.par; c < ChW<H>::NCH; c += 2) {
     float v[32], b[32];
     ch_load32(bias + 32 * c, b);
-    F.ld_chunk(g, c, v);
+    F.ld_chunk<H>(g, c, v);
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i] + b[i], 0.f);
     if (mask) mask[(int64_t)c * n + F.row] = ch_mask_word(v);
@@ -268,11 +277,11 @@ __device__ __forceinline__ void ch_out_layer(Feeder& F, int g, const float* bias
 
 // Backward seed through an output layer: d[c] = (sum_j dout[j] Wout[c][j]) where the mask word says the unit is active
 // -> optional transposed copy -> A
-template <int NJMAX>
+template <int H, int NJMAX>
 __device__ __forceinline__ void ch_seed(Feeder& F, const float (&dout)[NJMAX], int nj, const float* Wout,
                                         const uint32_t* mask, float* DT, int64_t n) {
 #pragma unroll 1
-  for (int c = 0; c < CH_NCH; ++c) {
+  for (int c = 0; c < ChW<H>::NCH; ++c) {
     if (!F.mine()) { ++F.a_cnt; continue; }
     float v[32];
     const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : mask[(int64_t)c * n + F.row];
@@ -305,17 +314,18 @@ __device__ __forceinline__ void ch_seed(Feeder& F, const float (&dout)[NJMAX], i
 
 // Backward hidden layer boundary: d = acc(g) where the mask word says the unit was active -> optional transposed copy ->
 // (optionally) A of the next GEMM
+template <int H>
 __device__ __forceinline__ void ch_feed_mask(Feeder& F, int g, const uint32_t* mask, float* DT, int64_t n, bool push) {
   F.wait_acc(g);
 #pragma unroll 1
-  for (int c = 0; c < CH_NCH; ++c) {
+  for (int c = 0; c < ChW<H>::NCH; ++c) {
     if (push ? !F.mine() : ((c & 1) != F.par)) {
       if (push) ++F.a_cnt;
       continue;
     }
     float v[32];
     const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : mask[(int64_t)c * n + F.row];
-    F.ld_chunk(g, c, v);
+    F.ld_chunk<H>(g, c, v);
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = ((mw >> i) & 1u) ? v[i] : 0.f;
     if (DT && !(F.dbg & 1)) ch_store_t(DT, n, F.row, c, v);
@@ -334,12 +344,14 @@ __device__ __forceinline__ float ch_tile_sum(float x, float* s_red, int fw, int 
   return (s_red[0] + s_red[1]) + (s_red[2] + s_red[3]);
 }
 
+template <int H>
 __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_constant__ ChainParams P) {
+  using W = ChW<H>;
   extern __shared__ uint8_t ch_smem_raw[];
   __shared__ uint32_t s_tmem;
   __shared__ float s_red[4];
   __shared__ float s_x[CH_BM][4];
-  __shared__ __align__(16) float s_vec[CH_VEC_FLOATS];   // biases / output-layer weights of this chain (see `stage`)
+  __shared__ __align__(16) float s_vec[W::VEC_FLOATS];   // biases / output-layer weights of this chain (see `stage`)
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int role = blockIdx.x & 1;                      // 0: actor chain, 1: critic chain
   const int tile = blockIdx.x >> 1;
@@ -350,7 +362,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
   const uint32_t base = (tc_smem(ch_smem_raw) + 1023u) & ~1023u;
   uint8_t* gen_base = ch_smem_raw + (base - tc_smem(ch_smem_raw));
   const uint32_t a_ring = base, b_ring = base + CH_NA * CH_A_STAGE;
-  const uint32_t bars = b_ring + CH_NB * CH_B_STAGE;
+  const uint32_t bars = b_ring + CH_NB * W::B_STAGE;
   const uint32_t a_full = bars, a_empty = bars + 8 * CH_NA, b_full = bars + 16 * CH_NA, b_empty = b_full + 8 * CH_NB,
                  acc_full = b_full + 16 * CH_NB;
   long long* tl = (P.tl != nullptr && tile == 0 && lane == 0) ? P.tl + 512 * role : nullptr;   // [role][512] stamps
@@ -363,7 +375,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem(&s_tmem)), "n"(512) : "memory");
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem(&s_tmem)), "n"(2 * H) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
@@ -381,21 +393,21 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
         for (int kb = 0; kb < nkb; ++kb, ++cnt) {
           const int s = cnt % CH_NB, round = cnt / CH_NB;
           if (round > 0) tc_bar_wait(b_empty + 8 * s, (uint32_t)(round - 1) & 1u);
-          const uint32_t dst = b_ring + s * CH_B_STAGE;
+          const uint32_t dst = b_ring + s * W::B_STAGE;
           const bool seg2 = kb >= G.nkb1;
           const CUtensorMap* mh = &P.maps[role][seg2 ? G.map2 : G.map1];
           const CUtensorMap* ml = mh + 1;
           const int k0 = (seg2 ? kb - G.nkb1 : kb) * CH_BK;
           if (tl && cnt < 88) tl[288 + cnt] = clock64();
-          tc_bar_expect_tx(b_full + 8 * s, CH_B_STAGE);                // zero-filled out-of-bounds rows count too
+          tc_bar_expect_tx(b_full + 8 * s, W::B_STAGE);                // zero-filled out-of-bounds rows count too
           if (G.b_mn) {
-            for (int j = 0; j < CH_BN / 32; ++j) {                                                             // [32 k][32 n]
+            for (int j = 0; j < H / 32; ++j) {                                                                 // [32 k][32 n]
               tc_tma_2d(dst + j * CH_MNBLK, mh, 32 * j, k0, b_full + 8 * s);
-              tc_tma_2d(dst + CH_B_HALF + j * CH_MNBLK, ml, 32 * j, k0, b_full + 8 * s);
+              tc_tma_2d(dst + W::B_HALF + j * CH_MNBLK, ml, 32 * j, k0, b_full + 8 * s);
             }
           } else {
-            tc_tma_2d(dst, mh, k0, 0, b_full + 8 * s);                                                         // [256 n][32 k]
-            tc_tma_2d(dst + CH_B_HALF, ml, k0, 0, b_full + 8 * s);
+            tc_tma_2d(dst, mh, k0, 0, b_full + 8 * s);                                                         // [H n][32 k]
+            tc_tma_2d(dst + W::B_HALF, ml, k0, 0, b_full + 8 * s);
           }
         }
       }
@@ -406,11 +418,11 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
     for (int g = 0; g < prog.n; ++g) {
       const ChGemm G = prog.g[g];
       const int nkb = G.nkb1 + G.nkb2;
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)G.b_mn << 16) | ((uint32_t)(CH_BN >> 3) << 17) |
+      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)G.b_mn << 16) | ((uint32_t)(H >> 3) << 17) |
                              ((uint32_t)(CH_BM >> 4) << 24);
       const uint32_t b_step = G.b_mn ? 1024u : 32u, b_lbo = G.b_mn ? (uint32_t)CH_MNBLK : 16u, b_sbo = G.b_mn ? 512u : 1024u,
                      b_lt = G.b_mn ? 1u : 2u;
-      const uint32_t acc = tmem + (uint32_t)((g & 1) * CH_BN);
+      const uint32_t acc = tmem + (uint32_t)((g & 1) * H);
       for (int kb = 0; kb < nkb; ++kb, ++cnt) {
         const int sa = cnt % CH_NA, ra = cnt / CH_NA, sb = cnt % CH_NB, rb = cnt / CH_NB;
         tc_bar_wait(b_full + 8 * sb, (uint32_t)rb & 1u);
@@ -419,7 +431,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
         if (lane == 0) {
           if (tl && cnt < 88) tl[8 + cnt] = clock64();
           const uint32_t a_hi = a_ring + sa * CH_A_STAGE, a_lo = a_hi + CH_A_HALF;
-          const uint32_t b_hi = b_ring + sb * CH_B_STAGE, b_lo = b_hi + CH_B_HALF;
+          const uint32_t b_hi = b_ring + sb * W::B_STAGE, b_lo = b_hi + W::B_HALF;
 #pragma unroll
           for (int ks = 0; ks < CH_BK / 8; ++ks) {
             const uint64_t dah = tc_desc(a_hi + ks * 32, 16u, 1024u, 2u), dal = tc_desc(a_lo + ks * 32, 16u, 1024u, 2u);
@@ -455,7 +467,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
     const bool lead = F.par == 0;                         // the warp of a pair that writes the per-row results
     const float inv_n = 1.0f / (float)P.grad_rows;
     const float none[4] = {0.f, 0.f, 0.f, 0.f};
-#define MW(l) ((int64_t)(l) * CH_NCH * n)            /* mask words of layer l */
+#define MW(l) ((int64_t)(l) * W::NCH * n)            /* mask words of layer l */
     int g = 0;                                            // index of the GEMM whose accumulator is read next
     // The small vectors every row needs (biases, output-layer weights) go to shared memory once: read from global per
     // chunk they cost an exposed L2 round trip each (measured 0.6 - 1.5 k cycles per chunk in the output-layer passes).
@@ -472,15 +484,15 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
       // ---------------- actor chain: main.pi (the first A operand goes out before anything else: the tensor pipe starts)
       ch_feed_x(F, P.Xpi, P.ld_spi, P.in_sp, 0, 0, none);
       if (P.in_g > 0) ch_feed_x(F, P.Xg, P.ld_g, P.in_g, 0, 0, none);
-      for (int l = 0; l < L; ++l) sbA[l] = stage(P.bP[l], CH_BN);
-      const float* sWoutP = stage(P.WoutP, CH_BN * d.dimu);
-      for (int l = 0; l < L; ++l) sbB[l] = stage(P.bQ[l], CH_BN);
-      const float* sWoutQ = stage(P.WoutQ, CH_BN);
-      const float* sW0act = stage(P.W0Q_act, d.dimu * CH_BN);
+      for (int l = 0; l < L; ++l) sbA[l] = stage(P.bP[l], H);
+      const float* sWoutP = stage(P.WoutP, H * d.dimu);
+      for (int l = 0; l < L; ++l) sbB[l] = stage(P.bQ[l], H);
+      const float* sWoutQ = stage(P.WoutQ, H);
+      const float* sW0act = stage(P.W0Q_act, d.dimu * H);
       asm volatile("bar.sync 3, 256;" ::: "memory");
-      for (int l = 1; l < L; ++l, ++g) ch_feed_relu(F, g, sbA[l - 1], P.hp[l - 1], P.mp + MW(l - 1), n);
+      for (int l = 1; l < L; ++l, ++g) ch_feed_relu<H>(F, g, sbA[l - 1], P.hp[l - 1], P.mp + MW(l - 1), n);
       float th[4];
-      ch_out_layer<4>(F, g, sbA[L - 1], P.hp[L - 1], P.mp + MW(L - 1), n, sWoutP, d.dimu, th);
+      ch_out_layer<H, 4>(F, g, sbA[L - 1], P.hp[L - 1], P.mp + MW(L - 1), n, sWoutP, d.dimu, th);
       ++g;
       float sth = 0.f;
 #pragma unroll
@@ -491,9 +503,9 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
       // ---------------- main.Q(o, g, pi): the action columns of the input come from `th`
       ch_feed_x(F, P.XQpi, P.ld_sq, P.in_sq, P.in_sp, d.dimu, th);
       if (P.in_g > 0) ch_feed_x(F, P.Xg, P.ld_g, P.in_g, 0, 0, none);
-      for (int l = 1; l < L; ++l, ++g) ch_feed_relu(F, g, sbB[l - 1], nullptr, P.mqp + MW(l - 1), n);
+      for (int l = 1; l < L; ++l, ++g) ch_feed_relu<H>(F, g, sbB[l - 1], nullptr, P.mqp + MW(l - 1), n);
       float qv[1];
-      ch_out_layer<1>(F, g, sbB[L - 1], nullptr, P.mqp + MW(L - 1), n, sWoutQ, 1, qv);
+      ch_out_layer<H, 1>(F, g, sbB[L - 1], nullptr, P.mqp + MW(L - 1), n, sWoutQ, 1, qv);
       ++g;
       const float q_pi = qv[0] + __ldg(P.boutQ);
       if (lead) {
@@ -506,24 +518,24 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
       // ---------------- backward through main.Q (actor-through-critic chain, data gradients only)
       {
         float dq[1] = {-inv_n};                                            // d(-mean(Q_pi)) / dQ_pi
-        ch_seed<1>(F, dq, 1, sWoutQ, P.mqp + MW(L - 1), nullptr, n);
+        ch_seed<H, 1>(F, dq, 1, sWoutQ, P.mqp + MW(L - 1), nullptr, n);
       }
-      for (int l = L - 1; l >= 2; --l, ++g) ch_feed_mask(F, g, P.mqp + MW(l - 1), nullptr, n, true);
+      for (int l = L - 1; l >= 2; --l, ++g) ch_feed_mask<H>(F, g, P.mqp + MW(l - 1), nullptr, n, true);
       // gradient wrt the action inputs: d h0 (masked) . W0[action rows]^T, then through tanh and the action penalty
       float dy[4] = {0.f, 0.f, 0.f, 0.f};
       F.wait_acc(g);
 #pragma unroll 1
-      for (int c = F.par; c < CH_NCH; c += 2) {
+      for (int c = F.par; c < ChW<H>::NCH; c += 2) {
         float v[32];
         const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : P.mqp[(int64_t)c * n + row];
-        F.ld_chunk(g, c, v);
+        F.ld_chunk<H>(g, c, v);
 #pragma unroll
         for (int i = 0; i < 32; ++i) v[i] = ((mw >> i) & 1u) ? v[i] : 0.f;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           if (j < d.dimu) {
             float w[32];
-            ch_load32(sW0act + j * CH_BN + 32 * c, w);
+            ch_load32(sW0act + j * H + 32 * c, w);
 #pragma unroll
             for (int i = 0; i < 32; ++i) dy[j] = fmaf(v[i], w[i], dy[j]);
           }
@@ -540,39 +552,39 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
         }
       }
       // ---------------- backward through main.pi
-      ch_seed<4>(F, dy, d.dimu, sWoutP, P.mp + MW(L - 1), P.dp[L - 1], n);
-      for (int l = L - 1; l >= 1; --l, ++g) ch_feed_mask(F, g, P.mp + MW(l - 1), P.dp[l - 1], n, l >= 2);
+      ch_seed<H, 4>(F, dy, d.dimu, sWoutP, P.mp + MW(L - 1), P.dp[L - 1], n);
+      for (int l = L - 1; l >= 1; --l, ++g) ch_feed_mask<H>(F, g, P.mp + MW(l - 1), P.dp[l - 1], n, l >= 2);
     } else {
       // ---------------- critic chain: target.pi
       ch_feed_x(F, P.Xpi_t, P.ld_spi, P.in_sp, 0, 0, none);
       if (P.in_g > 0) ch_feed_x(F, P.Xg_t, P.ld_g, P.in_g, 0, 0, none);
-      for (int l = 0; l < L; ++l) sbA[l] = stage(P.bPT[l], CH_BN);
-      const float* sWoutPT = stage(P.WoutPT, CH_BN * d.dimu);
-      for (int l = 0; l < L; ++l) sbB[l] = stage(P.bQT[l], CH_BN);
-      const float* sWoutQT = stage(P.WoutQT, CH_BN);
-      for (int l = 0; l < L; ++l) sbC[l] = stage(P.bQ[l], CH_BN);
-      const float* sWoutQ = stage(P.WoutQ, CH_BN);
+      for (int l = 0; l < L; ++l) sbA[l] = stage(P.bPT[l], H);
+      const float* sWoutPT = stage(P.WoutPT, H * d.dimu);
+      for (int l = 0; l < L; ++l) sbB[l] = stage(P.bQT[l], H);
+      const float* sWoutQT = stage(P.WoutQT, H);
+      for (int l = 0; l < L; ++l) sbC[l] = stage(P.bQ[l], H);
+      const float* sWoutQ = stage(P.WoutQ, H);
       asm volatile("bar.sync 3, 256;" ::: "memory");
-      for (int l = 1; l < L; ++l, ++g) ch_feed_relu(F, g, sbA[l - 1], nullptr, nullptr, n);
+      for (int l = 1; l < L; ++l, ++g) ch_feed_relu<H>(F, g, sbA[l - 1], nullptr, nullptr, n);
       float th[4];
-      ch_out_layer<4>(F, g, sbA[L - 1], nullptr, nullptr, n, sWoutPT, d.dimu, th);
+      ch_out_layer<H, 4>(F, g, sbA[L - 1], nullptr, nullptr, n, sWoutPT, d.dimu, th);
       ++g;
 #pragma unroll
       for (int j = 0; j < 4; ++j) th[j] = j < d.dimu ? tanhf(th[j] + __ldg(P.boutPT + j)) : 0.f;
       // ---------------- target.Q(o_2, g_2, pi_target) with the same td (ddpg.py:427-431)
       ch_feed_x(F, P.XQ_t, P.ld_sq, P.in_sq, P.in_sp, d.dimu, th);
       if (P.in_g > 0) ch_feed_x(F, P.Xg_t, P.ld_g, P.in_g, 0, 0, none);
-      for (int l = 1; l < L; ++l, ++g) ch_feed_relu(F, g, sbB[l - 1], nullptr, nullptr, n);
+      for (int l = 1; l < L; ++l, ++g) ch_feed_relu<H>(F, g, sbB[l - 1], nullptr, nullptr, n);
       float qt[1];
-      ch_out_layer<1>(F, g, sbB[L - 1], nullptr, nullptr, n, sWoutQT, 1, qt);
+      ch_out_layer<H, 1>(F, g, sbB[L - 1], nullptr, nullptr, n, sWoutQT, 1, qt);
       ++g;
       const float q_t = qt[0] + __ldg(P.boutQT);
       // ---------------- main.Q(o, g, u)
       ch_feed_x(F, P.XQu, P.ld_sq, P.in_sq, 0, 0, none);
       if (P.in_g > 0) ch_feed_x(F, P.Xg, P.ld_g, P.in_g, 0, 0, none);
-      for (int l = 1; l < L; ++l, ++g) ch_feed_relu(F, g, sbC[l - 1], P.hq[l - 1], P.mq + MW(l - 1), n);
+      for (int l = 1; l < L; ++l, ++g) ch_feed_relu<H>(F, g, sbC[l - 1], P.hq[l - 1], P.mq + MW(l - 1), n);
       float qv[1];
-      ch_out_layer<1>(F, g, sbC[L - 1], P.hq[L - 1], P.mq + MW(L - 1), n, sWoutQ, 1, qv);
+      ch_out_layer<H, 1>(F, g, sbC[L - 1], P.hq[L - 1], P.mq + MW(L - 1), n, sWoutQ, 1, qv);
       ++g;
       const float q = qv[0] + __ldg(P.boutQ);
       // ---------------- TD loss (ddpg.py:436-439) and its backward seed
@@ -586,8 +598,8 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
         if (fw == 0 && lane == 0) P.loss_part[4 * tile] = ssq;
       }
       // ---------------- backward through main.Q (critic chain)
-      ch_seed<1>(F, dq, 1, sWoutQ, P.mq + MW(L - 1), P.dc[L - 1], n);
-      for (int l = L - 1; l >= 1; --l, ++g) ch_feed_mask(F, g, P.mq + MW(l - 1), P.dc[l - 1], n, l >= 2);
+      ch_seed<H, 1>(F, dq, 1, sWoutQ, P.mq + MW(L - 1), P.dc[L - 1], n);
+      for (int l = L - 1; l >= 1; --l, ++g) ch_feed_mask<H>(F, g, P.mq + MW(l - 1), P.dc[l - 1], n, l >= 2);
     }
 #undef MW
     tc_fence_before();
@@ -596,7 +608,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
   if (tl && warp == 0) tl[1] = clock64();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(2 * H) : "memory");
   }
 }
 
@@ -809,8 +821,10 @@ int tc_chain_join(cudaStream_t s) {
 }
 
 // ---------------------------------------------------------------------------------------------------- host side
-bool tc_chain_supported(const cur_net_desc& d, int64_t n) {
-  if (d.hidden != CH_BN || n < CH_BM || (n % CH_BM) != 0 || d.dimu > 4 || d.layers < 2 || d.layers > 4) return false;
+bool tc_chain_width_supported(const cur_net_desc& d, int64_t n) {
+  if ((d.hidden != 64 && d.hidden != 128 && d.hidden != 256) || n < CH_BM || (n % CH_BM) != 0 || d.dimu > 4 ||
+      d.layers < 2 || d.layers > 4)
+    return false;
   const NetLayout q = net_layout(d, 0), p = net_layout(d, 1);
   if ((q.in_s + 31) / 32 + (q.in_g + 31) / 32 > 8) return false;
   // TMA: 16-byte aligned rows and bases of every weight block
@@ -819,6 +833,7 @@ bool tc_chain_supported(const cur_net_desc& d, int64_t n) {
     if ((q.off_W[l] % 4) || (p.off_W[l] % 4)) return false;
   return n / CH_BM <= (1 << 20);
 }
+bool tc_chain_supported(const cur_net_desc& d, int64_t n) { return d.hidden == 256 && tc_chain_width_supported(d, n); }
 
 // The 3xTF32 halves of the weights only depend on the previous update: split them on the side stream while the caller's
 // stream prepares the inputs (call before the input preparation is launched; tc_chain_launch then waits for the event).
@@ -838,13 +853,21 @@ int tc_chain_presplit_async(cudaStream_t s, const float* mQ, const float* tQ, fl
 static long long* g_chain_timeline = nullptr;
 void tc_chain_set_timeline(long long* dev) { g_chain_timeline = dev; }
 
-int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) {
-  CUR_REQUIRE(tc_chain_supported(d, io.n), "shape not supported by the chain kernel");
+template <int H>
+static int ch_kernel_launch(cudaStream_t s, int tiles, const ChainParams& P) {
   static bool configured = false;
   if (!configured) {
-    CUR_CUDA_TRY(cudaFuncSetAttribute(tc_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CH_SMEM_BYTES));
+    CUR_CUDA_TRY(cudaFuncSetAttribute(tc_chain_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      (int)ChW<H>::SMEM_BYTES));
     configured = true;
   }
+  tc_chain_kernel<H><<<2 * tiles, CH_THREADS, ChW<H>::SMEM_BYTES, s>>>(P);
+  CUR_CHECK_LAUNCH();
+  return CUR_OK;
+}
+
+int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) {
+  CUR_REQUIRE(tc_chain_width_supported(d, io.n), "shape not supported by the chain kernel");
   const NetLayout LQ = net_layout(d, 0), LP = net_layout(d, 1);
   const int L = d.layers, H = d.hidden;
   static thread_local ChainParams P;                      // 12 KB: kept off the stack; rebuilt on every call
@@ -921,7 +944,7 @@ int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) 
     for (int l = L - 1; l >= 1; --l) {
       ChGemm& g = pr.g[pr.n++];
       g.b_mn = 0; g.map1 = n_maps[role]; g.nkb1 = H / CH_BK; g.map2 = 0; g.nkb2 = 0;
-      CUR_TRY(map_pair(role, th + NL.off_W[l], H, CH_BN, false));
+      CUR_TRY(map_pair(role, th + NL.off_W[l], H, H, false));
     }
     return CUR_OK;
   };
@@ -931,8 +954,9 @@ int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) 
   CUR_REQUIRE(P.prog[0].n <= CH_MAX_GEMM && P.prog[1].n <= CH_MAX_GEMM, "chain program too long");
 
   const int tiles = (int)(io.n / CH_BM);
-  tc_chain_kernel<<<2 * tiles, CH_THREADS, CH_SMEM_BYTES, s>>>(P);
-  CUR_CHECK_LAUNCH();
+  if (H == 64) CUR_TRY(ch_kernel_launch<64>(s, tiles, P));
+  else if (H == 128) CUR_TRY(ch_kernel_launch<128>(s, tiles, P));
+  else CUR_TRY(ch_kernel_launch<256>(s, tiles, P));
   ChainLossParams LPm;
   LPm.part = io.loss_part; LPm.tiles = tiles; LPm.dimu = d.dimu; LPm.ring = io.loss_ring; LPm.n = io.n;
   LPm.action_l2 = io.action_l2; LPm.q_loss = io.q_loss; LPm.pi_loss = io.pi_loss; LPm.step_counter = io.step_counter;

@@ -56,9 +56,9 @@ struct TcChainIO {
   const float *XQpi, *XQ_t;                             // ... (action columns: taken from the policy output in the kernel)
   float* wsplit;                                        // 4 x arena floats: main hi | main lo | target hi | target lo
   int ld_spi, ld_sq, ld_g, lddy;
-  // TRANSPOSED copies [256][n] the weight gradients need: activations (main.pi, main.Q(u)), deltas (critic, actor chain)
+  // TRANSPOSED copies [H][n] the weight gradients need: activations (main.pi, main.Q(u)), deltas (critic, actor chain)
   float *hp[CUR_MAX_LAYERS], *hq[CUR_MAX_LAYERS], *dc[CUR_MAX_LAYERS], *dp[CUR_MAX_LAYERS];
-  uint32_t *mp, *mq, *mqp;                              // ReLU mask words [layers][8][n] of main.pi, main.Q(u), main.Q(pi)
+  uint32_t *mp, *mq, *mqp;                              // ReLU mask words [layers][H / 32][n] of main.pi, main.Q(u), main.Q(pi)
   float *Q, *Qt, *dQ, *dy, *q_pi;
   const float* r;
   float gamma, clip_return, action_l2;
@@ -87,7 +87,8 @@ int tc_chain_join(cudaStream_t s);                        // ... which `s` waits
 int tc_chain_lanes_fork(cudaStream_t s);
 int tc_chain_lane(int i, cudaStream_t* out);
 int tc_chain_lanes_join(cudaStream_t s);
-bool tc_chain_supported(const cur_net_desc& d, int64_t n);
+bool tc_chain_width_supported(const cur_net_desc& d, int64_t n);   // hidden 64, 128 or 256
+bool tc_chain_supported(const cur_net_desc& d, int64_t n);         // ... hidden 256 only (cur_ddpg_grads)
 int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io);
 int tc_chain_presplit_async(cudaStream_t s, const float* mQ, const float* tQ, float* wsplit, int64_t arena);
 void tc_chain_set_timeline(long long* dev);             // 128 x int64 debug stamps (CTA 0 / CTA 1) or NULL

@@ -74,10 +74,11 @@ class DDPG(object):
         #   True      always zero-padded to 256
         #   False     never: dependency-level kernels at the true width
         #   'native'  hidden 64 / 128 at the true width on the row kernels (train() up to 1024 rows, with the CUDA graph,
-        #             fused HER and fused Adam / the tile exchange) and the one-launch action kernel (get_actions up to 512
-        #             rows, compute_Q included).  Above 1024 rows the tcgen05 chain kernel needs 256 columns, so such a
-        #             batch runs the dependency-level kernels at the true width, like False.  Hidden 256 runs as always;
-        #             any other width raises ValueError.
+        #             fused HER and fused Adam / the tile exchange), on the tcgen05 chain kernel above (a multiple of 128
+        #             rows, cur_ddpg_chain_grads; weight gradients on K-sliced FFMA GEMMs, all-reduce + Adam after the graph
+        #             with several ranks, workers_per_rank > 1 as one wide batch) and on the one-launch action kernel
+        #             (get_actions up to 512 rows, compute_Q included).  Batches neither takes run the dependency-level
+        #             kernels at the true width, like False.  Hidden 256 runs as always; any other width raises ValueError.
         self.pad_hidden = kwargs.get('pad_hidden', 'auto')
         if self.pad_hidden == 'native' and self.hidden not in self.NATIVE_HIDDEN:
             raise ValueError("pad_hidden='native' needs hidden in %s, not %r" % (self.NATIVE_HIDDEN, self.hidden))
@@ -285,6 +286,23 @@ class DDPG(object):
             return False
         return ok
 
+    def _use_native_chain(self, n):
+        """A 'native' net narrower than 256 runs a batch of NATIVE_CHAIN_MIN_ROWS rows or more that the rows schedule does
+        not take on the chain kernel at its own width (cur_ddpg_chain_grads) when the library takes the shape - under
+        update_schedule 'auto' and 'levels' alike, as a hidden-256 net reaches the chain through cur_ddpg_grads from 1024
+        rows.  Smaller batches keep the paths they had: rows, or the level kernels at the true width."""
+        if (self.pad_hidden != 'native' or int(self.net.desc.hidden) >= self.KERNEL_HIDDEN or
+                n < self.NATIVE_CHAIN_MIN_ROWS or self._use_rows(n)):
+            return False
+        return bool(_lib.load().cur_ddpg_chain_supported(C.byref(self.net.desc), n))
+
+    def _workspace_chain(self, n):
+        key = ('chain', n)
+        if key not in self._ws:
+            floats = _lib.load().cur_ddpg_chain_workspace_floats(C.byref(self.net.desc), n)
+            self._ws[key] = torch.zeros(floats, dtype=torch.float32, device=self.device)
+        return self._ws[key]
+
     def _workspace_rows(self, n):
         key = ('rows', n)
         if key not in self._ws:
@@ -419,6 +437,9 @@ class DDPG(object):
         return ([u, slot['fin_q'].copy()] if compute_Q else u), True
 
     CHAIN_MIN_ROWS = 1024      # update_schedule='auto': rows schedule below, tcgen05 chain kernel from here
+    # pad_hidden='native', hidden 64 / 128: the narrow chain kernel from here (the rows schedule ends at 1024 rows and the
+    # chain takes multiples of 128; profiles/r04_native_chain.json)
+    NATIVE_CHAIN_MIN_ROWS = 1152
     ACTION_ROWS_MAX = 512      # rows per call served by the one-launch path (one CTA per 4 rows)
     ACTION_ZERO_COPY_MAX = 64  # ... of which up to this many rows travel zero-copy (kernel reads / writes host memory)
 
@@ -648,6 +669,12 @@ class DDPG(object):
                 C.byref(self._stats), C.byref(cb), C.byref(self._hyper), self._workspace_rows(n).data_ptr(),
                 self.grads.data_ptr(), self._q_loss.data_ptr(), self._pi_loss.data_ptr(), q_pi.data_ptr(), None, None),
                 'cur_ddpg_rows_step')
+        elif self._use_native_chain(n):
+            _lib.check(_lib.load().cur_ddpg_chain_grads(
+                _lib.stream_ptr(), C.byref(self.net.desc), self.theta_main.data_ptr(), self.theta_target.data_ptr(),
+                C.byref(self._stats), C.byref(cb), C.byref(self._hyper), self._workspace_chain(n).data_ptr(),
+                self.grads.data_ptr(), self._q_loss.data_ptr(), self._pi_loss.data_ptr(), q_pi.data_ptr()),
+                'cur_ddpg_chain_grads')
         else:
             _lib.check(_lib.load().cur_ddpg_grads(
                 _lib.stream_ptr(), C.byref(self.net.desc), self.theta_main.data_ptr(), self.theta_target.data_ptr(),
@@ -728,13 +755,14 @@ class DDPG(object):
         dev = self.device
         # several workers per rank as ONE wide batch: same gradient as k single-batch launches (loss seeds scaled by
         # 1 / batch_size, cur_ddpg_hyper.loss_rows) on the rows schedule up to 1024 rows or the tensor-core levels
-        # schedule above (3x faster at 19 workers); otherwise k accumulating launches of the rows schedule
+        # schedule above (3x faster at 19 workers), or the chain kernel at a native width; otherwise k accumulating
+        # launches of the rows schedule
         k = self.workers_per_rank
         lib = _lib.load()
         wide_rows = k * self.batch_size
         self._wide = bool(k > 1 and self.workers_mode != 'micro' and (
             (self.update_schedule != 'levels' and self._rows_shape_ok(wide_rows)) or
-            lib.cur_ddpg_uses_tensor_cores(C.byref(self.net.desc), wide_rows)))
+            lib.cur_ddpg_uses_tensor_cores(C.byref(self.net.desc), wide_rows) or self._use_native_chain(wide_rows)))
         self._graph_rows = self.batch_size * (k if self._wide else 1)
         self._micro = 1 if self._wide else k
         B = self._graph_rows
@@ -764,7 +792,12 @@ class DDPG(object):
         if self._micro > 1 and not self._use_rows(B):
             raise ValueError('workers_per_rank > 1 on the CUDA-graph path needs the rows schedule or a batch the '
                              'tensor-core levels schedule takes (workers x batch_size >= 1024, a multiple of 128)')
-        self._workspace_rows(B) if self._use_rows(B) else self._workspace(B)
+        if self._use_rows(B):
+            self._workspace_rows(B)
+        elif self._use_native_chain(B):
+            self._workspace_chain(B)
+        else:
+            self._workspace(B)
         self._peer = None
         self._xchg = None
         kind = self._exchange_kind()
@@ -904,6 +937,13 @@ class DDPG(object):
                     'cur_ddpg_rows_step')
             self._ghyper.transposes_valid = base_valid
             return fuse
+        if self._use_native_chain(n):
+            _lib.check(lib.cur_ddpg_chain_grads(
+                _lib.stream_ptr(), C.byref(self.net.desc), self.theta_main.data_ptr(), self.theta_target.data_ptr(),
+                C.byref(self._stats), C.byref(cb), C.byref(self._ghyper), self._workspace_chain(n).data_ptr(),
+                self.grads.data_ptr(), self._q_ring.data_ptr(), self._pi_ring.data_ptr(), self._q_pi.data_ptr()),
+                'cur_ddpg_chain_grads')
+            return False
         _lib.check(lib.cur_ddpg_grads(
             _lib.stream_ptr(), C.byref(self.net.desc), self.theta_main.data_ptr(), self.theta_target.data_ptr(),
             C.byref(self._stats), C.byref(cb), C.byref(self._ghyper), self._workspace(n).data_ptr(),

@@ -541,6 +541,19 @@ int cur_ddpg_uses_tensor_cores(const cur_net_desc* d, int64_t batch);
  * split-K weight-gradient GEMMs.  mode -1: default (on; CUR_DDPG_CHAIN=0 turns it off), 0: level-by-level schedule, 1: on. */
 int cur_ddpg_set_chain(int mode);
 int cur_ddpg_uses_chain(const cur_net_desc* d, int64_t batch);
+/* The same chain schedule at the net's own hidden width: DDPG._grads (ddpg.py:235-243: actor_critic.py:5-98 and
+ * util.py:56-107 forward, ddpg.py:412-449 losses and gradients) for hidden 64 or 128 without zero-padding to 256.
+ * cur_ddpg_uses_chain stays 0 for those nets and cur_ddpg_grads keeps the level-by-level schedule for them.
+ * cur_ddpg_chain_supported: 1 when cur_ddpg_chain_grads takes the desc and batch - hidden 64 or 128 (and the chain is on,
+ * cur_ddpg_set_chain), a batch that is a multiple of 128, dimu <= 4, 2-4 hidden layers; for hidden 256 the answer of
+ * cur_ddpg_uses_chain.  cur_ddpg_chain_grads: the arguments and outputs of cur_ddpg_grads, with a workspace of
+ * cur_ddpg_chain_workspace_floats(d, batch) floats; the weight gradients of a narrow net run as K-sliced FFMA GEMMs. */
+int cur_ddpg_chain_supported(const cur_net_desc* d, int64_t batch);
+int64_t cur_ddpg_chain_workspace_floats(const cur_net_desc* d, int64_t batch);
+int cur_ddpg_chain_grads(void* stream, const cur_net_desc* d, const float* theta_main,
+                         const float* theta_target, const cur_norm_stats* stats, const cur_batch* batch,
+                         const cur_ddpg_hyper* h, float* workspace, float* grads, float* q_loss,
+                         float* pi_loss, float* q_pi);
 /* debug: after updates run with CUR_ROWS_TIMELINE=1 (rows schedule, CUDA graph or not), print to stderr the %globaltimer
  * span of the two launches of the last updates and the gaps between them */
 int cur_rows_timeline_dump(void);
