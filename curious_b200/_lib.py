@@ -189,6 +189,7 @@ SIGNATURES = {
     'cur_ddpg_chain_grads': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_void_p, C.c_void_p,
                                        C.POINTER(NormStats), C.POINTER(Batch), C.POINTER(DdpgHyper), C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    'cur_ddpg_chain_grads_group': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_int, C.POINTER(DdpgExpert)]),
     'cur_tc_gemm_timeline': (C.c_int, [C.c_void_p]),
     'cur_tc_gemm_supported': (C.c_int, [C.c_int64, C.c_int64, C.c_int64]),
     'cur_tc_gemm_workspace_floats': (C.c_int64, [C.c_int64, C.c_int64, C.c_int64, C.c_int]),

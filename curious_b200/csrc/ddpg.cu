@@ -456,11 +456,15 @@ struct DwSliceSum {
   int64_t count;
   int splits;
 };
+constexpr int DW_PER_AGENT = 2 * (CUR_MAX_LAYERS + 1);   // weight-gradient problems of one agent, at most
+// CAP entries: one agent's (DW_PER_AGENT) or a grouped update's (CUR_MAX_TASKS x DW_PER_AGENT)
+template <int CAP>
 struct DwSliceSumBatch {
-  DwSliceSum p[2 * (CUR_MAX_LAYERS + 1)];
+  DwSliceSum p[CAP];
   int n;
 };
-__global__ void __launch_bounds__(256) dw_slice_sum_kernel(const __grid_constant__ DwSliceSumBatch R) {
+template <int CAP>
+__global__ void __launch_bounds__(256) dw_slice_sum_kernel(const __grid_constant__ DwSliceSumBatch<CAP> R) {
   for (int i = 0; i < R.n; ++i) {
     const DwSliceSum& P = R.p[i];
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < P.count; e += (int64_t)gridDim.x * blockDim.x) {
@@ -470,51 +474,79 @@ __global__ void __launch_bounds__(256) dw_slice_sum_kernel(const __grid_constant
     }
   }
 }
+template <int CAP>
+static int dw_slice_sum_launch(cudaStream_t s, const DwSliceSum* sums, int count) {
+  CUR_REQUIRE(count <= CAP, "too many weight-gradient problems");
+  DwSliceSumBatch<CAP> R;
+  R.n = count;
+  for (int i = 0; i < count; ++i) R.p[i] = sums[i];
+  dw_slice_sum_kernel<CAP><<<2 * sm_count(), 256, 0, s>>>(R);
+  CUR_CHECK_LAUNCH();
+  return CUR_OK;
+}
 
-// probs: dW problems with contiguous outputs (ldc == N), K = n, B K-major [N][n]; A K-major [M][n] (a_trans 0) or the
-// input matrix [n][lda] (a_trans 1).  part: CH_DW_MAX_SPLITS x (sum of M x N) floats.
-static int chain_dw_ffma(cudaStream_t s, const GemmProb* probs, int np, int64_t n, float* part) {
-  CUR_REQUIRE(np <= 2 * (CUR_MAX_LAYERS + 1) && part != nullptr, "bad weight-gradient list");
+// The K slices of one agent's problem list: enough for two CTAs per SM (the grouped GEMM's occupancy), each at least 256
+// rows, in whole GK chunks.  Every expert of a grouped update gets the slices it would get alone.
+struct DwSlicePlan {
+  int splits;
+  int64_t ks;              // rows per slice (the last one takes the rest)
+};
+static DwSlicePlan chain_dw_plan(const GemmProb* probs, int np, int64_t n) {
   int tiles = 0;
   for (int i = 0; i < np; ++i) tiles += ((probs[i].M + GT - 1) / GT) * ((probs[i].N + GT - 1) / GT);
-  // enough slices for two CTAs per SM (the grouped GEMM's occupancy), each at least 256 rows, in whole GK chunks
   int splits = (2 * sm_count() + tiles - 1) / (tiles > 0 ? tiles : 1);
   if (splits > CH_DW_MAX_SPLITS) splits = CH_DW_MAX_SPLITS;
   if (splits > n / 256) splits = (int)(n / 256);
   if (splits < 1) splits = 1;
-  const int64_t ks = ((n + splits - 1) / splits + GK - 1) / GK * GK;
-  splits = (int)((n + ks - 1) / ks);
+  DwSlicePlan pl;
+  pl.ks = ((n + splits - 1) / splits + GK - 1) / GK * GK;
+  pl.splits = (int)((n + pl.ks - 1) / pl.ks);
+  return pl;
+}
+
+// probs: n_e lists of np dW problems each (expert i's from probs + i * np, all lists of one shape) with contiguous outputs
+// (ldc == N), K = n, B K-major [N][n]; A K-major [M][n] (a_trans 0) or the input matrix [n][lda] (a_trans 1).  parts[i]:
+// expert i's CH_DW_MAX_SPLITS x (sum of M x N) floats.  The slice GEMMs of all experts share the grouped-GEMM launches
+// and one slice-sum launch adds every expert's slices.
+static int chain_dw_ffma(cudaStream_t s, const GemmProb* probs, int np, int n_e, int64_t n, float* const* parts) {
+  CUR_REQUIRE(np <= DW_PER_AGENT && n_e >= 1 && n_e <= CUR_MAX_TASKS, "bad weight-gradient list");
   GemmBatch G;
   G.n = 0; G.total_tiles = 0;
-  DwSliceSumBatch R;
-  R.n = 0;
-  float* pp = part;
-  for (int i = 0; i < np; ++i) {
-    const GemmProb& q = probs[i];
-    CUR_REQUIRE(q.ldc == q.N && q.b_trans == 1 && q.K == n, "bad weight-gradient problem");
-    const int64_t count = (int64_t)q.M * q.N;
-    for (int sl = 0; sl < splits; ++sl) {
-      const int64_t k0 = sl * ks;
-      GemmProb p = q;
-      p.split_k = 0;
-      p.K = (int)(k0 + ks <= n ? ks : n - k0);
-      p.A = q.a_trans ? q.A + k0 * q.lda : q.A + k0;
-      p.B = q.B + k0;
-      p.C = pp + sl * count;
-      G.p[G.n++] = p;
-      if (G.n == GEMM_MAX_PROBS) {
-        CUR_TRY(launch_gemm_batch(G, s));
-        G.n = 0;
+  DwSliceSum R[CUR_MAX_TASKS * DW_PER_AGENT];
+  int nr = 0;
+  for (int x = 0; x < n_e; ++x) {
+    const GemmProb* pr = probs + x * np;
+    const DwSlicePlan pl = chain_dw_plan(pr, np, n);
+    const int splits = pl.splits;
+    const int64_t ks = pl.ks;
+    float* pp = parts[x];
+    CUR_REQUIRE(pp != nullptr, "bad weight-gradient list");
+    for (int i = 0; i < np; ++i) {
+      const GemmProb& q = pr[i];
+      CUR_REQUIRE(q.ldc == q.N && q.b_trans == 1 && q.K == n, "bad weight-gradient problem");
+      const int64_t count = (int64_t)q.M * q.N;
+      for (int sl = 0; sl < splits; ++sl) {
+        const int64_t k0 = sl * ks;
+        GemmProb p = q;
+        p.split_k = 0;
+        p.K = (int)(k0 + ks <= n ? ks : n - k0);
+        p.A = q.a_trans ? q.A + k0 * q.lda : q.A + k0;
+        p.B = q.B + k0;
+        p.C = pp + sl * count;
+        G.p[G.n++] = p;
+        if (G.n == GEMM_MAX_PROBS) {
+          CUR_TRY(launch_gemm_batch(G, s));
+          G.n = 0;
+        }
       }
+      DwSliceSum& r = R[nr++];
+      r.part = pp; r.out = q.C; r.count = count; r.splits = splits;
+      pp += splits * count;
     }
-    DwSliceSum& r = R.p[R.n++];
-    r.part = pp; r.out = q.C; r.count = count; r.splits = splits;
-    pp += splits * count;
   }
   if (G.n > 0) CUR_TRY(launch_gemm_batch(G, s));
-  dw_slice_sum_kernel<<<2 * sm_count(), 256, 0, s>>>(R);
-  CUR_CHECK_LAUNCH();
-  return CUR_OK;
+  if (n_e == 1) return dw_slice_sum_launch<DW_PER_AGENT>(s, R, nr);
+  return dw_slice_sum_launch<CUR_MAX_TASKS * DW_PER_AGENT>(s, R, nr);
 }
 
 }  // namespace cur
@@ -657,14 +689,22 @@ struct GroupBatcher {
 
 // DDPG._grads for n_e experts of identical shape: every dependency level is ONE launch (per kernel kind) over all
 // experts - the grouped-GEMM form of structure='task_experts' (train.py:287-289 builds one DDPG per module).
-// narrow_chain: one agent of hidden 64 / 128 on the chain schedule (cur_ddpg_chain_grads)
+// narrow_chain: agents of hidden 64 / 128 on the chain schedule (cur_ddpg_chain_grads, cur_ddpg_chain_grads_group)
 static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_e, int64_t n, bool narrow_chain = false) {
   const NetLayout LQ = net_layout(*d, 0), LP = net_layout(*d, 1);
   const int L = d->layers, H = d->hidden;
   const bool chain = narrow_chain || use_chain(*d, n);
+  // the chain lanes of several narrow experts start from weights split by one launch beside the input preparation
+  const bool group_split = narrow_chain && n_e > 1;
   // ---- chain schedule, one agent: the 3xTF32 weight halves are split on a side stream beside the input preparation
   if (n_e == 1 && chain)
     CUR_TRY(tc_chain_presplit_async(s, E[0].mQ, E[0].tQ, E[0].w.chain_wsplit, r4(LQ.total) + r4(LP.total)));
+  if (group_split) {
+    const float *mQ[CUR_MAX_TASKS], *tQ[CUR_MAX_TASKS];
+    float* ws[CUR_MAX_TASKS];
+    for (int i = 0; i < n_e; ++i) { mQ[i] = E[i].mQ; tQ[i] = E[i].tQ; ws[i] = E[i].w.chain_wsplit; }
+    CUR_TRY(tc_chain_presplit_group_async(s, n_e, mQ, tQ, ws, r4(LQ.total) + r4(LP.total)));
+  }
   // ---- inputs
   for (int i = 0; i < n_e; ++i) {
     Expert& x = E[i];
@@ -688,10 +728,10 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
     // ---- chain schedule (tc_chain.cu): forward nets, losses and the data-gradient chains of a 128-row tile in one
     // CTA per chain, then every weight / bias gradient as split-K tensor-core GEMMs + row reductions, one level per net
     // (hidden 64 / 128: the weight gradients as K-sliced FFMA GEMMs, chain_dw_ffma)
-    CUR_REQUIRE(!narrow_chain || n_e == 1, "the narrow chain schedule runs one agent");
-    GemmProb dw_ffma[2 * (CUR_MAX_LAYERS + 1)];
+    GemmProb dw_ffma[CUR_MAX_TASKS * DW_PER_AGENT];
     int n_dw_ffma = 0;
 #define ADD_DW(prob) do { if (narrow_chain) dw_ffma[n_dw_ffma++] = (prob); else ADD(prob); } while (0)
+    if (group_split) CUR_TRY(tc_chain_presplit_wait(s));
     if (n_e > 1) CUR_TRY(tc_chain_lanes_fork(s));
     FOR_EXPERTS {
       Expert& x = E[i]; const Workspace& w = x.w;
@@ -709,6 +749,7 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
       io.loss_part = w.chain_loss; io.q_loss = x.q_loss; io.pi_loss = x.pi_loss;
       io.step_counter = x.h->step_counter; io.loss_ring = x.h->loss_ring;
       io.side_ok = n_e == 1 ? 1 : 0;
+      io.presplit = group_split ? 1 : 0;
       cudaStream_t cs = s;                         // several experts: independent chains on concurrent streams
       if (n_e > 1) CUR_TRY(tc_chain_lane(i, &cs));
       CUR_TRY(tc_chain_launch(cs, *d, io));
@@ -761,7 +802,11 @@ static int grads_levels(cudaStream_t s, const cur_net_desc* d, Expert* E, int n_
       CUR_TRY(tc_chain_rowsums(s, RS));             // side stream: next to the GEMM launches
     }
 #undef ADD_DW
-    if (narrow_chain) CUR_TRY(chain_dw_ffma(s, dw_ffma, n_dw_ffma, n, E[0].w.chain_dwpart));
+    if (narrow_chain) {
+      float* parts[CUR_MAX_TASKS];
+      for (int i = 0; i < n_e; ++i) parts[i] = E[i].w.chain_dwpart;
+      CUR_TRY(chain_dw_ffma(s, dw_ffma, n_dw_ffma / n_e, n_e, n, parts));
+    }
     CUR_TRY(B.flush());                             // (the batcher also flushes whenever a launch is full)
     CUR_TRY(B.B.T.finish(s));
     CUR_TRY(tc_chain_join(s));
@@ -962,4 +1007,22 @@ extern "C" int cur_ddpg_chain_grads(void* stream, const cur_net_desc* d, const f
   Expert x;
   CUR_TRY(fill_expert(x, d, theta_main, theta_target, stats, batch, h, workspace, grads, q_loss, pi_loss, q_pi, true));
   return grads_levels((cudaStream_t)stream, d, &x, 1, batch->n, d->hidden < 256);
+}
+
+extern "C" int cur_ddpg_chain_grads_group(void* stream, const cur_net_desc* d, int n_experts,
+                                          const cur_ddpg_expert* experts) {
+  CUR_TRY(check_desc(d));
+  CUR_REQUIRE(d->hidden < 256, "hidden-256 experts reach the chain schedule through cur_ddpg_grads_group");
+  CUR_REQUIRE(experts != nullptr && n_experts >= 1 && n_experts <= CUR_MAX_TASKS, "bad expert list");
+  const int64_t n = experts[0].batch.n;
+  CUR_REQUIRE(cur_ddpg_chain_supported(d, n), "shape not taken by the chain schedule");
+  for (int i = 1; i < n_experts; ++i)
+    CUR_REQUIRE(experts[i].batch.n == n, "all experts must train on the same batch size");
+  Expert E[CUR_MAX_TASKS];
+  for (int i = 0; i < n_experts; ++i) {
+    const cur_ddpg_expert& a = experts[i];
+    CUR_TRY(fill_expert(E[i], d, a.theta_main, a.theta_target, a.has_stats ? &a.stats : nullptr, &a.batch, &a.hyper,
+                        a.workspace, a.grads, a.q_loss, a.pi_loss, a.q_pi, true));
+  }
+  return grads_levels((cudaStream_t)stream, d, E, n_experts, n, true);
 }

@@ -614,9 +614,8 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
 
 // Once per update: every parameter of the four nets as the two TF32 halves of 3xTF32 (tc_ptx.cuh: tc_split1), laid out
 // like the parameter arenas themselves: out = [main hi | main lo | target hi | target lo], `arena` floats each
-__global__ void __launch_bounds__(256) tc_chain_presplit_kernel(const float* __restrict__ theta_main,
-                                                                 const float* __restrict__ theta_target, float* __restrict__ out,
-                                                                 int64_t arena4) {
+__device__ __forceinline__ void ch_presplit(const float* __restrict__ theta_main, const float* __restrict__ theta_target,
+                                            float* __restrict__ out, int64_t arena4) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= 2 * arena4) return;
   const bool tgt = i >= arena4;
@@ -627,6 +626,22 @@ __global__ void __launch_bounds__(256) tc_chain_presplit_kernel(const float* __r
   float4* o = reinterpret_cast<float4*>(out) + (tgt ? 2 * arena4 : 0);
   o[k] = h;
   o[arena4 + k] = l;
+}
+__global__ void __launch_bounds__(256) tc_chain_presplit_kernel(const float* __restrict__ theta_main,
+                                                                 const float* __restrict__ theta_target, float* __restrict__ out,
+                                                                 int64_t arena4) {
+  ch_presplit(theta_main, theta_target, out, arena4);
+}
+// the same for several experts of one shape, expert = blockIdx.y, each into its own buffer
+struct ChainPresplitGroup {
+  const float* mQ[CUR_MAX_TASKS];
+  const float* tQ[CUR_MAX_TASKS];
+  float* out[CUR_MAX_TASKS];
+  int64_t arena4;
+};
+__global__ void __launch_bounds__(256) tc_chain_presplit_group_kernel(const __grid_constant__ ChainPresplitGroup P) {
+  const int e = blockIdx.y;
+  ch_presplit(P.mQ[e], P.tQ[e], P.out[e], P.arena4);
 }
 
 // per-tile loss partials -> Q_loss / pi_loss (ring slot of the device step counter), fixed order; bumps the counter
@@ -850,6 +865,33 @@ int tc_chain_presplit_async(cudaStream_t s, const float* mQ, const float* tQ, fl
   return CUR_OK;
 }
 
+int tc_chain_presplit_group_async(cudaStream_t s, int n_e, const float* const* mQ, const float* const* tQ,
+                                  float* const* wsplit, int64_t arena) {
+  CUR_REQUIRE(n_e >= 1 && n_e <= CUR_MAX_TASKS, "bad expert count");
+  ChainSide* ss = nullptr;
+  CUR_TRY(chain_side(&ss));
+  ChainPresplitGroup P;
+  for (int i = 0; i < n_e; ++i) { P.mQ[i] = mQ[i]; P.tQ[i] = tQ[i]; P.out[i] = wsplit[i]; }
+  P.arena4 = arena / 4;
+  CUR_CUDA_TRY(cudaEventRecord(ss->fork0, s));
+  CUR_CUDA_TRY(cudaStreamWaitEvent(ss->stream, ss->fork0, 0));
+  tc_chain_presplit_group_kernel<<<dim3((unsigned)((2 * P.arena4 + 255) / 256), (unsigned)n_e), 256, 0, ss->stream>>>(P);
+  CUR_CHECK_LAUNCH();
+  CUR_CUDA_TRY(cudaEventRecord(ss->split_done, ss->stream));
+  ss->split_pending = true;
+  return CUR_OK;
+}
+
+int tc_chain_presplit_wait(cudaStream_t s) {
+  ChainSide* ss = nullptr;
+  CUR_TRY(chain_side(&ss));
+  if (ss->split_pending) {
+    CUR_CUDA_TRY(cudaStreamWaitEvent(s, ss->split_done, 0));
+    ss->split_pending = false;
+  }
+  return CUR_OK;
+}
+
 static long long* g_chain_timeline = nullptr;
 void tc_chain_set_timeline(long long* dev) { g_chain_timeline = dev; }
 
@@ -902,7 +944,9 @@ int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) 
   CUR_REQUIRE(io.wsplit != nullptr && io.mP == io.mQ + r4(LQ.total) && io.tP == io.tQ + r4(LQ.total), "parameter arenas expected");
   ChainSide* side = nullptr;
   CUR_TRY(chain_side(&side));
-  if (io.side_ok && side->split_pending) {
+  if (io.presplit) {
+    // split by tc_chain_presplit_group_async; the launch stream forked after tc_chain_presplit_wait
+  } else if (io.side_ok && side->split_pending) {
     CUR_CUDA_TRY(cudaStreamWaitEvent(s, side->split_done, 0));      // split by tc_chain_presplit_async
     side->split_pending = false;
   } else {

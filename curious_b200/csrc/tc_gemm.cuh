@@ -69,6 +69,8 @@ struct TcChainIO {
   int loss_ring;
   int side_ok;                                          // one agent, launched on the caller's stream: the weight split may have run on
                                                         // the side stream (tc_chain_presplit_async) and the loss fold goes with the row sums
+  int presplit;                                         // wsplit already holds the halves (tc_chain_presplit_group_async, then
+                                                        // tc_chain_presplit_wait on the stream the lanes fork from)
 };
 // bias / output-layer weight gradients from the transposed copies (tc_chain_rowsum_kernel)
 struct TcRowSum {
@@ -91,6 +93,11 @@ bool tc_chain_width_supported(const cur_net_desc& d, int64_t n);   // hidden 64,
 bool tc_chain_supported(const cur_net_desc& d, int64_t n);         // ... hidden 256 only (cur_ddpg_grads)
 int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io);
 int tc_chain_presplit_async(cudaStream_t s, const float* mQ, const float* tQ, float* wsplit, int64_t arena);
+// several experts: ONE launch on the side stream splits every expert's weights into its own wsplit; `s` waits for it in
+// tc_chain_presplit_wait
+int tc_chain_presplit_group_async(cudaStream_t s, int n_e, const float* const* mQ, const float* const* tQ,
+                                  float* const* wsplit, int64_t arena);
+int tc_chain_presplit_wait(cudaStream_t s);
 void tc_chain_set_timeline(long long* dev);             // 128 x int64 debug stamps (CTA 0 / CTA 1) or NULL
 // row-major [rows][cols] fp32 operand as a TMA tensor map in the layouts the tcgen05 descriptors expect (tc_gemm.cu)
 int tc_make_map(void* map /* CUtensorMap */, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows,

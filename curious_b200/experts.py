@@ -5,9 +5,11 @@ trains ONE of them per epoch (`policy[i_policy].train()`, train.py:108-113).  On
 expert leaves the GPU mostly idle (every GEMM level is latency-bound), so `TaskExperts.train()` steps ALL experts
 in one sequence of grouped launches: every dependency level of the DDPG graph is one launch over the problems of all
 experts (csrc/ddpg.cu cur_ddpg_grads_group; FFMA grouped GEMM at batch 256, the tcgen05 batch at batch >= 1024).
+Experts built with pad_hidden='native' at hidden 64 / 128 that train on the narrow chain (from 1152 rows) run
+cur_ddpg_chain_grads_group instead: their chain kernels side by side, their K-sliced weight gradients in shared launches.
 Semantically it is `for p in policies: p.train()` - every expert keeps its own parameters, Adam state, Philox
 stream, LP apportioning and buffers, and the result is bit-identical to stepping them one after the other on the
-levels schedule.
+levels schedule, or on the narrow chain for native experts.
 """
 import ctypes as C
 
@@ -23,7 +25,10 @@ class TaskExperts(object):
         """mode: 'grouped' = grouped launches; 'sequential' = p.train() one after the other; 'auto' = sequential
         when every expert runs the rows schedule at batch <= 512 (one expert's row CTAs already fill the 148 SMs;
         measured per round of 4 experts: batch 256 237 us vs 322 us grouped, 512 435 vs 524, 1024 841 vs 372),
-        grouped otherwise."""
+        grouped otherwise.  Native hidden-64 / 128 experts on the narrow chain give the same bits either way and grouped
+        is faster at every measured shape (one B200, 1000 W, profiles/r05_native_experts.json, 4 experts, Arm4, us per
+        round grouped vs sequential: hidden 64 1152 rows 191 vs 344, 4864 rows 460 vs 529; hidden 128 233 vs 429 and
+        589 vs 694; Arm8 alike), so they run grouped."""
         assert len(policies) >= 1 and mode in ('auto', 'grouped', 'sequential')
         self.mode = mode
         p0 = policies[0]
@@ -42,7 +47,19 @@ class TaskExperts(object):
         return self.policies[i]
 
     # ------------------------------------------------------------------------------------------
-    def _expert_array(self, graph):
+    def _native_chain(self):
+        """Every expert is a native hidden-64 / 128 net that trains on the narrow chain at its batch size
+        (DDPG._use_native_chain): the round runs as cur_ddpg_chain_grads_group, bit for bit what each expert's own
+        cur_ddpg_chain_grads gives."""
+        return all(p._use_native_chain(p.batch_size) for p in self.policies)
+
+    def _grads_group(self, arr, chain):
+        lib = _lib.load()
+        fn, name = ((lib.cur_ddpg_chain_grads_group, 'cur_ddpg_chain_grads_group') if chain else
+                    (lib.cur_ddpg_grads_group, 'cur_ddpg_grads_group'))
+        _lib.check(fn(_lib.stream_ptr(), C.byref(self.policies[0].net.desc), len(arr), arr), name)
+
+    def _expert_array(self, graph, chain):
         arr = (_lib.DdpgExpert * len(self.policies))()
         for e, p in zip(arr, self.policies):
             n = p.batch_size
@@ -56,7 +73,7 @@ class TaskExperts(object):
                                  b['td'].data_ptr() if p.modular else None, b['o_2'].data_ptr(), g2.data_ptr(),
                                  b['r'].data_ptr(), n)
             e.hyper = p._ghyper if graph else p._hyper
-            e.workspace = p._workspace(n).data_ptr()
+            e.workspace = (p._workspace_chain(n) if chain else p._workspace(n)).data_ptr()
             e.grads = p.grads.data_ptr()
             if graph:
                 e.q_loss, e.pi_loss, e.q_pi = p._q_ring.data_ptr(), p._pi_ring.data_ptr(), p._q_pi.data_ptr()
@@ -67,7 +84,6 @@ class TaskExperts(object):
 
     def _launch(self, graph):
         """HER sample per expert, grouped gradients, then (single rank) Adam per expert."""
-        lib = _lib.load()
         for p in self.policies:
             if graph:
                 segs = [(buf.device_view(), 0, ttr) for buf, ttr in p._all_segments()]
@@ -76,16 +92,17 @@ class TaskExperts(object):
                                                    dyn=p._dyn_dev.data_ptr(), call_offset=p.GRAPH_STREAM_OFFSET)
             else:
                 p.stage_batch()
-        arr = self._expert_array(graph)
+        chain = self._native_chain()
+        arr = self._expert_array(graph, chain)
         self._keep = arr
-        _lib.check(lib.cur_ddpg_grads_group(_lib.stream_ptr(), C.byref(self.policies[0].net.desc), len(arr), arr),
-                   'cur_ddpg_grads_group')
+        self._grads_group(arr, chain)
 
     def _build_graph(self):
+        chain = self._native_chain()
         for p in self.policies:
             p.grad_exchange = 'nccl'          # several ranks: NCCL all-reduce + Adam after the graph
             p._prepare_graph_state()
-            p._workspace(p.batch_size)
+            (p._workspace_chain if chain else p._workspace)(p.batch_size)
         dev = self.policies[0].device
         torch.cuda.current_stream().synchronize()
         states = [(p.theta_main.clone(), p._adam_m.clone(), p._adam_v.clone(), p._step.clone()) for p in self.policies]
@@ -141,10 +158,10 @@ class TaskExperts(object):
         if stage:
             self._launch(False)
         else:
-            arr = self._expert_array(False)
+            chain = self._native_chain()
+            arr = self._expert_array(False, chain)
             self._keep = arr
-            _lib.check(_lib.load().cur_ddpg_grads_group(_lib.stream_ptr(), C.byref(ps[0].net.desc), len(arr), arr),
-                       'cur_ddpg_grads_group')
+            self._grads_group(arr, chain)
         out = []
         for p in ps:
             p._update(p._view(p.grads, 'Q'), p._view(p.grads, 'pi'))

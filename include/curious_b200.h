@@ -554,6 +554,12 @@ int cur_ddpg_chain_grads(void* stream, const cur_net_desc* d, const float* theta
                          const float* theta_target, const cur_norm_stats* stats, const cur_batch* batch,
                          const cur_ddpg_hyper* h, float* workspace, float* grads, float* q_loss,
                          float* pi_loss, float* q_pi);
+/* cur_ddpg_grads_group on the narrow chain: n_experts (1..CUR_MAX_TASKS) agents of hidden 64 or 128 and one batch size
+ * that cur_ddpg_chain_supported takes, each with a workspace of cur_ddpg_chain_workspace_floats(d, batch) floats.  The
+ * experts' chain kernels run side by side, their K-sliced weight-gradient GEMMs share grouped launches; every expert gets
+ * the bits cur_ddpg_chain_grads gives it alone.  Hidden 256, a shape the chain does not take and differing batch sizes
+ * are refused before anything is launched. */
+int cur_ddpg_chain_grads_group(void* stream, const cur_net_desc* d, int n_experts, const cur_ddpg_expert* experts);
 /* debug: after updates run with CUR_ROWS_TIMELINE=1 (rows schedule, CUDA graph or not), print to stderr the %globaltimer
  * span of the two launches of the last updates and the gaps between them */
 int cur_rows_timeline_dump(void);
