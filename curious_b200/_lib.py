@@ -81,6 +81,10 @@ class NormStats(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('o_mean', 'o_std', 'g_mean', 'g_std')]
 
 
+class ActionsExpert(C.Structure):
+    _fields_ = [('theta', C.c_void_p), ('stats', NormStats)]
+
+
 class Batch(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('o', 'g', 'u', 'td', 'o_2', 'g_2', 'r')] + [('n', C.c_int64)]
 
@@ -154,13 +158,18 @@ SIGNATURES = {
     'cur_ddpg_actions_rows': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_void_p, C.POINTER(NormStats), C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_void_p,
                                         C.c_uint32]),
-    'cur_actions_finish_host': (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_void_p,
+    'cur_ddpg_actions_rows_group': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_int, C.POINTER(ActionsExpert),
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                              C.c_float, C.c_void_p, C.c_void_p, C.c_uint32]),
+    'cur_actions_finish_host':(C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_uint32, C.c_void_p, C.c_void_p,
                                           C.c_void_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_int64]),
     'cur_host_alloc': (C.c_int, [C.c_int64, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]),
     'cur_host_free': (C.c_int, [C.c_void_p]),
     'cur_copy_h2d': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]),
     'cur_action_noise': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_float, C.c_double, C.c_double,
                                    C.c_uint64, C.c_uint64]),
+    'cur_action_noise_rows': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_float, C.c_double, C.c_double,
+                                        C.c_void_p, C.c_void_p]),
     'cur_net_param_count': (C.c_int64, [C.POINTER(NetDesc), C.c_int]),
     'cur_theta_pi_offset': (C.c_int64, [C.POINTER(NetDesc), C.POINTER(C.c_int64)]),
     'cur_ddpg_workspace_floats': (C.c_int64, [C.POINTER(NetDesc), C.c_int64]),

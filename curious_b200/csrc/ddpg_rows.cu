@@ -1259,7 +1259,10 @@ struct ActParams {
   SChunk chunks[A_MAXCHUNK];
 };
 
-__device__ __forceinline__ float act_x_elem(const ActParams& P, int64_t row, int r, int k, int act_kind, const float* ths) {
+// (the normaliser statistics are arguments: the routed kernel takes them from its CTA's expert)
+template <class PT>
+__device__ __forceinline__ float act_x_elem(const PT& P, const float* o_mean, const float* o_std, const float* g_mean,
+                                            const float* g_std, int64_t row, int r, int k, int act_kind, const float* ths) {
   const cur_net_desc& d = P.d;
   const bool nrm = d.normalize_obs != 0;
   const int in_s = P.in_sp + (act_kind ? d.dimu : 0);
@@ -1269,7 +1272,7 @@ __device__ __forceinline__ float act_x_elem(const ActParams& P, int64_t row, int
   if (k < d.dimo) {
     v = P.o[row * d.dimo + k];
     if (clip > 0.f) v = fminf(fmaxf(v, -clip), clip);
-    if (nrm) v = norm1s(v, P.o_mean, P.o_std, k, d.norm_clip);
+    if (nrm) v = norm1s(v, o_mean, o_std, k, d.norm_clip);
   } else if (d.modular) {
     if (k < d.dimo + d.dimtd) v = P.td[row * d.dimtd + (k - d.dimo)];       // never normalised
     else if (k < in_s) aj = k - d.dimo - d.dimtd;
@@ -1282,7 +1285,7 @@ __device__ __forceinline__ float act_x_elem(const ActParams& P, int64_t row, int
     v = P.g[row * d.dimg + gj];
     if (P.ag) v = __fsub_rn(v, P.ag[row * d.dimg + gj]);
     if (clip > 0.f) v = fminf(fmaxf(v, -clip), clip);
-    if (nrm) v = norm1s(v, P.g_mean, P.g_std, gj, d.norm_clip);
+    if (nrm) v = norm1s(v, g_mean, g_std, gj, d.norm_clip);
   }
   if (aj >= 0) v = ths[r * S_DU + aj];
   return v;
@@ -1344,7 +1347,8 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
   auto build = [&](int act_kind) {
     for (int idx = tid; idx < S_ROWS * P.KP; idx += S_CONSUMERS) {
       const int k = idx >> 2, r = idx & 3;
-      xa[k * 4 + r] = act_x_elem(P, row0 + (r < nr ? r : nr - 1), r, k, act_kind, s_th);
+      xa[k * 4 + r] = act_x_elem(P, P.o_mean, P.o_std, P.g_mean, P.g_std, row0 + (r < nr ? r : nr - 1), r, k, act_kind,
+                                 s_th);
     }
   };
   build(0);
@@ -1371,6 +1375,110 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
   }
   A_TL(3);
 #undef A_TL
+}
+
+// ------------------------------------------------------------------------------------------------
+// The routed form (a task-experts evaluation step, rollout.py:211-223: each row is acted on by the expert of its module):
+// the same CTA per 4 rows, ring and GEMV core, but every CTA tile belongs to one expert and takes that expert's weights
+// and normaliser statistics from a per-launch table.  The host groups the rows by expert (each group padded to a multiple
+// of 4) into a row map; inputs are read from and outputs written to the rows' original positions.  All experts share one
+// cur_net_desc, so the chunk list is one list of offsets into any expert's theta.
+constexpr int G_MAXROWS = 512;                                   // rows per routed launch
+constexpr int G_MAXTILES = G_MAXROWS / S_ROWS + CUR_MAX_TASKS;   // each expert's group rounds up to whole tiles
+
+struct ActExpert {
+  const float* theta;
+  const float *o_mean, *o_std, *g_mean, *g_std;
+  const float *bP[S_MAXL], *bQ[S_MAXL];
+  const float *WoutP, *boutP, *WoutQ, *boutQ;
+};
+
+struct ActGroupParams {
+  cur_net_desc d;
+  int in_sp, in_g, KP, L, nchunks;
+  int dbg_skip_math;         // (read by the shared GEMV core)
+  int ch0[2];
+  const float *o, *g, *td, *ag;
+  float clip;
+  uint32_t seq;
+  void *pi, *q;
+  SChunk chunks[A_MAXCHUNK];           // nrows / k0 of every chunk (src unused: see coff)
+  int32_t coff[A_MAXCHUNK];            // float offset of every chunk in an expert's theta
+  ActExpert ex[CUR_MAX_TASKS];
+  uint8_t tile_ex[G_MAXTILES];         // expert of every CTA
+  int16_t tile_row[G_MAXTILES][S_ROWS];   // original row of every slot; -1: padding (valid slots come first)
+};
+
+template <int H>
+__global__ void __launch_bounds__(S_THREADS, 1)
+actions_group_kernel(const __grid_constant__ ActGroupParams P) {
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  float* ringf = reinterpret_cast<float*>(smem_raw);
+  float* xa = ringf + S_NSLOT * S_SLOT;
+  float* xb = xa + S_XT;
+  float* red = xb + S_XT;
+  float* misc = red + S_RED;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(misc + S_MISC);
+  float* s_th = misc;                 // [4][8] tanh output
+  float* s_q = misc + 64;             // [4][8]
+  const int tid = threadIdx.x;
+  const ActExpert& E = P.ex[P.tile_ex[blockIdx.x]];
+  const cur_net_desc& d = P.d;
+  const uint32_t full = smem_addr(bars), empty = smem_addr(bars + S_NSLOT);
+  if (tid == 0) {
+    for (int i = 0; i < S_NSLOT; ++i) {
+      mbar_init(full + 8 * i, 1);
+      mbar_init(empty + 8 * i, S_CONSUMERS / 32);
+    }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  if (tid >= S_CONSUMERS) {
+    if (tid == S_CONSUMERS) {
+      const uint32_t ring_s = smem_addr(ringf);
+      for (int i = 0; i < P.nchunks; ++i) {
+        const int slot = i % S_NSLOT, round = i / S_NSLOT;
+        if (round > 0) mbar_wait(empty + 8 * slot, (round - 1) & 1);
+        const uint32_t bytes = (uint32_t)P.chunks[i].nrows * H * 4;
+        mbar_expect_tx(full + 8 * slot, bytes);
+        bulk_g2s(ring_s + slot * S_SLOT * 4, E.theta + P.coff[i], bytes, full + 8 * slot);
+      }
+    }
+    return;
+  }
+  Ring rg;
+  rg.chunks = P.chunks; rg.slots = ringf; rg.full = full; rg.empty = empty; rg.cons = 0;
+  const int16_t* tile = P.tile_row[blockIdx.x];
+  int nr = 0;
+#pragma unroll
+  for (int r = 0; r < S_ROWS; ++r) nr += tile[r] >= 0;
+  auto row_of = [&](int r) -> int64_t { return tile[r] >= 0 ? tile[r] : tile[0]; };   // padding repeats the first row
+  auto build = [&](int act_kind) {
+    for (int idx = tid; idx < S_ROWS * P.KP; idx += S_CONSUMERS) {
+      const int k = idx >> 2, r = idx & 3;
+      xa[k * 4 + r] = act_x_elem(P, E.o_mean, E.o_std, E.g_mean, E.g_std, row_of(r), r, k, act_kind, s_th);
+    }
+  };
+  build(0);
+  consumer_sync();
+  float* xl = forward_net<H, 4>(P, rg, P.ch0[0], xa, xb, red, E.bP, nullptr, nullptr, 0);
+  small_out<H>(xl, 4, 0, 4, E.WoutP, d.dimu, 1, d.dimu, E.boutP, s_th);
+  consumer_sync();
+  if (tid < S_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) {
+    const float th = tanhf(s_th[tid]);                                  // actor_critic.py:89
+    s_th[tid] = th;
+    const int r = tid >> 3, j = tid & (S_DU - 1);
+    if (r < nr) put_out(P.pi, row_of(r) * d.dimu + j, d.max_u * th, P.seq);
+  }
+  consumer_sync();
+  if (P.q != nullptr) {
+    build(2);                                                          // Q(o, g, pi / max_u): the noise-free action
+    consumer_sync();
+    xl = forward_net<H, 4>(P, rg, P.ch0[1], xa, xb, red, E.bQ, nullptr, nullptr, 0);
+    small_out<H>(xl, 4, 0, 4, E.WoutQ, 1, 1, 1, E.boutQ, s_q);
+    consumer_sync();
+    if (tid < nr) put_out(P.q, row_of(tid), s_q[tid * S_DU], P.seq);
+  }
 }
 
 // W^T of the hidden layers (operands of the backward streams): dst[m][j][i] = src_m[i][j], H x H each
@@ -2085,14 +2193,19 @@ static int launch_stream(cudaLaunchConfig_t& cfg, const StreamParams& P) {
 }
 
 template <int H>
-static int launch_actions(unsigned blocks, cudaStream_t s, const ActParams& P) {
+static auto act_kernel(const ActParams*) { return actions_stream_kernel<H>; }
+template <int H>
+static auto act_kernel(const ActGroupParams*) { return actions_group_kernel<H>; }
+
+template <int H, class PT>
+static int launch_actions(unsigned blocks, cudaStream_t s, const PT& P) {
   static bool configured = false;
+  const auto kernel = act_kernel<H>(&P);
   if (!configured) {
-    CUR_CUDA_TRY(cudaFuncSetAttribute(actions_stream_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)S_SMEM_BYTES));
+    CUR_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S_SMEM_BYTES));
     configured = true;
   }
-  actions_stream_kernel<H><<<blocks, S_THREADS, S_SMEM_BYTES, s>>>(P);
+  kernel<<<blocks, S_THREADS, S_SMEM_BYTES, s>>>(P);
   return CUR_OK;
 }
 
@@ -2580,37 +2693,31 @@ extern "C" int cur_ddpg_rows_transposes(const cur_net_desc* d, float* workspace,
 }
 
 
-// One launch for DDPG.get_actions (see actions_stream_kernel).  o / ag / g / td / out_pi / out_q may be device
-// pointers of mapped pinned host memory.  seq != 0: the outputs are 8-byte words {float32 bits | seq << 32}.
-extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
-                                     const float* o, const float* ag, const float* g, const float* td, int64_t n,
-                                     float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
-  CUR_TRY(check_desc(d));
-  CUR_REQUIRE(theta && o && g && out_pi, "NULL argument");
-  CUR_REQUIRE(!d->modular || td, "task_descr required for a modular net");
-  CUR_REQUIRE(n > 0 && n <= 4096, "bad row count (the one-launch action path covers up to 4096 rows)");
-  CUR_REQUIRE(rows_supported(d, S_ROWS), "shape not supported by the rows schedule (see cur_ddpg_rows_supported)");
-  if (d->normalize_obs)
-    CUR_REQUIRE(stats && stats->o_mean && stats->o_std && stats->g_mean && stats->g_std, "normalizer stats required");
+// bias and output-layer pointers of the forward nets of `theta` (ActParams, ActExpert)
+template <class T>
+static void act_net_ptrs(T& P, const cur_net_desc& d, const float* theta) {
+  const NetLayout LQ = net_layout(d, 0), LP = net_layout(d, 1);
+  const float *thQ = theta, *thP = theta + r4(LQ.total);
+  for (int l = 0; l < S_MAXL; ++l) {
+    P.bP[l] = l < d.layers ? thP + ((l == 0) ? LP.off_b0 : LP.off_b[l]) : nullptr;
+    P.bQ[l] = l < d.layers ? thQ + ((l == 0) ? LQ.off_b0 : LQ.off_b[l]) : nullptr;
+  }
+  P.WoutP = thP + LP.off_Wout; P.boutP = thP + LP.off_bout;
+  P.WoutQ = thQ + LQ.off_Wout; P.boutQ = thQ + LQ.off_bout;
+}
+
+// What ActParams and ActGroupParams share: the shape, the inputs, the outputs and the weight chunks of `theta`
+template <class PT>
+static int act_common(PT& P, const cur_net_desc* d, const float* theta, const float* o, const float* ag, const float* g,
+                      const float* td, float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
   const NetLayout LQ = net_layout(*d, 0), LP = net_layout(*d, 1);
   const float *thQ = theta, *thP = theta + r4(LQ.total);
   const int L = d->layers, H = d->hidden;
-  static const bool tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
-  ActParams P;
   P.d = *d;
   P.in_sp = LP.in_s; P.in_g = LQ.in_g; P.L = L;
   P.KP = (LQ.in_s + LQ.in_g + 3) / 4 * 4;
   P.dbg_skip_math = 0;
-  P.n = n;
   P.o = o; P.g = g; P.td = td; P.ag = ag; P.clip = clip_obs; P.seq = seq;
-  P.o_mean = P.o_std = P.g_mean = P.g_std = nullptr;
-  if (stats) { P.o_mean = stats->o_mean; P.o_std = stats->o_std; P.g_mean = stats->g_mean; P.g_std = stats->g_std; }
-  for (int l = 0; l < S_MAXL; ++l) {
-    P.bP[l] = l < L ? thP + ((l == 0) ? LP.off_b0 : LP.off_b[l]) : nullptr;
-    P.bQ[l] = l < L ? thQ + ((l == 0) ? LQ.off_b0 : LQ.off_b[l]) : nullptr;
-  }
-  P.WoutP = thP + LP.off_Wout; P.boutP = thP + LP.off_bout;
-  P.WoutQ = thQ + LQ.off_Wout; P.boutQ = thQ + LQ.off_bout;
   P.pi = out_pi; P.q = out_q;
   int nc = 0;
   const int CK = chunk_rows(H);
@@ -2632,6 +2739,29 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
   P.ch0[0] = forward_net(thP, LP);
   P.ch0[1] = out_q != nullptr ? forward_net(thQ, LQ) : 0;
   P.nchunks = nc;
+  return CUR_OK;
+}
+
+// One launch for DDPG.get_actions (see actions_stream_kernel).  o / ag / g / td / out_pi / out_q may be device
+// pointers of mapped pinned host memory.  seq != 0: the outputs are 8-byte words {float32 bits | seq << 32}.
+extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
+                                     const float* o, const float* ag, const float* g, const float* td, int64_t n,
+                                     float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
+  CUR_TRY(check_desc(d));
+  CUR_REQUIRE(theta && o && g && out_pi, "NULL argument");
+  CUR_REQUIRE(!d->modular || td, "task_descr required for a modular net");
+  CUR_REQUIRE(n > 0 && n <= 4096, "bad row count (the one-launch action path covers up to 4096 rows)");
+  CUR_REQUIRE(rows_supported(d, S_ROWS), "shape not supported by the rows schedule (see cur_ddpg_rows_supported)");
+  if (d->normalize_obs)
+    CUR_REQUIRE(stats && stats->o_mean && stats->o_std && stats->g_mean && stats->g_std, "normalizer stats required");
+  const int H = d->hidden;
+  static const bool tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
+  ActParams P;
+  CUR_TRY(act_common(P, d, theta, o, ag, g, td, clip_obs, out_pi, out_q, seq));
+  P.n = n;
+  P.o_mean = P.o_std = P.g_mean = P.g_std = nullptr;
+  if (stats) { P.o_mean = stats->o_mean; P.o_std = stats->o_std; P.g_mean = stats->g_mean; P.g_std = stats->g_std; }
+  act_net_ptrs(P, *d, theta);
   static long long* tl_dev = nullptr;
   static int tl_calls = 0;
   if (tl_on && tl_dev == nullptr) {
@@ -2651,6 +2781,66 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
     fprintf(stderr, "[actions timeline] inputs %lld | pi forward %lld | outputs (+ Q) %lld | total %lld ns\n", t[1] - t[0],
             t[2] - t[1], t[3] - t[2], t[3] - t[0]);
   }
+  return CUR_OK;
+}
+
+// The routed form of cur_ddpg_actions_rows (see actions_group_kernel): row i is acted on by experts[row_expert[i]].  The
+// rows of each expert fill whole 4-row tiles in their original order; outputs go to the rows' original positions.
+extern "C" int cur_ddpg_actions_rows_group(void* stream, const cur_net_desc* d, int n_experts,
+                                           const cur_actions_expert* experts, const int32_t* row_expert, const float* o,
+                                           const float* ag, const float* g, const float* td, int64_t n, float clip_obs,
+                                           void* out_pi, void* out_q, uint32_t seq) {
+  CUR_TRY(check_desc(d));
+  CUR_REQUIRE(n_experts >= 1 && n_experts <= CUR_MAX_TASKS, "n_experts must be 1..CUR_MAX_TASKS");
+  CUR_REQUIRE(experts && row_expert && o && g && out_pi, "NULL argument");
+  CUR_REQUIRE(!d->modular || td, "task_descr required for a modular net");
+  CUR_REQUIRE(n > 0 && n <= G_MAXROWS, "bad row count (the routed action launch covers up to 512 rows)");
+  CUR_REQUIRE(rows_supported(d, S_ROWS), "shape not supported by the rows schedule (see cur_ddpg_rows_supported)");
+  int count[CUR_MAX_TASKS] = {0};
+  for (int64_t i = 0; i < n; ++i) {
+    CUR_REQUIRE(row_expert[i] >= 0 && row_expert[i] < n_experts, "row_expert entry out of range");
+    ++count[row_expert[i]];
+  }
+  int first = -1;
+  for (int e = 0; e < n_experts; ++e) {
+    if (count[e] == 0) continue;
+    const cur_actions_expert& X = experts[e];
+    CUR_REQUIRE(X.theta, "NULL theta");
+    if (d->normalize_obs)
+      CUR_REQUIRE(X.stats.o_mean && X.stats.o_std && X.stats.g_mean && X.stats.g_std, "normalizer stats required");
+    if (first < 0) first = e;
+  }
+  ActGroupParams P;
+  memset(&P, 0, sizeof(P));
+  const float* theta0 = experts[first].theta;
+  CUR_TRY(act_common(P, d, theta0, o, ag, g, td, clip_obs, out_pi, out_q, seq));
+  for (int i = 0; i < P.nchunks; ++i) {
+    P.coff[i] = (int32_t)(P.chunks[i].src - theta0);
+    P.chunks[i].src = nullptr;
+  }
+  int base[CUR_MAX_TASKS], fill[CUR_MAX_TASKS] = {0}, tiles = 0;
+  for (int e = 0; e < n_experts; ++e) {
+    base[e] = tiles;
+    tiles += (count[e] + S_ROWS - 1) / S_ROWS;
+    if (count[e] == 0) continue;
+    ActExpert& E = P.ex[e];
+    E.theta = experts[e].theta;
+    E.o_mean = experts[e].stats.o_mean; E.o_std = experts[e].stats.o_std;
+    E.g_mean = experts[e].stats.g_mean; E.g_std = experts[e].stats.g_std;
+    act_net_ptrs(E, *d, E.theta);
+  }
+  for (int t = 0; t < tiles; ++t)
+    for (int r = 0; r < S_ROWS; ++r) P.tile_row[t][r] = -1;
+  for (int64_t i = 0; i < n; ++i) {
+    const int e = row_expert[i], k = fill[e]++;
+    P.tile_ex[base[e] + k / S_ROWS] = (uint8_t)e;
+    P.tile_row[base[e] + k / S_ROWS][k % S_ROWS] = (int16_t)i;
+  }
+  const int H = d->hidden;
+  if (H == 64) CUR_TRY(launch_actions<64>((unsigned)tiles, (cudaStream_t)stream, P));
+  else if (H == 128) CUR_TRY(launch_actions<128>((unsigned)tiles, (cudaStream_t)stream, P));
+  else CUR_TRY(launch_actions<256>((unsigned)tiles, (cudaStream_t)stream, P));
+  CUR_CHECK_LAUNCH();
   return CUR_OK;
 }
 

@@ -196,17 +196,14 @@ static int grid_for(int64_t n, int threads, int max_waves = 4) {
 // action array is updated in place by float64 operands), rounded to float32 where the reference's `+=` rounds.
 constexpr uint32_t ACTION_NOISE_TAG = 0x40000000u;
 
-__global__ void action_noise_kernel(float* __restrict__ u, int64_t n, int dimu, float max_u, double noise_eps,
-                                    double random_eps, uint64_t seed, uint64_t call) {
-  const int pairs = (dimu + 1) / 2;
-  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= n * pairs) return;
-  const int64_t r = idx / pairs;
-  const int p = (int)(idx - r * pairs);
+// components 2p, 2p + 1 of row r of u; `ctr` is the row's counter word (its row number in the call)
+__device__ __forceinline__ void action_noise_pair(float* __restrict__ u, int64_t r, uint32_t ctr, int p, int dimu,
+                                                  float max_u, double noise_eps, double random_eps, uint64_t seed,
+                                                  uint64_t call) {
   const uint32_t c2 = (uint32_t)call, c3 = (uint32_t)(call >> 32) ^ ACTION_NOISE_TAG;
   const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-  const Philox x = philox4x32_10((uint32_t)r, (uint32_t)p, c2, c3, k0, k1);
-  const Philox b = philox4x32_10((uint32_t)r, 0xFFFFFFFFu, c2, c3, k0, k1);
+  const Philox x = philox4x32_10(ctr, (uint32_t)p, c2, c3, k0, k1);
+  const Philox b = philox4x32_10(ctr, 0xFFFFFFFFu, c2, c3, k0, k1);
   const bool explore = u01_from_u32(b.x[0]) < random_eps;                       // binomial(1, random_eps)
   const double rad = sqrt(-2.0 * log(u01_from_u32(x.x[0])));
   const double ang = 6.283185307179586 * u01_from_u32(x.x[1]);
@@ -225,6 +222,29 @@ __global__ void action_noise_kernel(float* __restrict__ u, int64_t n, int dimu, 
     }
     u[r * dimu + k] = v;
   }
+}
+
+__global__ void action_noise_kernel(float* __restrict__ u, int64_t n, int dimu, float max_u, double noise_eps,
+                                    double random_eps, uint64_t seed, uint64_t call) {
+  const int pairs = (dimu + 1) / 2;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n * pairs) return;
+  const int64_t r = idx / pairs;
+  const int p = (int)(idx - r * pairs);
+  action_noise_pair(u, r, (uint32_t)r, p, dimu, max_u, noise_eps, random_eps, seed, call);
+}
+
+// Per-row keys: row r gets exactly what a one-row call cur_action_noise(u + r * dimu, 1, ..., seed[r], call[r]) gives it
+// (counter row 0), so one launch stands for a loop of one-row get_actions calls of different agents.
+__global__ void action_noise_rows_kernel(float* __restrict__ u, int64_t n, int dimu, float max_u, double noise_eps,
+                                         double random_eps, const uint64_t* __restrict__ seed,
+                                         const uint64_t* __restrict__ call) {
+  const int pairs = (dimu + 1) / 2;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n * pairs) return;
+  const int64_t r = idx / pairs;
+  const int p = (int)(idx - r * pairs);
+  action_noise_pair(u, r, 0u, p, dimu, max_u, noise_eps, random_eps, seed[r], call[r]);
 }
 
 }  // namespace cur
@@ -345,6 +365,19 @@ extern "C" int cur_action_noise(void* stream, float* u, int64_t n, int dimu, flo
   if (n == 0) return CUR_OK;
   const int64_t threads = n * ((dimu + 1) / 2);
   action_noise_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+      u, n, dimu, max_u, noise_eps, random_eps, seed, call);
+  CUR_CHECK_LAUNCH();
+  return CUR_OK;
+}
+
+extern "C" int cur_action_noise_rows(void* stream, float* u, int64_t n, int dimu, float max_u, double noise_eps,
+                                     double random_eps, const uint64_t* seed, const uint64_t* call) {
+  CUR_REQUIRE(u && seed && call, "NULL argument");
+  CUR_REQUIRE(n >= 0 && n < (1ll << 32) && dimu > 0, "bad shape");
+  CUR_REQUIRE(noise_eps >= 0.0 && random_eps >= 0.0 && random_eps <= 1.0, "bad noise parameters");
+  if (n == 0) return CUR_OK;
+  const int64_t threads = n * ((dimu + 1) / 2);
+  action_noise_rows_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
       u, n, dimu, max_u, noise_eps, random_eps, seed, call);
   CUR_CHECK_LAUNCH();
   return CUR_OK;

@@ -367,11 +367,13 @@ class DDPG(object):
             self._action_slots[n] = slot
         return slot
 
-    def _actions_one_launch(self, o, ag, g, task_descr, n, theta, compute_Q, device_noise, noise_eps, random_eps):
+    def _actions_one_launch(self, o, ag, g, task_descr, n, theta, compute_Q, device_noise, noise_eps, random_eps,
+                            route=None):
         """cur_ddpg_actions_rows: inputs read from / actions written to mapped pinned memory by the kernel; completion =
         every output word carries this call's number (no copies, no stream synchronisation, no fence).  Returns
         (result, finished): the finished get_actions result on the zero-copy path (post-processing included), else the
-        flat [pi | q] host array that `_finish_actions` still has to post-process."""
+        flat [pi | q] host array that `_finish_actions` still has to post-process.  `route` (experts._Route): the rows
+        go to several experts of this shape in one routed launch, with its own noise pass and host draws."""
         lib = _lib.load()
         slot = self._action_slot(n)
         np.copyto(slot['o'], o.reshape(-1))
@@ -396,28 +398,37 @@ class DDPG(object):
                            'cur_copy_h2d')
                 base = slot['dev_in'].data_ptr()
             rel = lambda name: base + (slot[name] - slot['d_o'])
-            _lib.check(lib.cur_ddpg_actions_rows(
-                _lib.stream_ptr(), C.byref(self.net.desc), theta.data_ptr(), C.byref(self._stats), base,
-                rel('d_ag') if self.relative_goals else None, rel('d_g'), rel('d_td') if self.modular else None, n,
-                float(self.clip_obs), out.data_ptr(), out.data_ptr() + 4 * n * self.dimu if compute_Q else None, 0),
-                'cur_ddpg_actions_rows')
-            if noisy:
+            ptrs = (base, rel('d_ag') if self.relative_goals else None, rel('d_g'), rel('d_td') if self.modular else None,
+                    n, float(self.clip_obs), out.data_ptr(), out.data_ptr() + 4 * n * self.dimu if compute_Q else None, 0)
+            if route is None:
+                _lib.check(lib.cur_ddpg_actions_rows(_lib.stream_ptr(), C.byref(self.net.desc), theta.data_ptr(),
+                                                     C.byref(self._stats), *ptrs), 'cur_ddpg_actions_rows')
+            else:
+                route.launch(*ptrs)
+            if noisy and route is None:
                 _lib.check(lib.cur_action_noise(_lib.stream_ptr(), out.data_ptr(), n, self.dimu, float(self.max_u),
                                                 float(noise_eps), float(random_eps), int(self.noise_seed) & (2 ** 64 - 1),
                                                 self._action_calls), 'cur_action_noise')
+            elif noisy:
+                route.noise(out.data_ptr(), n, noise_eps, random_eps)
             return out[:n_out].cpu().numpy(), False
         slot['seq'] = seq = slot['seq'] % 0xFFFFFFF0 + 1
-        desc_ref, stats_ref = slot['refs']
-        _lib.check(lib.cur_ddpg_actions_rows(
-            _lib.stream_ptr(), desc_ref, theta.data_ptr(), stats_ref, slot['d_o'],
-            slot['d_ag'] if self.relative_goals else None, slot['d_g'], slot['d_td'] if self.modular else None, n,
-            float(self.clip_obs), slot['d_out'], slot['d_q'] if compute_Q else None, seq), 'cur_ddpg_actions_rows')
+        if route is None:
+            desc_ref, stats_ref = slot['refs']
+            _lib.check(lib.cur_ddpg_actions_rows(
+                _lib.stream_ptr(), desc_ref, theta.data_ptr(), stats_ref, slot['d_o'],
+                slot['d_ag'] if self.relative_goals else None, slot['d_g'], slot['d_td'] if self.modular else None, n,
+                float(self.clip_obs), slot['d_out'], slot['d_q'] if compute_Q else None, seq), 'cur_ddpg_actions_rows')
+        else:
+            route.launch(slot['d_o'], slot['d_ag'] if self.relative_goals else None, slot['d_g'],
+                         slot['d_td'] if self.modular else None, n, float(self.clip_obs), slot['d_out'],
+                         slot['d_q'] if compute_Q else None, seq)
         # The host RNG draws of ddpg.py:148-151 do not depend on the kernel's answer: take them (in reference order) while
         # the launch is in flight - ~10 us of NumPy calls hidden behind ~15 us of launch latency + weight stream.  The
         # arithmetic on the answer is one C call (cur_actions_finish_host: poll the words, NumPy's own evaluation types).
         p_randn = p_explore = p_u_rand = None
         if not device_noise:
-            randn, explore, u_rand = self._draw_action_noise(n, random_eps)
+            randn, explore, u_rand = (self._draw_action_noise if route is None else route.draw)(n, random_eps)
             np.copyto(slot['randn'], randn)
             np.copyto(slot['explore'], explore)
             np.copyto(slot['u_rand'], u_rand)
@@ -508,12 +519,13 @@ class DDPG(object):
         binomial (which rows act randomly), uniform (_random_action) - also when the eps are 0, like the reference."""
         return np.random.randn(n, self.dimu), np.random.binomial(1, random_eps, n), self._random_action(n)
 
-    def _finish_actions(self, res, n, compute_Q, device_noise, noise_eps, random_eps):
+    def _finish_actions(self, res, n, compute_Q, device_noise, noise_eps, random_eps, draw=None):
         """Action postprocessing (ddpg.py:147-155) on the flat [pi | q] host array `res` (owned by this call); the
-        zero-copy path does the same arithmetic in cur_actions_finish_host (compared in tests/test_host_logic.py)."""
+        zero-copy path does the same arithmetic in cur_actions_finish_host (compared in tests/test_host_logic.py).
+        `draw`: the host draws, when they are not this agent's _draw_action_noise (a routed expert step)."""
         u = res[:n * self.dimu].reshape(n, self.dimu)
         if not device_noise:
-            randn, explore, u_rand = self._draw_action_noise(n, random_eps)
+            randn, explore, u_rand = (draw or self._draw_action_noise)(n, random_eps)
             u += noise_eps * self.max_u * randn                                             # ddpg.py:148-149
             lim = self.max_u
             np.minimum(np.maximum(u, -lim, out=u), lim, out=u)                              # np.clip, ddpg.py:150

@@ -10,9 +10,14 @@ cur_ddpg_chain_grads_group instead: their chain kernels side by side, their K-sl
 Semantically it is `for p in policies: p.train()` - every expert keeps its own parameters, Adam state, Philox
 stream, LP apportioning and buffers, and the result is bit-identical to stepping them one after the other on the
 levels schedule, or on the narrow chain for native experts.
+
+Acting (`get_actions`, the evaluation step of the experts, rollout.py:211-223) routes each row to the expert of its
+module in ONE launch (cur_ddpg_actions_rows_group): bit for bit the loop of one-row get_actions calls it stands for,
+np.random stream and device-noise counters included.
 """
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -39,6 +44,24 @@ class TaskExperts(object):
         self.use_cuda_graph = use_cuda_graph
         self._graph = None
         self._experts = None
+
+    @staticmethod
+    def router(policies):
+        """A TaskExperts over `policies` when they are DDPG agents of one network shape on one device (their evaluation
+        step can then be one routed launch); None for any other list."""
+        from .ddpg import DDPG
+        if isinstance(policies, TaskExperts):
+            return policies
+        if not isinstance(policies, (list, tuple)):
+            return None
+        ps = list(policies)
+        if not ps or len(ps) > _lib.CUR_MAX_TASKS or not all(isinstance(p, DDPG) for p in ps):
+            return None
+        p0 = ps[0]
+        if not all(bytes(p.net.desc) == bytes(p0.net.desc) and p.batch_size == p0.batch_size and p.device == p0.device
+                   for p in ps):
+            return None
+        return TaskExperts(ps)
 
     def __len__(self):
         return len(self.policies)
@@ -173,3 +196,93 @@ class TaskExperts(object):
     def update_target_net(self):
         for p in self.policies:
             p.update_target_net()
+
+    # ------------------------------------------------------------------------------------------ acting
+    def _routed_ok(self):
+        """Every expert would take the one-launch action path, and the options the launch shares agree."""
+        ps = self.policies
+        p0 = ps[0]
+        return len(ps) <= _lib.CUR_MAX_TASKS and all(
+            p._action_rows_ok() and (p.clip_obs, p.relative_goals, p.modular, p.action_noise) ==
+            (p0.clip_obs, p0.relative_goals, p0.modular, p0.action_noise) for p in ps)
+
+    def get_actions(self, o, ag, g, task_descr, noise_eps=0., random_eps=0., use_target_net=False, compute_Q=False):
+        """Each row acted on by policies[argmax(task_descr[row])] (rollout.py:211-223).  Returns u float64 [n, dimu], and
+        with compute_Q [u, q float64 [n, 1]]: exactly what a loop of one-row get_actions calls builds, including the
+        np.random draws (per row: randn, binomial, uniform) and every expert's device-noise counter.  Up to
+        ACTION_ROWS_MAX rows of experts on the one-launch path: ONE routed launch (cur_ddpg_actions_rows_group);
+        otherwise that loop."""
+        p0 = self.policies[0]
+        o = np.asarray(o, np.float32).reshape(-1, p0.dimo)
+        n = o.shape[0]
+        g = np.asarray(g, np.float32).reshape(n, p0.dimg)
+        td = np.asarray(task_descr, np.float32).reshape(n, -1)
+        which = np.argmax(td, axis=1).astype(np.int32)
+        if n > p0.ACTION_ROWS_MAX or not self._routed_ok():
+            return self._actions_loop(o, ag, g, td, which, noise_eps, random_eps, use_target_net, compute_Q)
+        device_noise = p0.action_noise == 'device'
+        route = _Route(self.policies, which, use_target_net)
+        res, finished = p0._actions_one_launch(o, ag, g, td, n, None, compute_Q, device_noise, noise_eps, random_eps,
+                                               route=route)
+        if device_noise:                                   # one call per row in the loop
+            for p, c in zip(self.policies, np.bincount(which, minlength=len(self.policies))):
+                p._action_calls += int(c)
+        if not finished:
+            res = p0._finish_actions(res, n, compute_Q, device_noise, noise_eps, random_eps, draw=route.draw)
+        u = np.asarray(res[0] if compute_Q else res, np.float64).reshape(n, p0.dimu)
+        return [u, np.asarray(res[1], np.float64).reshape(n, 1)] if compute_Q else u
+
+    def _actions_loop(self, o, ag, g, td, which, noise_eps, random_eps, use_target_net, compute_Q):
+        """One get_actions call per row, by the row's expert (rollout.py:211-223)."""
+        n = len(o)
+        u = np.zeros((n, self.policies[0].dimu))
+        q = np.zeros((n, 1))
+        for i in range(n):
+            out = self.policies[which[i]].get_actions(
+                o[i:i + 1], None if ag is None else ag[i:i + 1], g[i:i + 1], task_descr=td[i:i + 1], noise_eps=noise_eps,
+                random_eps=random_eps, use_target_net=use_target_net, compute_Q=compute_Q)
+            if compute_Q:
+                u[i], q[i, 0] = out[0], np.asarray(out[1]).reshape(-1)[0]
+            else:
+                u[i] = out
+        return [u, q] if compute_Q else u
+
+
+class _Route(object):
+    """One routed action launch as DDPG._actions_one_launch asks for it: the launch (cur_ddpg_actions_rows_group), the
+    device-side noise pass and the host draws, each as the loop of one-row calls would have made them."""
+
+    def __init__(self, policies, which, use_target_net):
+        self.policies, self.which = policies, which
+        self.arr = (_lib.ActionsExpert * len(policies))()
+        for e, p in zip(self.arr, policies):
+            e.theta = (p.theta_target if use_target_net else p.theta_main).data_ptr()
+            e.stats = p._stats
+
+    def launch(self, o, ag, g, td, n, clip_obs, out_pi, out_q, seq):
+        ps = self.policies
+        _lib.check(_lib.load().cur_ddpg_actions_rows_group(
+            _lib.stream_ptr(), C.byref(ps[0].net.desc), len(ps), self.arr, self.which.ctypes.data, o, ag, g, td, n,
+            clip_obs, out_pi, out_q, seq), 'cur_ddpg_actions_rows_group')
+
+    def noise(self, out, n, noise_eps, random_eps):
+        """Row i is the k-th one-row call of its expert in this step: Philox key = the expert's noise_seed, call number =
+        its _action_calls + k (cur_action_noise_rows)."""
+        ps = self.policies
+        keys = np.empty((2, n), np.uint64)
+        taken = [0] * len(ps)
+        for i, e in enumerate(self.which):
+            p = ps[e]
+            keys[0, i] = int(p.noise_seed) & (2 ** 64 - 1)
+            keys[1, i] = p._action_calls + taken[e]
+            taken[e] += 1
+        dev = torch.from_numpy(keys.view(np.int64)).to(ps[0].device)
+        p0 = ps[0]
+        _lib.check(_lib.load().cur_action_noise_rows(_lib.stream_ptr(), out, n, p0.dimu, float(p0.max_u), float(noise_eps),
+                                                     float(random_eps), dev[0].data_ptr(), dev[1].data_ptr()),
+                   'cur_action_noise_rows')
+
+    def draw(self, n, random_eps):
+        """The host draws of the loop: per row, the row's expert's _draw_action_noise(1, random_eps)."""
+        rows = [self.policies[e]._draw_action_noise(1, random_eps) for e in self.which]
+        return tuple(np.concatenate([r[k] for r in rows]) for k in range(3))

@@ -125,6 +125,10 @@ class RolloutWorker(object):
                   random_eps=0. if quiet else self.random_eps, use_target_net=self.use_target_net)
         if self.structure == 'task_experts' and self.eval:
             # evaluation of experts: the expert of the demanded task acts (rollout.py:211-223)
+            experts = self._expert_router()
+            if experts is not None:             # one routed launch, bit for bit the loop below
+                out = experts.get_actions(o, ag, self.g, self.task_descr, **kw)
+                return (out[0], out[1]) if self.compute_Q else (out, None)
             u = np.zeros((len(o), self.dims['u']))
             q = np.zeros((len(o), 1))
             for i in range(len(o)):
@@ -138,6 +142,13 @@ class RolloutWorker(object):
         out = self.policy.get_actions(o, ag, self.g, task_descr=self.task_descr if self.modular else None, **kw)
         u, q = (out if self.compute_Q else (out, None))
         return np.asarray(u).reshape(len(o), -1), q
+
+    def _expert_router(self):
+        """experts.TaskExperts over the policy list when it is made of DDPG agents of one shape, else None (the loop)."""
+        if getattr(self, '_router', (None,))[0] is not self.policy:
+            from .experts import TaskExperts
+            self._router = (self.policy, TaskExperts.router(self.policy))
+        return self._router[1]
 
     def generate_rollouts(self):
         """`rollout_batch_size` episodes of T steps with the current policy (rollout.py:178-406).

@@ -283,6 +283,22 @@ int cur_ddpg_actions(void* stream, const cur_net_desc* d, const float* theta,
 int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
                           const float* o, const float* ag /* or NULL */, const float* g, const float* td, int64_t n,
                           float clip_obs, void* out_pi, void* out_q /* or NULL */, uint32_t seq);
+/* The routed form of cur_ddpg_actions_rows for a task-experts evaluation step: row i is acted on by
+ * experts[row_expert[i]] (its main or target theta and its normaliser statistics), all experts of one shape `d`.  One
+ * launch: the rows of each expert fill whole 4-row CTA tiles, and every output lands at the row's original position, in
+ * the same two forms (seq == 0: float32; seq != 0: {float32 bits | seq << 32} words for cur_actions_finish_host).
+ * row_expert is a HOST array of n entries; the other pointers follow cur_ddpg_actions_rows.  Refused before any launch:
+ * n_experts outside 1..CUR_MAX_TASKS, a row_expert entry outside 0..n_experts-1, a shape cur_ddpg_rows_supported(d, 4)
+ * refuses, n outside 1..CUR_ACTIONS_GROUP_MAX_ROWS. */
+#define CUR_ACTIONS_GROUP_MAX_ROWS 512
+typedef struct cur_actions_expert {
+  const float* theta;
+  cur_norm_stats stats;            /* may hold NULLs when normalize_obs == 0 */
+} cur_actions_expert;
+int cur_ddpg_actions_rows_group(void* stream, const cur_net_desc* d, int n_experts, const cur_actions_expert* experts,
+                                const int32_t* row_expert, const float* o, const float* ag /* or NULL */, const float* g,
+                                const float* td, int64_t n, float clip_obs, void* out_pi, void* out_q /* or NULL */,
+                                uint32_t seq);
 /* Host-side tail of a seq != 0 call of cur_ddpg_actions_rows (ddpg.py:147-155): polls the n * dimu (+ n with_q) output
  * words in the mapped buffer until all carry `seq`, then applies the reference's exploration post-processing with the
  * caller's np.random draws (randn [n, dimu] float64, explore [n] int64 = binomial(1, random_eps), u_rand [n, dimu] float64 =
@@ -307,6 +323,11 @@ int cur_copy_h2d(void* stream, void* dst, const void* src, int64_t bytes);
  * The default path keeps the noise on the host (the caller's np.random stream, like the reference). */
 int cur_action_noise(void* stream, float* u, int64_t n, int dimu, float max_u, double noise_eps,
                      double random_eps, uint64_t seed, uint64_t call);
+/* The same noise with per-row keys: row r gets what the one-row call cur_action_noise(u + r * dimu, 1, ..., seed[r],
+ * call[r]) would give it (counter row 0).  seed / call: n entries each, readable by the device (device memory or
+ * mapped pinned host memory).  Stands for a loop of one-row get_actions calls of different agents. */
+int cur_action_noise_rows(void* stream, float* u, int64_t n, int dimu, float max_u, double noise_eps,
+                          double random_eps, const uint64_t* seed, const uint64_t* call);
 
 typedef struct cur_batch {
   const float *o, *g, *u, *td, *o_2, *g_2, *r; /* staged batch (ddpg.py:75-83); td NULL if flat */
