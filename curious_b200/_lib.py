@@ -15,6 +15,7 @@ CUR_MAX_TASKS = 16
 CUR_MAX_SLICE = 8
 CUR_MAX_SEGMENTS = 17
 CUR_MAX_COPIES = 64
+CUR_MAX_WORKERS = 64
 
 MODE_BUFFER, MODE_RANDOM_TASK, MODE_CP_TASK, MODE_CURRENT_TASK, MODE_FLAT = range(5)
 
@@ -69,6 +70,15 @@ class HerArgs(C.Structure):
                 ('td', C.c_void_p), ('change', C.c_void_p), ('info', C.c_void_p), ('o_2', C.c_void_p),
                 ('ag_2', C.c_void_p), ('g_2', C.c_void_p), ('r', C.c_void_p), ('idx_out', C.c_void_p),
                 ('dyn', C.c_void_p)]
+
+
+class HerWorker(C.Structure):
+    _fields_ = [('seed', C.c_uint64), ('n_segments', C.c_int32), ('_pad', C.c_int32), ('seg', Segment * CUR_MAX_SEGMENTS)]
+
+
+class HerWorkerDyn(C.Structure):
+    _fields_ = [('n_episodes', C.c_int32 * CUR_MAX_SEGMENTS), ('count', C.c_int32 * CUR_MAX_SEGMENTS),
+                ('cdf', C.c_double * CUR_MAX_TASKS)]
 
 
 class NetDesc(C.Structure):
@@ -140,6 +150,8 @@ SIGNATURES = {
                                      C.POINTER(C.c_int32), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                      C.POINTER(C.c_int64)]),
     'cur_her_sample': (C.c_int, [C.c_void_p, C.POINTER(HerArgs)]),
+    'cur_her_sample_workers': (C.c_int, [C.c_void_p, C.POINTER(HerArgs), C.c_int, C.c_int, C.POINTER(HerWorker),
+                                         C.c_void_p, C.c_void_p]),
     'cur_philox4x32_10': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     'cur_norm_accumulate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
     'cur_norm_recompute': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_int,

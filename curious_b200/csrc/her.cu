@@ -119,13 +119,11 @@ __device__ __forceinline__ void emit2(float* __restrict__ outa, float* __restric
 //   (o, o_2, u, ag, ag_2, change, info: warps 1 - 3) | the relabelled outputs (g, g_2, task_descr: all warps).
 // (A persistent double-buffered variant - draws and gather of tile i+1 issued before tile i is waited for - was measured
 // slower, 70 % vs 81 % of the HBM peak: throughput follows the number of resident tiles per SM, profiles/README.md.)
-template <int TILE, int HER_THREADS>
-__global__ void __launch_bounds__(HER_THREADS)
-her_sample_kernel(const __grid_constant__ HerKernelParams P) {
+// draw(j, row, src): her_draw_row of output row j (her_draw_row_worker in the worker-major form).
+template <int TILE, int HER_THREADS, class Draw>
+__device__ __forceinline__ void her_tile(const cur_her_args& a, const HerPlan& pl, Draw draw) {
   constexpr int HER_WARPS = HER_THREADS / 32;
-  const cur_her_args& a = P.a;
   const cur_layout& L = a.L;
-  const HerPlan& pl = P.p;
   extern __shared__ __align__(128) unsigned char smem_raw[];
 
   float* stage = reinterpret_cast<float*>(smem_raw);                              // TILE * stage_stride
@@ -142,7 +140,7 @@ her_sample_kernel(const __grid_constant__ HerKernelParams P) {
   // ---------------------------------------------------------------- phase A: draws (warp 0)
   HerRow row;
   row.ft = -1; row.choice = -1; row.ep = 0; row.t = 0; row.ttr = -1; row.her = false;
-  if (warp == 0 && lane < nrows) her_draw_row(a, pl, j0 + lane, row, m_src + 3 * lane);
+  if (warp == 0 && lane < nrows) draw(j0 + lane, row, m_src + 3 * lane);
   __syncthreads();
 
   // ---------------------------------------------------------------- copies: global -> shared
@@ -238,6 +236,35 @@ her_sample_kernel(const __grid_constant__ HerKernelParams P) {
           [&](int tr, int k) { return clip1(stage[tr * ss + iG + k]); },
           [&](int tr, int k) { return clip1(stage[tr * ss + iG + k]); });
   }
+}
+
+template <int TILE, int HER_THREADS>
+__global__ void __launch_bounds__(HER_THREADS)
+her_sample_kernel(const __grid_constant__ HerKernelParams P) {
+  const cur_her_args& a = P.a;
+  const HerPlan& pl = P.p;
+  her_tile<TILE, HER_THREADS>(a, pl, [&](int64_t j, HerRow& row, const float** src) { her_draw_row(a, pl, j, row, src); });
+}
+
+struct HerWorkersParams {
+  cur_her_args a;
+  HerPlan p;
+  int32_t rows_per_worker;
+  const cur_her_worker_dyn* dyn;
+  const int64_t* step;
+  HerWorkerTab w[CUR_MAX_WORKERS];
+};
+static_assert(sizeof(HerWorkersParams) <= 32764, "kernel parameter limit");
+
+// cur_her_sample_workers: the tile of her_sample_kernel, each row drawn from its worker's segments and stream.
+template <int TILE, int HER_THREADS>
+__global__ void __launch_bounds__(HER_THREADS)
+her_sample_workers_kernel(const __grid_constant__ HerWorkersParams P) {
+  const cur_her_args& a = P.a;
+  const HerPlan& pl = P.p;
+  her_tile<TILE, HER_THREADS>(a, pl, [&](int64_t j, HerRow& row, const float** src) {
+    her_draw_row_worker(a, pl, j, P.rows_per_worker, P.w, P.dyn, P.step, row, src);
+  });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -377,30 +404,12 @@ extern "C" int cur_store_episodes(void* stream, const cur_layout* L, const cur_e
   return CUR_OK;
 }
 
-extern "C" int cur_her_sample(void* stream, const cur_her_args* args) {
-  CUR_REQUIRE(args != nullptr, "args is NULL");
-  const cur_her_args& a = *args;
-  CUR_REQUIRE(a.batch >= 0, "negative batch");
-  if (a.batch == 0) return CUR_OK;
-  CUR_REQUIRE(a.n_segments >= 1 && a.n_segments <= CUR_MAX_SEGMENTS, "n_segments out of range");
+// Checks shared by both sampling entries: mode, reward table, injected stream, relative goals.
+static int check_her_common(const cur_her_args& a) {
   CUR_REQUIRE(a.mode >= CUR_MODE_BUFFER && a.mode <= CUR_MODE_FLAT, "unknown mode");
   CUR_REQUIRE(a.tasks.n_tasks >= 0 && a.tasks.n_tasks <= CUR_MAX_TASKS, "n_tasks out of range");
   CUR_REQUIRE(a.mode == CUR_MODE_FLAT || a.tasks.n_tasks == a.L.dimtd, "n_tasks must equal dimtd");
   CUR_REQUIRE(a.L.row_stride > 0 && (a.L.row_stride & 3) == 0, "layout not initialised");
-  int64_t total = 0;
-  for (int i = 0; i < a.n_segments; ++i) {
-    CUR_REQUIRE(a.seg[i].count >= 0, "negative segment count");
-    if (a.dyn != nullptr) {
-      CUR_REQUIRE(a.seg[i].base != nullptr, "segment base is NULL");
-    } else if (a.seg[i].count > 0) {
-      CUR_REQUIRE(a.seg[i].base != nullptr, "segment base is NULL");
-      CUR_REQUIRE(a.seg[i].n_episodes > 0, "sampling from an empty buffer (replay_buffer.py:43)");
-      CUR_REQUIRE(a.seg[i].task_to_replay < a.tasks.n_tasks, "task_to_replay out of range");
-    }
-    total += a.seg[i].count;
-  }
-  CUR_REQUIRE(a.dyn != nullptr || total == a.batch, "segment counts must sum to batch (ddpg.py:323)");
-  CUR_REQUIRE(a.dyn == nullptr || a.inj_ep == nullptr, "a device control block implies Philox draws");
   for (int m = 0; m < a.tasks.n_tasks; ++m) {
     CUR_REQUIRE(a.tasks.len[m] >= 0 && a.tasks.len[m] <= CUR_MAX_SLICE, "module slice too long");
     for (int k = 0; k < a.tasks.len[m]; ++k) {
@@ -416,6 +425,49 @@ extern "C" int cur_her_sample(void* stream, const cur_her_args* args) {
   if (a.inj_ep != nullptr)
     CUR_REQUIRE(a.inj_t && a.inj_u_her && a.inj_u_off, "incomplete injected stream");
   if (a.relative_goals) CUR_REQUIRE(a.L.dimg == a.L.dimag, "relative goals need dimg == dimag");
+  return CUR_OK;
+}
+
+// CTA shape: 32 rows / 128 threads.  16 / 64 and 32 / 64 measured the same (Arm4 0.827 / 0.828 vs 0.830 of the HBM peak),
+// 16 / 128 slower (0.655): at full size the kernel sits at the DRAM pipe, not at its own latency (profiles/README.md)
+constexpr int HER_TILE = 32, HER_THREADS = 128;
+
+template <class Params>
+static int launch_her(void (*kernel)(Params), const Params& P, int64_t batch, cudaStream_t stream, size_t* configured) {
+  size_t smem = (size_t)HER_TILE * P.p.stage_stride * 4 + 3 * HER_TILE * sizeof(void*) + 16;
+  if (smem > 48 * 1024 && smem > *configured) {
+    CUR_REQUIRE(smem <= 227 * 1024, "row too large for the shared-memory stage");
+    CUR_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    *configured = smem;
+  }
+  const int64_t blocks = (batch + HER_TILE - 1) / HER_TILE;
+  CUR_REQUIRE(blocks <= 0x7fffffff, "batch too large for one launch");
+  kernel<<<(unsigned)blocks, HER_THREADS, smem, stream>>>(P);
+  CUR_CHECK_LAUNCH();
+  return CUR_OK;
+}
+
+extern "C" int cur_her_sample(void* stream, const cur_her_args* args) {
+  CUR_REQUIRE(args != nullptr, "args is NULL");
+  const cur_her_args& a = *args;
+  CUR_REQUIRE(a.batch >= 0, "negative batch");
+  if (a.batch == 0) return CUR_OK;
+  CUR_REQUIRE(a.n_segments >= 1 && a.n_segments <= CUR_MAX_SEGMENTS, "n_segments out of range");
+  if (int st = check_her_common(a)) return st;
+  int64_t total = 0;
+  for (int i = 0; i < a.n_segments; ++i) {
+    CUR_REQUIRE(a.seg[i].count >= 0, "negative segment count");
+    if (a.dyn != nullptr) {
+      CUR_REQUIRE(a.seg[i].base != nullptr, "segment base is NULL");
+    } else if (a.seg[i].count > 0) {
+      CUR_REQUIRE(a.seg[i].base != nullptr, "segment base is NULL");
+      CUR_REQUIRE(a.seg[i].n_episodes > 0, "sampling from an empty buffer (replay_buffer.py:43)");
+      CUR_REQUIRE(a.seg[i].task_to_replay < a.tasks.n_tasks, "task_to_replay out of range");
+    }
+    total += a.seg[i].count;
+  }
+  CUR_REQUIRE(a.dyn != nullptr || total == a.batch, "segment counts must sum to batch (ddpg.py:323)");
+  CUR_REQUIRE(a.dyn == nullptr || a.inj_ep == nullptr, "a device control block implies Philox draws");
 
   HerKernelParams P;
   P.a = a;
@@ -423,22 +475,48 @@ extern "C" int cur_her_sample(void* stream, const cur_her_args* args) {
   if (P.p.cold4 > 0)
     for (int i = 0; i < a.n_segments; ++i)
       CUR_REQUIRE(a.seg[i].count == 0 || a.seg[i].cold != nullptr, "change/info/ag requested but segment has no cold rows");
-  // CTA shape: 32 rows / 128 threads.  16 / 64 and 32 / 64 measured the same (Arm4 0.827 / 0.828 vs 0.830 of the HBM peak),
-  // 16 / 128 slower (0.655): at full size the kernel sits at the DRAM pipe, not at its own latency (profiles/README.md)
-  constexpr int TILE = 32, THREADS = 128;
-  size_t smem = (size_t)TILE * P.p.stage_stride * 4 + 3 * TILE * sizeof(void*) + 16;
   static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    CUR_REQUIRE(smem <= 227 * 1024, "row too large for the shared-memory stage");
-    CUR_CUDA_TRY(cudaFuncSetAttribute(her_sample_kernel<TILE, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)smem));
-    configured = smem;
+  return launch_her(her_sample_kernel<HER_TILE, HER_THREADS>, P, a.batch, (cudaStream_t)stream, &configured);
+}
+
+extern "C" int cur_her_sample_workers(void* stream, const cur_her_args* args, int n_workers, int rows_per_worker,
+                                      const cur_her_worker* w, const cur_her_worker_dyn* dyn, const int64_t* step) {
+  CUR_REQUIRE(args != nullptr && w != nullptr && dyn != nullptr, "NULL argument");
+  CUR_REQUIRE(n_workers >= 1 && n_workers <= CUR_MAX_WORKERS, "n_workers out of range (1..CUR_MAX_WORKERS)");
+  CUR_REQUIRE(rows_per_worker >= 1, "rows_per_worker must be positive");
+  const cur_her_args& a = *args;
+  CUR_REQUIRE(a.batch == (int64_t)n_workers * rows_per_worker, "batch must equal n_workers * rows_per_worker");
+  if (int st = check_her_common(a)) return st;
+  HerWorkersParams P;
+  P.a = a;
+  make_plan(a, &P.p);
+  for (int j = 0; j < n_workers; ++j) {
+    const cur_her_worker& wj = w[j];
+    CUR_REQUIRE(wj.n_segments >= 1 && wj.n_segments <= CUR_MAX_SEGMENTS, "a worker has n_segments outside 1..17");
+    int64_t total = 0;
+    HerWorkerTab& t = P.w[j];
+    t.seed = wj.seed;
+    t.n_segments = wj.n_segments;
+    for (int i = 0; i < wj.n_segments; ++i) {
+      const cur_segment& sg = wj.seg[i];
+      CUR_REQUIRE(sg.count >= 0, "negative segment count");
+      CUR_REQUIRE(sg.base != nullptr, "segment base is NULL");
+      CUR_REQUIRE(sg.count == 0 || sg.n_episodes > 0, "sampling from an empty buffer (replay_buffer.py:43)");
+      CUR_REQUIRE(sg.task_to_replay < a.tasks.n_tasks, "task_to_replay out of range");
+      CUR_REQUIRE(P.p.cold4 == 0 || sg.count == 0 || sg.cold != nullptr,
+                  "change/info/ag requested but segment has no cold rows");
+      t.base[i] = sg.base;
+      t.cold[i] = sg.cold;
+      t.ttr[i] = sg.task_to_replay;
+      total += sg.count;
+    }
+    CUR_REQUIRE(total == rows_per_worker, "a worker's segment counts must sum to rows_per_worker");
   }
-  const int64_t blocks = (a.batch + TILE - 1) / TILE;
-  CUR_REQUIRE(blocks <= 0x7fffffff, "batch too large for one launch");
-  her_sample_kernel<TILE, THREADS><<<(unsigned)blocks, THREADS, smem, (cudaStream_t)stream>>>(P);
-  CUR_CHECK_LAUNCH();
-  return CUR_OK;
+  P.rows_per_worker = rows_per_worker;
+  P.dyn = dyn;
+  P.step = step;
+  static size_t configured = 0;
+  return launch_her(her_sample_workers_kernel<HER_TILE, HER_THREADS>, P, a.batch, (cudaStream_t)stream, &configured);
 }
 
 // ---------------------------------------------------------------- known-answer access to the generator

@@ -28,6 +28,51 @@ struct HerRow {
   bool her;
 };
 
+// Draws of one row whose segment is known (base, E episodes): c indexes the injected stream, (ctr, call_offset) is the
+// Philox counter under `seed`; then the three source addresses.  cdf(k): the CP_TASK cdf, cold(): the segment's cold rows.
+template <class Cdf, class Cold>
+__device__ __forceinline__ void her_draw_at(const cur_her_args& a, const HerPlan& pl, int64_t c, int64_t ctr,
+                                            uint64_t call_offset, uint64_t seed, const float* base, int E, HerRow& row,
+                                            const float** src, Cdf cdf, Cold cold) {
+  const cur_layout& L = a.L;
+  double u_her, u_off;
+  if (a.inj_ep != nullptr) {
+    row.ep = a.inj_ep[c];
+    row.t = a.inj_t[c];
+    u_her = a.inj_u_her[c];
+    u_off = a.inj_u_off[c];
+    if (a.inj_choice) row.choice = a.inj_choice[c];
+  } else {
+    Philox x = philox4x32_10((uint32_t)ctr, (uint32_t)(ctr >> 32), (uint32_t)call_offset, (uint32_t)(call_offset >> 32),
+                             (uint32_t)seed, (uint32_t)(seed >> 32));
+    row.ep = (int)mulhi32(x.x[0], (uint32_t)E);
+    row.t = (int)mulhi32(x.x[1], (uint32_t)L.T);
+    u_her = u01_from_u32(x.x[2]);
+    u_off = u01_from_u32(x.x[3]);
+    if (a.mode == CUR_MODE_RANDOM_TASK || a.mode == CUR_MODE_CP_TASK) {
+      Philox y = philox4x32_10((uint32_t)ctr, (uint32_t)(ctr >> 32), (uint32_t)call_offset,
+                               (uint32_t)(call_offset >> 32) ^ 0x80000000u, (uint32_t)seed,
+                               (uint32_t)(seed >> 32));
+      if (a.mode == CUR_MODE_RANDOM_TASK) {
+        row.choice = (int)mulhi32(y.x[0], (uint32_t)a.tasks.n_tasks);
+      } else {
+        // np.random.choice(p=): cdf.searchsorted(u, side='right')
+        double u = u01_from_u32(y.x[0]);
+        int k = 0;
+        while (k < a.tasks.n_tasks - 1 && cdf(k) <= u) ++k;
+        row.choice = k;
+      }
+    }
+  }
+  row.her = u_her < a.future_p;                                                   // her.py:115
+  row.ft = row.her ? row.t + 1 + (int)(u_off * (double)(L.T - row.t)) : -1;       // her.py:116-118
+  const int64_t tr = (int64_t)row.ep * L.T + row.t;
+  src[0] = base + tr * (int64_t)L.trans_stride;
+  // ag(future_t) is the ag(t+1) block of transition future_t - 1 (future_t >= 1)
+  src[1] = row.her ? base + ((int64_t)row.ep * L.T + (row.ft - 1)) * (int64_t)L.trans_stride + pl.iAG2 : nullptr;
+  src[2] = (pl.cold4 > 0) ? cold() + tr * (int64_t)L.cold_stride : nullptr;
+}
+
 // Draws of concat row j (injected stream or Philox), segment lookup, and the three source addresses of the row:
 // src[0] main span, src[1] future achieved goal (NULL: not a HER row), src[2] cold row (NULL: not requested).
 // dyn_copy / step_val (optional): the caller's copy of the device control block and of *dyn->step, fetched up front in two round
@@ -35,7 +80,6 @@ struct HerRow {
 __device__ __forceinline__ void her_draw_row(const cur_her_args& a, const HerPlan& pl, int64_t j, HerRow& row,
                                              const float** src, const cur_her_dyn* dyn_copy = nullptr,
                                              const int64_t* step_val = nullptr) {
-  const cur_layout& L = a.L;
   const int64_t c = a.perm ? (int64_t)a.perm[j] : j;
   // segment lookup: concat rows are the segments' counts laid end to end (ddpg.py:326-345)
   // (with a device control block - CUDA-graph replays - counts / sizes / counter come from memory)
@@ -53,42 +97,43 @@ __device__ __forceinline__ void her_draw_row(const cur_her_args& a, const HerPla
   row.ttr = a.seg[s].task_to_replay;
   row.choice = -1;
   const uint64_t call_offset = a.call_offset + (dyn ? (uint64_t)(step_val ? *step_val : *dyn->step) : 0ull);
-  double u_her, u_off;
-  if (a.inj_ep != nullptr) {
-    row.ep = a.inj_ep[c];
-    row.t = a.inj_t[c];
-    u_her = a.inj_u_her[c];
-    u_off = a.inj_u_off[c];
-    if (a.inj_choice) row.choice = a.inj_choice[c];
-  } else {
-    Philox x = philox4x32_10((uint32_t)c, (uint32_t)(c >> 32), (uint32_t)call_offset, (uint32_t)(call_offset >> 32),
-                             (uint32_t)a.seed, (uint32_t)(a.seed >> 32));
-    row.ep = (int)mulhi32(x.x[0], (uint32_t)E);
-    row.t = (int)mulhi32(x.x[1], (uint32_t)L.T);
-    u_her = u01_from_u32(x.x[2]);
-    u_off = u01_from_u32(x.x[3]);
-    if (a.mode == CUR_MODE_RANDOM_TASK || a.mode == CUR_MODE_CP_TASK) {
-      Philox y = philox4x32_10((uint32_t)c, (uint32_t)(c >> 32), (uint32_t)call_offset,
-                               (uint32_t)(call_offset >> 32) ^ 0x80000000u, (uint32_t)a.seed,
-                               (uint32_t)(a.seed >> 32));
-      if (a.mode == CUR_MODE_RANDOM_TASK) {
-        row.choice = (int)mulhi32(y.x[0], (uint32_t)a.tasks.n_tasks);
-      } else {
-        // np.random.choice(p=): cdf.searchsorted(u, side='right')
-        double u = u01_from_u32(y.x[0]);
-        int k = 0;
-        while (k < a.tasks.n_tasks - 1 && (dyn ? dyn->cdf[k] : a.tasks.cdf[k]) <= u) ++k;
-        row.choice = k;
-      }
-    }
+  her_draw_at(a, pl, c, c, call_offset, a.seed, base, E, row, src,
+              [&](int k) { return dyn ? dyn->cdf[k] : a.tasks.cdf[k]; }, [&]() { return a.seg[s].cold; });
+}
+
+// One worker of cur_her_sample_workers: its Philox key and its own segments (the counts and sizes are read from the
+// worker's device control block).
+struct HerWorkerTab {
+  uint64_t seed;
+  int32_t n_segments;
+  int32_t ttr[CUR_MAX_SEGMENTS];
+  const float* base[CUR_MAX_SEGMENTS];
+  const float* cold[CUR_MAX_SEGMENTS];
+};
+
+// her_draw_row of the worker-major form: concat row c = perm ? perm[j] : j belongs to worker c / rpw at local row
+// i = c % rpw, which is looked up in that worker's segments and drawn at Philox counter (i, call_offset + *step) under its key.
+__device__ __forceinline__ void her_draw_row_worker(const cur_her_args& a, const HerPlan& pl, int64_t j, int rpw,
+                                                    const HerWorkerTab* wt, const cur_her_worker_dyn* dyn,
+                                                    const int64_t* step, HerRow& row, const float** src) {
+  const int64_t c = a.perm ? (int64_t)a.perm[j] : j;
+  const int w = (int)(c / rpw);
+  const int64_t i = c - (int64_t)w * rpw;
+  const HerWorkerTab& t = wt[w];
+  const cur_her_worker_dyn& d = dyn[w];
+  int s = 0;
+  int64_t acc = 0;
+  while (s + 1 < t.n_segments) {
+    const int cnt = d.count[s];
+    if (i < acc + cnt) break;
+    acc += cnt;
+    ++s;
   }
-  row.her = u_her < a.future_p;                                                   // her.py:115
-  row.ft = row.her ? row.t + 1 + (int)(u_off * (double)(L.T - row.t)) : -1;       // her.py:116-118
-  const int64_t tr = (int64_t)row.ep * L.T + row.t;
-  src[0] = base + tr * (int64_t)L.trans_stride;
-  // ag(future_t) is the ag(t+1) block of transition future_t - 1 (future_t >= 1)
-  src[1] = row.her ? base + ((int64_t)row.ep * L.T + (row.ft - 1)) * (int64_t)L.trans_stride + pl.iAG2 : nullptr;
-  src[2] = (pl.cold4 > 0) ? a.seg[s].cold + tr * (int64_t)L.cold_stride : nullptr;
+  row.ttr = t.ttr[s];
+  row.choice = -1;
+  const uint64_t call_offset = a.call_offset + (step ? (uint64_t)*step : 0ull);
+  her_draw_at(a, pl, c, i, call_offset, t.seed, t.base[s], d.n_episodes[s], row, src, [&](int k) { return d.cdf[k]; },
+              [&]() { return t.cold[s]; });
 }
 
 // Squared distance of module m (float64, NumPy's operation order: difference, square, running sum - no FMA

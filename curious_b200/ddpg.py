@@ -14,7 +14,8 @@ the exploration noise of get_actions - they consume the caller's np.random strea
 Extra keyword arguments (all optional): device, comm (torch.distributed group; default WORLD when
 initialised), her_rng ('philox' default | 'numpy' = replay the reference's np.random draws),
 action_noise ('host' default | 'device': exploration noise of get_actions from counter-based draws on the device),
-seed (Xavier init seed; the reference uses TF's graph seed).
+seed (Xavier init seed; the reference uses TF's graph seed), workers_per_rank / workers_mode / worker_buffers
+('shared' default | 'own': every hosted worker with its own buffers and random streams, DESIGN.md section 7).
 """
 import ctypes as C
 import pickle
@@ -24,7 +25,7 @@ import numpy as np
 import torch
 
 from . import _lib, apportion
-from .her import HostDraws
+from .her import DeviceEpisodes, HostDraws
 from .mpi_adam import MpiAdam, adam_step_scale
 from .normalizer import Normalizer, recompute_stats_packed
 from .parallel import allreduce_sum_, world as _world
@@ -104,6 +105,12 @@ class DDPG(object):
         # takes workers x batch_size rows
         self.workers_mode = kwargs.get('workers_mode', 'auto')
         assert self.workers_mode in ('auto', 'wide', 'micro')
+        # 'shared' = the k workers of a rank sample their batches from the rank's one buffer set; 'own' = every worker j has
+        # its own buffers, np.random stream and Philox key (reference rank r * k + j, train.py:221-243; workers.py), its
+        # own episodes in store_episode and its own share of the normaliser batch - one rank only, learner only
+        self.worker_buffers = kwargs.get('worker_buffers', 'shared')
+        if self.worker_buffers not in ('shared', 'own'):
+            raise ValueError("worker_buffers must be 'shared' or 'own', not %r" % (self.worker_buffers,))
         # exploration noise of get_actions (ddpg.py:147-152): 'host' = the caller's np.random stream in reference order,
         # 'device' = counter-based draws applied on the device before the one D2H copy (SURVEY 8f row 1)
         # train() on the CUDA-graph path returns views of fixed device buffers (no copy per update); True = owned copies
@@ -149,6 +156,8 @@ class DDPG(object):
                 for i in range(6, len(self.buffer)):        # distractor buffers are one buffer (ddpg.py:104-110)
                     self.buffer[i] = self.buffer[5]
         self._create_network(reuse=reuse)
+        if self.worker_buffers == 'own':
+            self._init_own_workers()
         self.first = True
         self.cp = None
         self._staged = None
@@ -212,6 +221,40 @@ class DDPG(object):
         self._graph_sig = None
         self._graph_fused = False
         self._wT_dirty = True
+
+    def _init_own_workers(self):
+        """worker_buffers='own': worker 0 keeps the buffers the caller passed, workers 1.. get buffers of the same shapes
+        and sizes (buffers 6.. aliasing 5 like the caller's, ddpg.py:104-110)."""
+        if _world(self.comm)[1] > 1:
+            raise ValueError("worker_buffers='own' runs on one rank")
+        if self.structure == 'task_experts':
+            raise ValueError("worker_buffers='own' does not take structure='task_experts'")
+        if self.workers_mode == 'micro':
+            raise ValueError("worker_buffers='own' runs the workers as one wide batch, not workers_mode='micro'")
+        if getattr(self, 'buffer', None) is None:
+            raise ValueError("worker_buffers='own' needs the buffers")
+        from .replay_buffer import ReplayBuffer
+        from .workers import WorkerStreams
+        k = self.workers_per_rank
+        new = lambda b: ReplayBuffer(b.buffer_shapes, b.size * b.T, b.T, b.sample_transitions, device=b.device)
+        self._worker_buffers = [self.buffer]
+        for _ in range(1, k):
+            if isinstance(self.buffer, list):
+                bufs = []
+                for i, b in enumerate(self.buffer):
+                    bufs.append(bufs[5] if i > 5 else new(b))
+            else:
+                bufs = new(self.buffer)
+            self._worker_buffers.append(bufs)
+        self.worker_streams = WorkerStreams(self.seed, k)
+        self._hyper.loss_rows = self.batch_size        # each worker's loss is a mean over its own batch
+
+    def worker_buffer_set(self, j):
+        """Worker j's buffers (worker_buffers='own'): a list like `buffers`, or one ReplayBuffer."""
+        return self._worker_buffers[j]
+
+    def _own(self):
+        return self.worker_buffers == 'own'
 
     def _mark_weights_changed(self):
         """theta_main was written outside the fused update: W^T kept by the rows graph must be rebuilt (_refresh_wT)."""
@@ -540,7 +583,11 @@ class DDPG(object):
         return 'buffer' in self.task_replay or self.task_replay == 'hand_designed'
 
     def store_episode(self, episode_batch, cp, n_ep, update_stats=True):
-        """episode_batch: {key: [rollout_batch_size, T or T+1, dim]} (ddpg.py:163-223)."""
+        """episode_batch: {key: [rollout_batch_size, T or T+1, dim]} (ddpg.py:163-223).  worker_buffers='own': the k
+        workers' episodes stacked worker-major, [k * rollout_batch_size, ...]; episode b belongs to worker
+        b // rollout_batch_size."""
+        if self._own():
+            return self._store_episode_own(episode_batch, cp, n_ep, update_stats)
         batch_size = episode_batch['ag'].shape[0]
         self.cp = cp
         self.n_episodes = n_ep
@@ -549,19 +596,7 @@ class DDPG(object):
         staged = StagedEpisodes({k: episode_batch[k] for k in keys}, some_buffer.layout, some_buffer.info_keys,
                                 some_buffer.has_td, some_buffer.has_change, self.device)
         copies = []
-        if self.modular:
-            change = np.asarray(episode_batch['change'])
-            for b in range(batch_size):
-                active_tasks = apportion.active_modules(change[b, -1], self.tasks_ag_id, self.tasks_g_id)
-                # (the reference all-reduces an unused counter here, ddpg.py:185 - dropped)
-                if self._multi_buffer():
-                    for task in active_tasks:                        # buffer[0] is never written (ddpg.py:191-195)
-                        copies.append(self.buffer[task + 1].store_staged(staged, b))
-                else:
-                    copies.append(self.buffer.store_staged(staged, b))
-        else:
-            for b in range(batch_size):
-                copies.append(self.buffer.store_staged(staged, b))
+        self._route_episodes(episode_batch, staged, range(batch_size), self.buffer, copies)
         staged.store(copies)
         self._staged = staged
 
@@ -584,6 +619,71 @@ class DDPG(object):
             self.g_stats.update(res['g'])
             recompute_stats_packed((self.o_stats, self.g_stats), self._stats_partial, self.comm)
 
+    def _route_episodes(self, episode_batch, staged, episodes, buffer, copies):
+        """Slot choice of every episode in `episodes` into `buffer` (a list of module buffers, or one), appended to
+        `copies` as store_staged descriptors."""
+        if self.modular:
+            change = np.asarray(episode_batch['change'])
+            for b in episodes:
+                active_tasks = apportion.active_modules(change[b, -1], self.tasks_ag_id, self.tasks_g_id)
+                # (the reference all-reduces an unused counter here, ddpg.py:185 - dropped)
+                if self._multi_buffer():
+                    for task in active_tasks:                        # buffer[0] is never written (ddpg.py:191-195)
+                        copies.append(buffer[task + 1].store_staged(staged, b))
+                else:
+                    copies.append(buffer.store_staged(staged, b))
+        else:
+            for b in episodes:
+                copies.append(buffer.store_staged(staged, b))
+
+    def _store_episode_own(self, episode_batch, cp, n_ep, update_stats):
+        """store_episode of k workers with their own buffers: each worker routes its episodes into its buffers, slot draws
+        from its own stream; one upload, the copies in as few cur_store_episodes launches as CUR_MAX_COPIES allows.  The
+        normaliser batch: every worker HER-samples rollout_batch_size * T fresh transitions of its own episodes with its
+        own draws, all into the one packed partial, which recompute divides by k (the reference's mean over ranks,
+        normalizer.py:84-94)."""
+        k = self.workers_per_rank
+        n_total = episode_batch['ag'].shape[0]
+        if n_total % k:
+            raise ValueError('store_episode with %d workers needs k * rollout_batch_size episodes, got %d' % (k, n_total))
+        rb = n_total // k
+        self.cp = cp
+        self.n_episodes = n_ep
+        some_buffer = self.buffer[1] if type(self.buffer) is list else self.buffer
+        keys = list(some_buffer.buffer_shapes.keys())
+        staged = StagedEpisodes({key: episode_batch[key] for key in keys}, some_buffer.layout, some_buffer.info_keys,
+                                some_buffer.has_td, some_buffer.has_change, self.device)
+        copies = []
+        for j in range(k):
+            with self.worker_streams.use(j):
+                self._route_episodes(episode_batch, staged, range(j * rb, (j + 1) * rb), self._worker_buffers[j], copies)
+        staged.store(copies)
+        self._staged = staged
+        if not update_stats:
+            return
+        episode_batch['o_2'] = episode_batch['o'][:, 1:, :]
+        episode_batch['ag_2'] = episode_batch['ag'][:, 1:, :]
+        per = transitions_in_episode_batch(episode_batch) // k
+        epi = episodes_to_device({key: episode_batch[key] for key in keys}, self.device, staged=staged)
+        sampler = self.sample_transitions
+        L = epi.layout
+        hot, cold = L.T * L.trans_stride * rb, L.T * L.cold_stride * rb
+        workers, draws = [], None if self.her_rng != 'numpy' else []
+        for j in range(k):
+            part = DeviceEpisodes(epi.storage[j * hot:(j + 1) * hot], epi.cold[j * cold:(j + 1) * cold], rb, L,
+                                  epi.info_keys, epi.has_td, epi.has_change)
+            workers.append((self.worker_streams.philox_key(j), [(part, per, None)]))
+            if draws is not None:
+                with self.worker_streams.use(j):
+                    d = HostDraws(rb, L.T, per)
+                    d.draw_choices(sampler.mode, sampler.future_p, getattr(self, 'nb_tasks', 0), None)
+                draws.append(d)
+        res = sampler.sample_workers(workers, per, draws=draws, clip_obs=self.clip_obs,
+                                     relative_goals=self.relative_goals, want=('o', 'g'))
+        self.o_stats.update(res['o'])
+        self.g_stats.update(res['g'])
+        recompute_stats_packed((self.o_stats, self.g_stats), self._stats_partial, self.comm, workers=k)
+
     def get_current_buffer_size(self):
         return sum([self.buffer[i].get_current_size() for i in range(self.nb_tasks)])
 
@@ -593,9 +693,11 @@ class DDPG(object):
         self._wT_dirty = True
 
     # ------------------------------------------------------------------------------------------
-    def _proportions(self):
-        """LP-weighted apportioning of the batch over the module buffers (ddpg.py:255-286, 302-318)."""
-        sizes = [self.buffer[i].current_size for i in range(self.nb_tasks + 1)]
+    def _proportions(self, buffers=None):
+        """LP-weighted apportioning of the batch over the module buffers (ddpg.py:255-286, 302-318); `buffers`: a
+        worker's buffer set (worker_buffers='own': shared cp, that worker's fill levels)."""
+        buffers = self.buffer if buffers is None else buffers
+        sizes = [buffers[i].current_size for i in range(self.nb_tasks + 1)]
         if self.structure == 'curious':
             prop = apportion.proportions_curious(sizes, self.T, self.batch_size, self.task_replay, self.cp,
                                                  self.eps_task)
@@ -604,9 +706,11 @@ class DDPG(object):
         self.proportions = prop
         return prop
 
-    def _sample_device(self, want, rng=None):
-        """Run the fused HER kernel for one batch; returns {key: float32 cuda tensor}."""
+    def _sample_device(self, want, rng=None, want_idx=False):
+        """Run the fused HER kernel for one batch; returns {key: float32 cuda tensor} (+ 'idx' with want_idx)."""
         rng = rng or self.her_rng
+        if self._own():
+            return self._sample_workers(want, rng, want_idx=want_idx)
         sampler = self.sample_transitions
         B = self.batch_size
         cp_proba = None
@@ -643,7 +747,55 @@ class DDPG(object):
                 np.random.shuffle(perm)                                   # ddpg.py:338-339
                 self._last_perm = perm
         return sampler.sample_device(segs, B, cp_proba=cp_proba, draws=draws, perm=perm, clip_obs=self.clip_obs,
-                                     relative_goals=self.relative_goals, want=want)
+                                     relative_goals=self.relative_goals, want=want, want_idx=want_idx)
+
+    def _worker_segments(self, j):
+        """Worker j's (buffer, count, task_to_replay) table over ALL its buffers in buffer order (count 0 where nothing is
+        sampled), the apportioning of `_sample_device`, whether the batch is shuffled, and cp_proba as `_sample_device`
+        passes it to the sampler."""
+        bufs = self._worker_buffers[j]
+        cp_proba = None
+        if self.modular and self._multi_buffer() and (
+                self.structure == 'curious' or self.task_replay == 'replay_current_task_buffer'):
+            prop = self._proportions(bufs)
+            segs = []
+            for i in range(self.nb_tasks + 1):
+                ttr = (i - 1 if i > 0 else None) if self.structure == 'curious' else self.t_id
+                segs.append((bufs[i], int(prop[i]), ttr))
+            return segs, True, cp_proba
+        if self.modular and self.structure == 'curious' and self.task_replay == 'replay_cp_task_transition':
+            cp_proba = apportion.cp_probabilities(self.cp, self.eps_task)       # ddpg.py:288-296
+        return [(bufs, self.batch_size, None)], False, cp_proba
+
+    def _sample_workers(self, want, rng=None, want_idx=False, out=None, dyn=None, step=None, call_offset=None):
+        """worker_buffers='own': the batches of the k workers, each from its own buffers with its own draws, as one
+        cur_her_sample_workers launch; rows [j * batch_size, (j + 1) * batch_size) are worker j's batch."""
+        rng = rng or self.her_rng
+        sampler = self.sample_transitions
+        B = self.batch_size
+        workers, draws, perms, cp_proba = [], [], [], None
+        for j in range(self.workers_per_rank):
+            segs, shuffle, cp_proba = self._worker_segments(j)
+            for buf, count, _ in segs:
+                assert count == 0 or buf.current_size > 0
+            workers.append((self.worker_streams.philox_key(j), [(b.device_view(), c, t) for b, c, t in segs]))
+            if rng == 'numpy':
+                with self.worker_streams.use(j):
+                    for b, count, _ in segs:          # one sampler call per non-empty buffer, in buffer order
+                        if count > 0:
+                            d = HostDraws(b.current_size, b.T, count)
+                            d.draw_choices(sampler.mode, sampler.future_p, getattr(self, 'nb_tasks', 0), cp_proba)
+                            draws.append(d)
+                    if shuffle:
+                        perm = np.arange(B)
+                        np.random.shuffle(perm)                           # ddpg.py:338-339
+                        perms.append(perm + j * B)
+        perm = np.concatenate(perms) if perms else None
+        if perm is not None:
+            self._last_perm = perm[:B]
+        return sampler.sample_workers(workers, B, dyn=dyn, step=step, cdf=cp_proba, draws=draws if rng == 'numpy' else None,
+                                      perm=perm, clip_obs=self.clip_obs, relative_goals=self.relative_goals, want=want,
+                                      want_idx=want_idx, out=out, call_offset=call_offset)
 
     _STAGE_TO_KERNEL = {'ag': 'ag', 'g': 'g', 'o': 'o', 'task_descr': 'td', 'u': 'u', 'o_2': 'o_2', 'g_2': 'g_2',
                         'r': 'r'}
@@ -653,7 +805,8 @@ class DDPG(object):
         want = tuple(self._STAGE_TO_KERNEL[k] for k in self.stage_shapes.keys())
         res = self._sample_device(want)
         torch.cuda.current_stream().synchronize()
-        return [res[self._STAGE_TO_KERNEL[k]].cpu().numpy().astype(np.float64) for k in self.stage_shapes.keys()]
+        B = self.batch_size                # worker_buffers='own': worker 0's batch
+        return [res[self._STAGE_TO_KERNEL[k]][:B].cpu().numpy().astype(np.float64) for k in self.stage_shapes.keys()]
 
     def stage_batch(self, batch=None):
         """ddpg.py:362-366.  With batch=None the batch is sampled on the device and never leaves it."""
@@ -734,14 +887,21 @@ class DDPG(object):
         return [(self.buffer, None)]
 
     def _dyn_signature(self):
-        segs = self._all_segments()
         cp = None if self.cp is None else tuple(np.asarray(self.cp, np.float64).tolist())
+        if self._own():
+            sets = [b if isinstance(b, list) else [b] for b in self._worker_buffers]
+            return tuple(b.current_size for bufs in sets for b in bufs), cp
+        segs = self._all_segments()
         return tuple(b.current_size for b, _ in segs), cp
 
     def _refresh_dyn(self):
         """Recompute the LP apportioning (ddpg.py:255-318) and push it to the device control block."""
         sig = self._dyn_signature()
         if sig == self._graph_sig:
+            return
+        if self._own():
+            self._refresh_worker_dyn()
+            self._graph_sig = sig
             return
         segs = self._all_segments()
         d = self._dyn_struct
@@ -762,6 +922,22 @@ class DDPG(object):
         self._dyn_dev.copy_(self._dyn_host, non_blocking=True)
         self._graph_sig = sig
 
+    def _refresh_worker_dyn(self):
+        """worker_buffers='own': every worker's apportioning (shared cp, its own fill levels) and cdf into the device
+        control blocks of the captured worker sampler."""
+        d = self._wdyn_struct
+        for j in range(self.workers_per_rank):
+            segs, _, cp_proba = self._worker_segments(j)
+            for i, (buf, count, _) in enumerate(segs):
+                d[j].n_episodes[i] = int(buf.current_size)
+                d[j].count[i] = int(count)
+            if cp_proba is not None:
+                _lib.set_cdf(d[j], cp_proba)
+            elif self.sample_transitions.mode == _lib.MODE_CP_TASK:
+                _lib.set_cdf(d[j], np.ones(self.nb_tasks) / self.nb_tasks)
+        C.memmove(self._wdyn_host.data_ptr(), C.addressof(d), C.sizeof(d))
+        self._wdyn_dev.copy_(self._wdyn_host, non_blocking=True)
+
     def _prepare_graph_state(self):
         """Device-resident state of the graph path (control block, loss rings, Adam tables, fixed batch buffers)."""
         dev = self.device
@@ -775,6 +951,9 @@ class DDPG(object):
         self._wide = bool(k > 1 and self.workers_mode != 'micro' and (
             (self.update_schedule != 'levels' and self._rows_shape_ok(wide_rows)) or
             lib.cur_ddpg_uses_tensor_cores(C.byref(self.net.desc), wide_rows) or self._use_native_chain(wide_rows)))
+        if self._own() and k > 1 and not self._wide:
+            raise ValueError("worker_buffers='own' needs a schedule that takes workers x batch_size rows in one update "
+                             "(rows up to 1024, the chain kernel or the tensor-core levels schedule above)")
         self._graph_rows = self.batch_size * (k if self._wide else 1)
         self._micro = 1 if self._wide else k
         B = self._graph_rows
@@ -784,6 +963,10 @@ class DDPG(object):
         nbytes = C.sizeof(_lib.HerDyn)
         self._dyn_host = torch.zeros(nbytes, dtype=torch.uint8, pin_memory=True)
         self._dyn_dev = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
+        if self._own():
+            self._wdyn_struct = (_lib.HerWorkerDyn * k)()
+            self._wdyn_host = torch.zeros(C.sizeof(self._wdyn_struct), dtype=torch.uint8, pin_memory=True)
+            self._wdyn_dev = torch.zeros(C.sizeof(self._wdyn_struct), dtype=torch.uint8, device=dev)
         self._q_ring = torch.zeros(self.LOSS_RING, dtype=torch.float32, device=dev)
         self._pi_ring = torch.zeros(self.LOSS_RING, dtype=torch.float32, device=dev)
         self._q_pi = torch.zeros((B, 1), dtype=torch.float32, device=dev)
@@ -799,7 +982,7 @@ class DDPG(object):
         self._ghyper = _lib.DdpgHyper(self._hyper.gamma, self._hyper.clip_return, self._hyper.action_l2,
                                       self._hyper.clip_pos_returns, self._step.data_ptr(), self.LOSS_RING,
                                       self._micro if self._micro > 1 else 0)
-        if self._wide:
+        if self._wide or self._own():
             self._ghyper.loss_rows = self.batch_size
         if self._micro > 1 and not self._use_rows(B):
             raise ValueError('workers_per_rank > 1 on the CUDA-graph path needs the rows schedule or a batch the '
@@ -904,7 +1087,11 @@ class DDPG(object):
         sampler = self.sample_transitions
         segs = [(buf.device_view(), 0, ttr) for buf, ttr in self._all_segments()]
         her_args = None
-        if self._use_rows(self._graph_rows) and self.fuse_her:
+        if self._own():
+            # the workers' batches: one standalone sampler launch (not fused into the rows prologue)
+            self._sample_workers(self._gwant, rng='philox', out=self._gbatch, dyn=self._wdyn_dev.data_ptr(),
+                                 step=self._step.data_ptr(), call_offset=self.GRAPH_STREAM_OFFSET)
+        elif self._use_rows(self._graph_rows) and self.fuse_her:
             # rows schedule: every CTA of the update kernel samples its own rows (no separate HER launch)
             her_args, self._her_keep = sampler.sample_device(
                 segs, self._graph_rows, clip_obs=self.clip_obs, relative_goals=self.relative_goals, want=(),
@@ -1043,7 +1230,7 @@ class DDPG(object):
         if stage:
             self.stage_batch()
         critic_loss, actor_loss, Q_grad, pi_grad = self._grads()
-        if self.workers_per_rank > 1:
+        if self.workers_per_rank > 1 and not self._own():
             # several reference workers on this rank: sum of their single-batch gradients (ddpg.py:452-453)
             assert stage, 'workers_per_rank > 1 samples its own batches'
             total = self.grads.clone()
@@ -1053,7 +1240,8 @@ class DDPG(object):
                 total += self.grads
             self.grads.copy_(total)
         self._update(Q_grad, pi_grad)
-        self._step += self.workers_per_rank   # the device counter counts sampled batches (Philox stream position)
+        # the device counter counts sampled batches (Philox stream position); the workers of 'own' are one wide batch
+        self._step += 1 if self._own() else self.workers_per_rank
         self._n_updates += 1
         return LazyHost(critic_loss.clone().reshape(())), LazyHost(actor_loss)
 
@@ -1068,8 +1256,9 @@ class DDPG(object):
                                           self.theta_main.numel(), float(self.polyak)), 'cur_polyak')
 
     def clear_buffer(self):
-        for i in range(self.nb_tasks):
-            self.buffer[i].clear_buffer()
+        for bufs in (self._worker_buffers if self._own() else [self.buffer]):
+            for i in range(self.nb_tasks):
+                bufs[i].clear_buffer()
 
     # ------------------------------------------------------------------------------------------
     def logs(self, prefix=''):
@@ -1137,6 +1326,8 @@ class DDPG(object):
         accumulators, the Philox stream positions and (optionally) the replay buffers and the host np.random state.
         The reference can only save weights + normaliser statistics (ddpg.py:481-497, SURVEY 8f row 3): its Adam
         state, replay data and RNG position are lost on restart.  One torch.save file, tensors on the host."""
+        if self._own():
+            raise ValueError("save_checkpoint does not cover worker_buffers='own' (per-worker buffers and streams)")
         self._gather_adam_state()
         cpu = lambda t: t.detach().cpu().clone()
         st = dict(format=1, arena=int(self.net.arena), net=self._net_signature(), theta_main=cpu(self.theta_main), theta_target=cpu(self.theta_target),
@@ -1166,6 +1357,8 @@ class DDPG(object):
 
     def load_checkpoint(self, path):
         """Inverse of save_checkpoint on an agent built with the same arguments (checked: arena size, buffer layouts)."""
+        if self._own():
+            raise ValueError("load_checkpoint does not cover worker_buffers='own' (per-worker buffers and streams)")
         st = torch.load(path, map_location='cpu', weights_only=False)
         if st.get('format') != 1 or st['arena'] != int(self.net.arena) or st.get('net', self._net_signature()) != \
                 self._net_signature():

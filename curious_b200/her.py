@@ -134,20 +134,7 @@ class HerSampler:
             mode_of(self.task_replay, self.flat)
         lib = _lib.load()
         first = segments[0][0]
-        L = first.layout
-        dev = first.storage.device
-        if self.reward.needs_info() and self._info_layout != first.info_keys:
-            self._info_layout = first.info_keys
-            self.task_table = self.reward.task_table(first.info_keys)
         a = _lib.HerArgs()
-        a.L = L
-        a.tasks = self.task_table
-        if cp_proba is not None:
-            _lib.set_cdf(a.tasks, cp_proba)
-        elif self.mode == _lib.MODE_CP_TASK:
-            # np.random.choice(range(n), p=None) is uniform (the store_episode stats path, ddpg.py:213)
-            _lib.set_cdf(a.tasks, np.ones(max(self.nb_tasks, 1)) / max(self.nb_tasks, 1))
-        a.mode = self.mode
         a.n_segments = len(segments)
         if len(segments) > _lib.CUR_MAX_SEGMENTS:
             raise ValueError('too many buffers in one sample call')
@@ -163,6 +150,32 @@ class HerSampler:
             total += int(count)
         assert dyn is not None or total == B                                 # ddpg.py:323
         a.dyn = dyn
+        a.seed = int(self.seed) & 0xFFFFFFFFFFFFFFFF
+        res, keep = self._fill_args(a, first, B, cp_proba, draws, perm, call_offset, clip_obs, relative_goals, want,
+                                    want_idx, out)
+        if args_only:
+            # the caller launches a kernel that samples for itself (cur_ddpg_rows_step with `her`)
+            res['_keep'] = keep
+            return a, res
+        _lib.check(lib.cur_her_sample(_lib.stream_ptr(stream), C.byref(a)), 'cur_her_sample')
+        res['_keep'] = keep
+        return res
+
+    def _fill_args(self, a, first, B, cp_proba, draws, perm, call_offset, clip_obs, relative_goals, want, want_idx, out):
+        """The cur_her_args fields both sampling entries share: layout, reward table, draws, shuffle, outputs."""
+        L = first.layout
+        dev = first.storage.device
+        if self.reward.needs_info() and self._info_layout != first.info_keys:
+            self._info_layout = first.info_keys
+            self.task_table = self.reward.task_table(first.info_keys)
+        a.L = L
+        a.tasks = self.task_table
+        if cp_proba is not None:
+            _lib.set_cdf(a.tasks, cp_proba)
+        elif self.mode == _lib.MODE_CP_TASK:
+            # np.random.choice(range(n), p=None) is uniform (the store_episode stats path, ddpg.py:213)
+            _lib.set_cdf(a.tasks, np.ones(max(self.nb_tasks, 1)) / max(self.nb_tasks, 1))
+        a.mode = self.mode
         a.batch = B
         a.future_p = float(self.future_p)
         keep = []
@@ -173,7 +186,6 @@ class HerSampler:
             a.inj_u_her, a.inj_u_off = d['u_her'].data_ptr(), d['u_off'].data_ptr()
             a.inj_choice = d['choice'].data_ptr() if d.get('choice') is not None else None
         else:
-            a.seed = int(self.seed) & 0xFFFFFFFFFFFFFFFF
             a.call_offset = self.calls if call_offset is None else call_offset
         if call_offset is None:
             self.calls += 1
@@ -196,11 +208,51 @@ class HerSampler:
         if want_idx:
             res['idx'] = torch.empty((B, 4), dtype=torch.int32, device=dev)
             a.idx_out = res['idx'].data_ptr()
-        if args_only:
-            # the caller launches a kernel that samples for itself (cur_ddpg_rows_step with `her`)
-            res['_keep'] = keep
-            return a, res
-        _lib.check(lib.cur_her_sample(_lib.stream_ptr(stream), C.byref(a)), 'cur_her_sample')
+        return res, keep
+
+    def sample_workers(self, workers, rows_per_worker, *, dyn=None, step=None, cdf=None, draws=None, perm=None,
+                       clip_obs=0.0, relative_goals=False, want=('o', 'ag', 'g', 'u', 'td', 'change', 'info', 'o_2',
+                                                                  'ag_2', 'r'),
+                       want_idx=False, out=None, stream=None, call_offset=None):
+        """Worker-major form (cur_her_sample_workers): `workers` = [(philox_key, [(DeviceEpisodes, count, ttr), ...])],
+        one entry per worker; worker j's rows are [j * rows_per_worker, (j + 1) * rows_per_worker) of every output.
+        dyn: device address of len(workers) cur_her_worker_dyn (CUDA graph: the caller rewrites it between replays);
+        None = built from the segments' counts / sizes and `cdf` and uploaded for this call.  step: device int64 counter
+        added to the Philox call offset, or None.  draws: the workers' HostDraws, worker after worker; perm: the
+        permutation of all concat rows (worker j's shuffle inside its own block)."""
+        lib = _lib.load()
+        n = len(workers)
+        B = n * rows_per_worker
+        first = workers[0][1][0][0]
+        W = (_lib.HerWorker * max(n, 1))()
+        host_dyn = (_lib.HerWorkerDyn * max(n, 1))()
+        for j, (key, segs) in enumerate(workers):
+            if len(segs) > _lib.CUR_MAX_SEGMENTS:
+                raise ValueError('worker %d has %d buffers; at most %d' % (j, len(segs), _lib.CUR_MAX_SEGMENTS))
+            W[j].seed = int(key) & 0xFFFFFFFFFFFFFFFF
+            W[j].n_segments = len(segs)
+            for i, (epi, count, ttr) in enumerate(segs):
+                s = W[j].seg[i]
+                s.base = epi.storage.data_ptr()
+                s.cold = None if epi.cold is None else epi.cold.data_ptr()
+                s.n_episodes = host_dyn[j].n_episodes[i] = int(epi.n_episodes)
+                s.count = host_dyn[j].count[i] = int(count)
+                s.task_to_replay = -1 if ttr is None else int(ttr)
+            if cdf is not None:
+                _lib.set_cdf(host_dyn[j], cdf)
+        a = _lib.HerArgs()
+        res, keep = self._fill_args(a, first, B, None, draws, perm, call_offset, clip_obs, relative_goals, want,
+                                    want_idx, out)
+        if dyn is None:
+            if cdf is None and self.mode == _lib.MODE_CP_TASK:
+                for j in range(n):
+                    host_dyn[j].cdf = a.tasks.cdf
+            blob = torch.frombuffer(bytearray(host_dyn), dtype=torch.uint8).pin_memory()
+            dev = blob.to(first.storage.device, non_blocking=True)
+            keep.append((blob, dev))
+            dyn = dev.data_ptr()
+        _lib.check(lib.cur_her_sample_workers(_lib.stream_ptr(stream), C.byref(a), n, rows_per_worker, W, dyn, step),
+                   'cur_her_sample_workers')
         res['_keep'] = keep
         return res
 

@@ -121,13 +121,14 @@ class Normalizer:
         self.std.copy_(torch.from_numpy(sd).to(self.device))
 
 
-def recompute_stats_packed(normalizers, packed, comm=None):
+def recompute_stats_packed(normalizers, packed, comm=None, workers=1):
     """`recompute_stats` of several normalisers whose partials are slices of `packed`: ONE all-reduce for all of them
     per store_episode (the reference issues three blocking all-reduces per normaliser, normalizer.py:84-94, six per
-    store; SURVEY 8e asks for one packed collective), then each one's `+=` / mean / std kernel."""
+    store; SURVEY 8e asks for one packed collective), then each one's `+=` / mean / std kernel.  `workers`: reference
+    workers per rank whose batches all went into the partials - the mean is over workers x ranks."""
     world = allreduce_sum_(packed, comm)
     for nz in normalizers:
-        nz.recompute_stats(world=world)
+        nz.recompute_stats(world=world * workers)
     return world
 
 

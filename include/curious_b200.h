@@ -187,6 +187,36 @@ typedef struct cur_her_args {
 
 int cur_her_sample(void* stream, const cur_her_args* args);
 
+/* Worker-major form of cur_her_sample: one launch samples the batches of n_workers reference workers, each from its own
+ * buffers with its own random stream (the reference's MPI workers, train.py:221-243, hosted on one rank).  Concat row c
+ * belongs to worker j = c / rows_per_worker, at local row i = c % rows_per_worker; the segment lookup runs over worker
+ * j's own segments (w[j].seg: base, cold, task_to_replay; the counts and sizes the kernel reads are dyn[j]'s).
+ *   Philox draws: key w[j].seed, counter (i, a->call_offset + (step ? *step : 0)) - the position a lone agent keyed
+ *   w[j].seed draws its row i from at the same update.
+ *   Injected draws (a->inj_*) and a->perm stay indexed by the concat row: the caller lays worker j's draws and its
+ *   shuffle out in rows [j * rows_per_worker, (j + 1) * rows_per_worker).
+ * Everything else (relabelling, reward table, clip, outputs, idx_out) is cur_her_sample's with a->batch ==
+ * n_workers * rows_per_worker; a->seg, a->n_segments, a->seed and a->dyn are ignored.  `dyn` (DEVICE, n_workers entries)
+ * and `step` (DEVICE or NULL) are read at run time, so a CUDA graph replays with frozen arguments.  w is a HOST array
+ * whose seg[].count / seg[].n_episodes are checked here; refused before any launch: n_workers outside
+ * 1..CUR_MAX_WORKERS, a worker with n_segments outside 1..CUR_MAX_SEGMENTS, counts of a worker that do not sum to
+ * rows_per_worker, a->batch != n_workers * rows_per_worker. */
+#define CUR_MAX_WORKERS 64
+typedef struct cur_her_worker {
+  uint64_t seed;                       /* Philox key of this worker's draws                         */
+  int32_t n_segments;
+  int32_t _pad;
+  cur_segment seg[CUR_MAX_SEGMENTS];   /* the worker's buffers, in buffer order                      */
+} cur_her_worker;
+typedef struct cur_her_worker_dyn {
+  int32_t n_episodes[CUR_MAX_SEGMENTS];
+  int32_t count[CUR_MAX_SEGMENTS];     /* sums to rows_per_worker                                   */
+  double cdf[CUR_MAX_TASKS];           /* CP_TASK mode: normalised cumsum(cp_proba)                  */
+} cur_her_worker_dyn;
+int cur_her_sample_workers(void* stream, const cur_her_args* a, int n_workers, int rows_per_worker,
+                           const cur_her_worker* w, const cur_her_worker_dyn* dyn /* device */,
+                           const int64_t* step /* device or NULL */);
+
 /* The kernels' counter-based generator on its own: out[i] = Philox4x32-10(counter = in[i][0..3], key = in[i][4..5])
  * evaluated ON THE DEVICE by the same device function the sampling and exploration-noise kernels call (known-answer
  * tests against the Random123 vectors; the reference draws from np.random, her.py:108-116, which this mode replaces). */
