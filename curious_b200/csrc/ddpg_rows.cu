@@ -24,8 +24,7 @@
 //             layers.  History (profiles/README.md): column split over an 8-CTA cluster with a per-layer
 //             exchange (lost to the synchronisation), one CTA for everything, main / target CTA pair with
 //             main.Q streamed once for 8 stacked rows (FFMA-bound passes, idle target CTA), this split; round 2:
-//             ddpg_stream_pair_kernel, the columns of every layer split over a 2-CTA cluster (half the weight
-//             bytes per SM, st.async exchange through distributed shared memory) - correct, slower, opt-in.
+//             the columns of every layer split over a 2-CTA cluster - correct, slower, removed.
 //   launch 2  rows_dw_kernel     every dW = X^T dY and db = 1^T dY of both nets as one grouped GEMM with
 //             the full batch as K (deterministic, no atomics), written into the flat GetFlat-ordered
 //             gradient arena; optionally Adam is applied to the element in the same epilogue (world
@@ -39,7 +38,6 @@
 #include "her_device.cuh"
 #include "net_layout.cuh"
 #include "tc_gemm.cuh"
-#include "tc_ptx.cuh"
 
 namespace cur {
 
@@ -114,9 +112,7 @@ struct StreamParams {
   float* loss_part;          // [n / 4][4]
   float* q_pi;               // [n]
   long long* tl;             // optional debug timeline (clock64 stamps of CTA 0), CUR_ROWS_TIMELINE=1
-  int dbg_skip_math;         // debug: consumers only wait/release (measures the pure streaming rate)
   const int64_t* tl_step;    // debug: device step counter (update number of the timeline marks) or NULL
-  int pdl_late;              // programmatic dependent launch: trigger the next kernel when this CTA is done (not at its start)
   int fused_her;             // sample the CTA's 4 rows here (her, plan) instead of reading a staged batch
   HerPlan plan;
   cur_her_args her;
@@ -157,37 +153,6 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                "l"(src), "r"(bytes), "r"(bar)
                : "memory");
 }
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\nbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t local_addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local_addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void st_remote_f32(uint32_t remote_addr, float v) {
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(remote_addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t remote_bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote_bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAITC_LOOP:\n"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra WAITC_DONE;\n"
-      "bra WAITC_LOOP;\n"
-      "WAITC_DONE:\n"
-      "}\n" ::"r"(bar), "r"(parity)
-      : "memory");
-}
 __device__ __forceinline__ unsigned long long globaltimer_ns() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -197,11 +162,6 @@ __device__ __forceinline__ void st_ll(unsigned long long* p, float v, uint32_t f
   const unsigned long long w = ((unsigned long long)flag << 32) | (unsigned long long)__float_as_uint(v);
   asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(w) : "memory");
 }
-// Programmatic dependent launch: the next kernel of the stream may be scheduled while this one still runs (its CTAs
-// take SMs as they free up and park in pdl_wait); pdl_wait returns once the previous kernel has completed and its
-// writes are visible.  Both are no-ops for a launch without the attribute.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void consumer_sync() { asm volatile("bar.sync 1, %0;" ::"n"(S_CONSUMERS) : "memory"); }
 
 
@@ -248,9 +208,8 @@ __device__ __forceinline__ void fma_row(float2 (&acc)[NR / 2][4], const float* _
 }
 
 // acc += sum over this thread's k rows of the next `nchunks` weight chunks of  xT[k][r] * W[k][4cg + c]
-template <int H, int NR, class PT>
-__device__ __forceinline__ void gemv_chunks(const PT& P, Ring& rg, int nchunks, const float* __restrict__ xT,
-                                            float2 (&acc)[NR / 2][4]) {
+template <int H, int NR>
+__device__ __forceinline__ void gemv_chunks(Ring& rg, int nchunks, const float* __restrict__ xT, float2 (&acc)[NR / 2][4]) {
   using Wd = Width<H>;
   constexpr int RK = Wd::RK;
   const int cg = threadIdx.x % Wd::CG, ks = threadIdx.x / Wd::CG;
@@ -261,8 +220,7 @@ __device__ __forceinline__ void gemv_chunks(const PT& P, Ring& rg, int nchunks, 
     mbar_wait(rg.full + 8 * slot, (rg.cons / S_NSLOT) & 1);
     const float* ws = rg.slots + slot * S_SLOT + 4 * cg;
     const float* xs = xT + (k0 + ks * RK) * NR;
-    if (P.dbg_skip_math) {
-    } else if (nrows == Wd::CK) {
+    if (nrows == Wd::CK) {
       // full chunk (all but the ragged first-layer blocks): no guards, so the LDS.128 of the thread's RK k rows
       // are issued up front and the FFMA2s run back to back
       float4 w[RK];
@@ -289,16 +247,15 @@ __device__ __forceinline__ bool owns_col(int col) { return H == S_CONSUMERS || c
 
 // One dense layer for NR rows: chunks -> split-K partials -> fixed-order sum.  Returns, for the thread's column
 // `col = tid` (if owns_col), the NR pre-activation sums in v[] (without bias).
-template <int H, int NR, class PT>
-__device__ __forceinline__ void layer_gemv(const PT& P, Ring& rg, int nchunks, const float* xT, float* red,
-                                           float (&v)[NR]) {
+template <int H, int NR>
+__device__ __forceinline__ void layer_gemv(Ring& rg, int nchunks, const float* xT, float* red, float (&v)[NR]) {
   using Wd = Width<H>;
   float2 acc[NR / 2][4];
 #pragma unroll
   for (int p = 0; p < NR / 2; ++p)
 #pragma unroll
     for (int c = 0; c < 4; ++c) acc[p][c] = make_float2(0.f, 0.f);
-  gemv_chunks<H, NR>(P, rg, nchunks, xT, acc);
+  gemv_chunks<H, NR>(rg, nchunks, xT, acc);
   const int cg = threadIdx.x % Wd::CG, ks = threadIdx.x / Wd::CG;
 #pragma unroll
   for (int p = 0; p < NR / 2; ++p) {
@@ -402,7 +359,7 @@ __device__ __noinline__ void build_x(const StreamParams& P, float* xT, int NR, i
 // the same per-row device functions as her_sample_kernel (bit-identical batches).  Both CTAs of a pair sample the
 // same rows (a 4 x ~0.5 KB gather).
 __device__ __forceinline__ void sample_rows(const StreamParams& P, int64_t row0, float* stage, const float** m_src,
-                                            float* s_r, float* scratch /* >= 1 KB, 16-byte aligned */, int nrows = S_ROWS) {
+                                            float* s_r, float* scratch /* >= 1 KB, 16-byte aligned */) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const HerPlan& pl = P.plan;
   HerRow row;
@@ -419,9 +376,9 @@ __device__ __forceinline__ void sample_rows(const StreamParams& P, int64_t row0,
     if (tid == 0) *step_s = __ldcg(reinterpret_cast<const long long*>(dyn_s->step));
     consumer_sync();
   }
-  if (tid < nrows) her_draw_row(P.her, pl, row0 + tid, row, m_src + 3 * tid, dyn_s, step_s);
+  if (tid < S_ROWS) her_draw_row(P.her, pl, row0 + tid, row, m_src + 3 * tid, dyn_s, step_s);
   consumer_sync();
-  if (warp < nrows) {
+  if (warp < S_ROWS) {
     const int per_row = pl.img4 + pl.fut4 + pl.cold4;   // (cold rows only for an `info` reward or relative goals)
     float* dst = stage + warp * pl.stage_stride;
     for (int c = lane; c < per_row; c += 32) {
@@ -435,7 +392,7 @@ __device__ __forceinline__ void sample_rows(const StreamParams& P, int64_t row0,
   cp_commit();
   cp_wait0();
   consumer_sync();
-  if (tid < nrows) {
+  if (tid < S_ROWS) {
     int relab;
     s_r[tid] = her_relabel_row(P.her, pl, stage + tid * pl.stage_stride, row, &relab);
   }
@@ -482,7 +439,7 @@ __device__ __forceinline__ float* forward_net(const PT& P, Ring& rg, int ch0, fl
   for (int l = 0; l < P.L; ++l) {
     float v[NR];
     const float b = on ? bias[l][col] : 0.f;      // in flight during the layer (an exposed L2 round trip otherwise)
-    layer_gemv<H, NR>(P, rg, l == 0 ? ch0 : H / Width<H>::CK, xin, red, v);
+    layer_gemv<H, NR>(rg, l == 0 ? ch0 : H / Width<H>::CK, xin, red, v);
 #pragma unroll
     for (int r = 0; r < NR; ++r) v[r] = fmaxf(v[r] + b, 0.f);
     if (on && h_a != nullptr) {
@@ -541,8 +498,6 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (!P.pdl_late) pdl_launch_dependents();
-  pdl_wait();               // everything below reads what the previous kernel (weight gradients + Adam of the last update) wrote
   __syncthreads();          // barriers initialised before the producer / consumers use them
 
   const SChunk* my_chunks = role == 0 ? P.chunks : P.chunks_t;
@@ -630,7 +585,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
 #pragma unroll
       for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hq[l - 1] + (row0 + r) * H + col) : 0.f;   // ReLU masks of layer l-1
       float v[4];
-      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
+      layer_gemv<H, 4>(rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         v[r] = relu_mask(v[r], m[r]);
@@ -642,7 +597,6 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
     }
     if (P.tl != nullptr && tid == 0 && blockIdx.x < 512) P.tl[65 + 2 * blockIdx.x] = (long long)globaltimer_ns();
     if (P.tl != nullptr && P.tl_step != nullptr && tid == 0) tl_mark_max(P.tl + TL_MARKS + 4 * (int)(*P.tl_step & 7) + 1);
-    pdl_launch_dependents();
     return;
   }
 
@@ -700,7 +654,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
 #pragma unroll
       for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hqp[l - 1] + (row0 + r) * H + col) : 0.f;
       float v[4];
-      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
+      layer_gemv<H, 4>(rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) v[r] = relu_mask(v[r], m[r]);
       put_xT<H, 4>(xout, v);
@@ -750,7 +704,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
 #pragma unroll
       for (int r = 0; r < 4; ++r) m[r] = on ? __ldcg(P.hp[l - 1] + (row0 + r) * H + col) : 0.f;
       float v[4];
-      layer_gemv<H, 4>(P, rg, H / Width<H>::CK, xin, red, v);
+      layer_gemv<H, 4>(rg, H / Width<H>::CK, xin, red, v);
 #pragma unroll
       for (int r = 0; r < 4; ++r) {
         v[r] = relu_mask(v[r], m[r]);
@@ -764,473 +718,6 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
   S_TL(7);
   if (P.tl != nullptr && tid == 0 && blockIdx.x < 512) P.tl[65 + 2 * blockIdx.x] = (long long)globaltimer_ns();
   if (P.tl != nullptr && P.tl_step != nullptr && tid == 0) tl_mark_max(P.tl + TL_MARKS + 4 * (int)(*P.tl_step & 7) + 1);
-  pdl_launch_dependents();
-}
-
-// ------------------------------------------------------------------------------------------------
-// CTA-PAIR form of the stream kernel (batch a multiple of 8): a 2-CTA cluster walks one chain for EIGHT rows, and each CTA
-// owns HALF the output columns of every hidden layer.  An SM then ingests only half of its chain's weights (1.1 MB
-// instead of 2.2 MB - per-SM L2 -> shared bandwidth, ~42 B/clk, is what bounds the 4-row kernel) while doing the same
-// number of FMAs (8 rows x 128 columns; scratch/micro/gemv_micro.cu: 690 cycles per 32 KB chunk against ~780 of ingest).
-// After every layer the two CTAs swap their halves of the activations through distributed shared memory: each thread
-// stores its 16 bytes into both CTAs' transposed activation buffer and arrives on the partner's mbarrier; the next layer
-// starts with the k rows of the CTA's OWN columns (already local) and only then waits for the partner's half, so the
-// exchange latency hides behind half a layer.  Weight chunks are 64 k rows x 128 columns = 32 KB, one 2-D TMA box each
-// (64 bulk copies of 512 bytes per chunk, the first version, ran at ~8 B/clk: 100 us per update).
-constexpr int PR_ROWS = 8;                // batch rows per CTA pair
-constexpr int PR_NC = 128;                // output columns per CTA
-constexpr int PR_CK = 64;                 // k rows per weight chunk (64 x 128 floats = S_SLOT)
-constexpr int PR_MAXCHUNK = 64;           // chunks per (chain, rank): L = 4, 256 first-layer inputs -> 3 * 17 + 12 = 63
-constexpr int PR_MISC = 4096;             // floats of small per-CTA state + the staged HER images of the 8 rows
-constexpr int PR_STAGE_OFF = 512;
-constexpr size_t PR_SMEM_BYTES = (size_t)(S_NSLOT * S_SLOT + 2 * S_XT + S_RED + PR_MISC) * 4 + 128;
-static_assert(PR_CK * PR_NC == S_SLOT && PR_ROWS * S_H == S_XT && 8 * PR_ROWS * PR_NC == S_RED, "pair kernel reuses the ring / xT / partial areas");
-
-constexpr int PR_MAXMAPS = 28;            // weight blocks of the four nets + the transposes (L = 4: 4 * 5 + 2 * 3 = 26)
-
-struct PairChunk {
-  int map;            // tensor map of the weight block [rows][256] this chunk comes from
-  int krow;           // first row of the block
-  short nrows;        // rows of the chunk that exist (<= 64; the TMA unit zero-fills the rest of the box)
-  short wait;         // 1: the first chunk of a layer whose k rows are the PARTNER's columns of the previous layer
-  int k0;             // first k row of the layer this chunk covers
-};
-
-struct PairParams {
-  StreamParams S;
-  int nch[2][2];                          // [role][rank]
-  int pch0[2];                            // chunks of a first layer: [0] pi nets, [1] Q nets
-  PairChunk ch[2][2][PR_MAXCHUNK];        // [role: actor, critic][cluster rank]
-  alignas(64) CUtensorMap maps[PR_MAXMAPS];   // box = 128 columns x 64 rows, dense
-};
-
-struct PairRing {
-  const PairChunk* chunks;
-  const float* slots;
-  uint32_t full, empty;
-  int cons;
-};
-
-// the activation exchange of a CTA pair (see above); every consumer thread holds the same state.  A thread's 16 bytes
-// travel as ONE st.async that also counts its bytes on the receiver's mbarrier (complete_tx, like a TMA copy): no
-// release / acquire round trip and no per-thread arrive (256 remote arrives per layer cost ~4 k cycles, measured).
-struct PairX {
-  uint32_t bar_local[2], bar_remote[2];   // mbarriers (count 1 = the receiver's own expect_tx), alternating per exchange
-  uint32_t x_local, x_remote;             // shared address of xa here / in the partner (xb follows at + S_XT floats)
-  uint32_t word_remote;                   // a scratch word of the partner (payload of a data-less rendezvous)
-  int step;                               // exchanges issued so far
-  bool pending;                           // the partner's half of exchange `step - 1` has not been waited for yet
-  long long* dbg;                         // debug stamps (thread 0 of CTA 0, CUR_ROWS_TIMELINE=1) or nullptr
-  __device__ __forceinline__ void stamp() {
-    if (dbg != nullptr) *dbg++ = clock64();
-  }
-  __device__ __forceinline__ void wait() {
-    if (pending) {
-      const int s = step - 1;
-      stamp();
-      mbar_wait_cluster(bar_local[s & 1], (uint32_t)((s >> 1) & 1));
-      stamp();
-      pending = false;
-    }
-  }
-  // 4 rows (4 * rh ..) of column `gcol` of the layer output: into both CTAs' transposed buffer `xT`
-  __device__ __forceinline__ void put(float* xT, int gcol, int rh, const float (&v)[4]) {
-    float* dst = xT + gcol * PR_ROWS + 4 * rh;
-    *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-    const uint32_t ra = x_remote + (smem_addr(dst) - x_local);
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.f32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(ra),
-                 "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "r"(bar_remote[step & 1])
-                 : "memory");
-    if (threadIdx.x == 0) mbar_expect_tx(bar_local[step & 1], S_CONSUMERS * 16);     // what the partner sends me
-    ++step;
-    pending = true;
-  }
-  // pair-wide rendezvous of the consumers without data: nobody passes before both CTAs are done with what they read
-  // so far (a first layer / a backward seed does not depend on the partner, so it could otherwise overwrite a buffer the
-  // partner is still reading)
-  __device__ __forceinline__ void sync() {
-    wait();
-    consumer_sync();                      // every thread of this CTA is done reading
-    if (threadIdx.x == 0) {
-      asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.f32 [%0], %1, [%2];" ::"r"(word_remote),
-                   "f"(0.f), "r"(bar_remote[step & 1])
-                   : "memory");
-      mbar_expect_tx(bar_local[step & 1], 4);
-    }
-    ++step;
-    pending = true;
-    wait();
-  }
-};
-
-template <class PT>
-__device__ __forceinline__ void pair_gemv_chunks(const PT& P, PairRing& rg, PairX& X, int nchunks, const float* __restrict__ xT,
-                                                 float2 (&acc)[4][4]) {
-  const int cg = threadIdx.x & 31, ks = threadIdx.x >> 5;
-#pragma unroll 1
-  for (int c = 0; c < nchunks; ++c) {
-    const int slot = rg.cons % S_NSLOT;
-    const int nrows = rg.chunks[rg.cons].nrows, k0 = rg.chunks[rg.cons].k0;
-    if (rg.chunks[rg.cons].wait) X.wait();
-    mbar_wait(rg.full + 8 * slot, (rg.cons / S_NSLOT) & 1);
-    const float* ws = rg.slots + slot * S_SLOT + 4 * cg;
-    const float* xs = xT + (k0 + ks * 8) * PR_ROWS;
-    if (P.dbg_skip_math) {
-    } else if (ks * 8 < nrows) {
-      // a ragged first-layer block: the TMA unit zero-filled the box rows beyond nrows and pair_build_x zeroed the x
-      // rows beyond the fan-in, so a k-slice that starts inside the block runs unguarded (warp-uniform test)
-      float4 w[8];
-#pragma unroll
-      for (int kk = 0; kk < 8; ++kk) w[kk] = *reinterpret_cast<const float4*>(ws + (ks * 8 + kk) * PR_NC);
-#pragma unroll
-      for (int kk = 0; kk < 8; ++kk) fma_row<PR_ROWS>(acc, xs + kk * PR_ROWS, w[kk]);
-    }
-    __syncwarp();
-    if ((threadIdx.x & 31) == 0) mbar_arrive(rg.empty + 8 * slot);
-    ++rg.cons;
-  }
-}
-
-// One dense layer for the pair's 8 rows and this CTA's 128 columns.  Returns, for the thread's column `tid & 127` and
-// its 4 rows 4 * (tid >> 7) .., the pre-activation sums (without bias).
-template <class PT>
-__device__ __forceinline__ void pair_layer_gemv(const PT& P, PairRing& rg, PairX& X, int nchunks, const float* xT, float* red,
-                                                float (&v)[4]) {
-  float2 acc[4][4];
-#pragma unroll
-  for (int p = 0; p < 4; ++p)
-#pragma unroll
-    for (int c = 0; c < 4; ++c) acc[p][c] = make_float2(0.f, 0.f);
-  X.stamp();
-  pair_gemv_chunks(P, rg, X, nchunks, xT, acc);
-  X.stamp();
-  const int cg = threadIdx.x & 31, ks = threadIdx.x >> 5;
-#pragma unroll
-  for (int p = 0; p < 4; ++p) {
-    *reinterpret_cast<float4*>(red + (ks * PR_ROWS + 2 * p) * PR_NC + 4 * cg) =
-        make_float4(acc[p][0].x, acc[p][1].x, acc[p][2].x, acc[p][3].x);
-    *reinterpret_cast<float4*>(red + (ks * PR_ROWS + 2 * p + 1) * PR_NC + 4 * cg) =
-        make_float4(acc[p][0].y, acc[p][1].y, acc[p][2].y, acc[p][3].y);
-  }
-  consumer_sync();
-  const int col = threadIdx.x & (PR_NC - 1), rh = threadIdx.x >> 7;
-#pragma unroll
-  for (int r = 0; r < 4; ++r) {
-    const float* p = red + (4 * rh + r) * PR_NC + col;
-    constexpr int SL = PR_ROWS * PR_NC;             // one k-slice of partials
-    v[r] = ((p[0] + p[SL]) + (p[2 * SL] + p[3 * SL])) + ((p[4 * SL] + p[5 * SL]) + (p[6 * SL] + p[7 * SL]));
-  }
-}
-
-// One forward net for the pair's 8 rows (first-layer input already in `xa` of both CTAs).  Returns the buffer that holds
-// the last hidden activations; the partner's half of it is still in flight (X.wait() before reading all of it).
-template <class PT>
-__device__ __forceinline__ float* pair_forward_net(const PT& P, PairRing& rg, PairX& X, int ch0, int L, int gc0, float* xa,
-                                                   float* xb, float* red, const float* const* bias, float* const* h_out,
-                                                   int64_t row0) {
-  const int col = threadIdx.x & (PR_NC - 1), rh = threadIdx.x >> 7, gcol = gc0 + col;
-  float* xin = xa;
-  float* xout = xb;
-  for (int l = 0; l < L; ++l) {
-    float v[4];
-    const float b = bias[l][gcol];                // in flight during the layer (an exposed L2 round trip otherwise)
-    pair_layer_gemv(P, rg, X, l == 0 ? ch0 : S_H / PR_CK, xin, red, v);
-#pragma unroll
-    for (int r = 0; r < 4; ++r) v[r] = fmaxf(v[r] + b, 0.f);
-    if (h_out != nullptr) {
-#pragma unroll
-      for (int r = 0; r < 4; ++r) h_out[l][(row0 + 4 * rh + r) * S_H + gcol] = v[r];
-    }
-    X.put(xout, gcol, rh, v);
-    consumer_sync();
-    X.stamp();
-    float* t = xin; xin = xout; xout = t;
-  }
-  return xin;
-}
-
-// backward through the hidden layers L-1 .. 1 of one net from the seed already exchanged into `xin`: masks from the
-// row-major activations `h`, deltas optionally stored row-major into `dout`
-template <class PT>
-__device__ __forceinline__ float* pair_backward_net(const PT& P, PairRing& rg, PairX& X, int L, int gc0, float* xin, float* xout,
-                                                    float* red, float* const* h, float* const* dout, int64_t row0) {
-  const int col = threadIdx.x & (PR_NC - 1), rh = threadIdx.x >> 7, gcol = gc0 + col;
-  for (int l = L - 1; l >= 1; --l) {
-    float m[4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r) m[r] = __ldcg(h[l - 1] + (row0 + 4 * rh + r) * S_H + gcol);   // ReLU masks of layer l-1
-    float v[4];
-    pair_layer_gemv(P, rg, X, S_H / PR_CK, xin, red, v);
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      v[r] = relu_mask(v[r], m[r]);
-      if (dout != nullptr) dout[l - 1][(row0 + 4 * rh + r) * S_H + gcol] = v[r];
-    }
-    X.put(xout, gcol, rh, v);
-    consumer_sync();
-    float* t = xin; xin = xout; xout = t;
-  }
-  return xin;
-}
-
-// first-layer input of the pair's 8 rows (two 4-row halves of build_x); the row-major global copy only from rank 0
-__device__ __forceinline__ void pair_build_x(const StreamParams& P, float* xT, int64_t row0, bool target, int act_kind,
-                                             const float* ths, float* gout, const float* stage) {
-  const int ss = P.plan.stage_stride;
-  build_x(P, xT, PR_ROWS, 0, row0, target, act_kind, ths, gout, stage);
-  build_x(P, xT, PR_ROWS, 4, row0 + 4, target, act_kind, ths ? ths + 4 * S_DU : nullptr, gout,
-          stage ? stage + 4 * ss : nullptr);
-  // k rows [KP, KP + 64) are multiplied with zero-filled weight rows of the ragged first-layer chunks: keep them finite
-  const int kend = (P.KP + PR_CK < S_H) ? P.KP + PR_CK : S_H;
-  for (int i = P.KP * PR_ROWS + threadIdx.x; i < kend * PR_ROWS; i += S_CONSUMERS) xT[i] = 0.f;
-}
-
-__device__ __forceinline__ void pair_consumer(const PairParams& PP, float* ringf, float* xa, float* xb, float* red,
-                                              float* misc, uint32_t full, uint32_t empty, uint32_t xbar) {
-  const StreamParams& P = PP.S;
-  float* s_th = misc;                 // [8][8] tanh output of this chain's pi net (= pi / max_u)
-  float* s_q = misc + 64;             // [8][8] main.Q of the 8 rows
-  float* s_qt = misc + 128;           // [8][8] target.Q
-  float* s_dq = misc + 192;           // [8] backward seed; [8..16): squared TD error
-  float* s_dy = misc + 256;           // [8][8]
-  float* s_r = misc + 320;            // [8] rewards of the rows (fused HER sampling)
-  const float** m_src = reinterpret_cast<const float**>(misc + 336);     // [8][3] source addresses
-  float* her_stage = misc + PR_STAGE_OFF;                                 // [8][stage_stride]
-
-  const int tid = threadIdx.x;
-  const uint32_t rank = cluster_ctarank();
-  const uint32_t pair = blockIdx.x >> 1;
-  const uint32_t role = pair & 1;                              // 0: actor chain, 1: critic chain (independent pairs)
-  const int64_t row0 = (int64_t)(pair >> 1) * PR_ROWS;
-  const cur_net_desc& d = P.d;
-  const int L = P.L;
-  const int gc0 = (int)rank * PR_NC, col = tid & (PR_NC - 1), rh = tid >> 7, gcol = gc0 + col;
-  const bool lead = rank == 0;                                 // writes what both CTAs compute redundantly
-
-  PairRing rg;
-  rg.chunks = PP.ch[role][rank]; rg.slots = ringf; rg.full = full; rg.empty = empty; rg.cons = 0;
-  PairX X;
-  X.bar_local[0] = xbar; X.bar_local[1] = xbar + 8;
-  X.bar_remote[0] = map_to_cta(xbar, rank ^ 1u); X.bar_remote[1] = map_to_cta(xbar + 8, rank ^ 1u);
-  X.x_local = smem_addr(xa); X.x_remote = map_to_cta(X.x_local, rank ^ 1u);
-  X.word_remote = map_to_cta(smem_addr(misc + 400), rank ^ 1u);
-  X.step = 0; X.pending = false;
-  X.dbg = nullptr;
-
-  const float inv_n = 1.0f / (float)P.grad_rows;      // scale of the backward seeds
-  const float* stage = nullptr;
-  if (P.fused_her) {
-    sample_rows(P, row0, her_stage, m_src, s_r, red, PR_ROWS);
-    stage = her_stage;
-  }
-  const float hi_clip = P.clip_pos ? 0.f : INFINITY;
-  const bool tl_on = P.tl != nullptr && blockIdx.x == 0 && tid == 0;
-#define PR_TL(i) do { if (tl_on) P.tl[i] = clock64(); } while (0)
-
-  if (role == 1) {
-    // ===== critic pair: target.pi -> target.Q(o2, g2, pi_target), main.Q(o, g, u), TD loss, the critic's backward chain
-    pair_build_x(P, xa, row0, true, 0, nullptr, nullptr, stage);
-    consumer_sync();
-    float* xl = pair_forward_net(P, rg, X, PP.pch0[0], L, gc0, xa, xb, red, P.bPT, nullptr, row0);
-    X.wait();
-    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutPT, d.dimu, 1, d.dimu, P.boutPT, s_th);
-    consumer_sync();
-    if (tid < PR_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);
-    X.sync();
-    consumer_sync();
-    pair_build_x(P, xa, row0, true, 2, s_th, nullptr, stage);
-    consumer_sync();
-    xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQT, nullptr, row0);
-    X.wait();
-    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQT, 1, 1, 1, P.boutQT, s_qt);
-    X.sync();
-    consumer_sync();
-    // main.Q(o, g, u)
-    pair_build_x(P, xa, row0, false, 1, nullptr, lead ? P.Xq : nullptr, stage);
-    consumer_sync();
-    xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQ, P.hq, row0);
-    X.wait();
-    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
-    consumer_sync();
-    // critic loss (ddpg.py:436-439) and its backward seed
-    if (tid < PR_ROWS) {
-      const int64_t row = row0 + tid;
-      const float rew = stage ? s_r[tid] : P.r[row];
-      const float tgt = fminf(fmaxf(rew + P.gamma * s_qt[tid * S_DU], -P.clip_return), hi_clip);
-      const float diff = tgt - s_q[tid * S_DU];
-      s_dq[tid] = -2.0f * inv_n * diff;          // d mean((tgt - Q)^2) / dQ
-      s_dq[8 + tid] = diff * diff;
-      if (lead) P.dQ[row] = s_dq[tid];
-    }
-    X.sync();
-    consumer_sync();
-    if (lead && tid < 2) {                        // per 4 rows, like the 4-row kernel (same fold in rows_dw_kernel)
-      float ssq = 0.f;
-      for (int r = 0; r < 4; ++r) ssq += s_dq[8 + 4 * tid + r];
-      P.loss_part[((row0 >> 2) + tid) * 4] = ssq;
-    }
-    // backward through main.Q (critic chain): gradient at the last hidden layer is dQ * Wout^T (Wout is [H][1])
-    {
-      const float wq = __ldg(P.WoutQ + gcol);
-      float v[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        v[r] = relu_mask(s_dq[4 * rh + r] * wq, __ldcg(P.hq[L - 1] + (row0 + 4 * rh + r) * S_H + gcol));
-        P.dc[L - 1][(row0 + 4 * rh + r) * S_H + gcol] = v[r];
-      }
-      X.put(xa, gcol, rh, v);
-      consumer_sync();
-    }
-    pair_backward_net(P, rg, X, L, gc0, xa, xb, red, P.hq, P.dc, row0);
-    X.wait();
-    return;
-  }
-
-  // ===== actor pair: main.pi -> main.Q(o, g, pi) -> actor loss -> backward through main.Q and main.pi =====
-  PR_TL(0);
-  pair_build_x(P, xa, row0, false, 0, nullptr, lead ? P.Xp : nullptr, stage);
-  consumer_sync();
-  PR_TL(1);
-  {
-    if (tl_on) X.dbg = P.tl + 8;          // main.pi forward in detail: 24 stamps at most
-    X.stamp();
-    float* xl = pair_forward_net(P, rg, X, PP.pch0[0], L, gc0, xa, xb, red, P.bP, P.hp, row0);
-    X.wait();
-    X.dbg = nullptr;
-    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutP, d.dimu, 1, d.dimu, P.boutP, s_th);
-    consumer_sync();
-    if (tid < PR_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) s_th[tid] = tanhf(s_th[tid]);   // actor_critic.py:89
-    X.sync();
-    consumer_sync();
-  }
-  PR_TL(2);
-  PR_TL(3);
-  pair_build_x(P, xa, row0, false, 2, s_th, nullptr, stage);
-  consumer_sync();
-  {
-    float* xl = pair_forward_net(P, rg, X, PP.pch0[1], L, gc0, xa, xb, red, P.bQ, P.hqp, row0);
-    X.wait();
-    small_out<S_H>(xl, PR_ROWS, 0, PR_ROWS, P.WoutQ, 1, 1, 1, P.boutQ, s_q);
-    consumer_sync();
-  }
-  PR_TL(4);
-  PR_TL(5);
-  // ===== actor loss terms (ddpg.py:440-441) and backward seed =====
-  if (tid < PR_ROWS) {
-    s_dq[tid] = -inv_n;                        // d (-mean(Q_pi)) / dQ_pi
-    if (lead) P.q_pi[row0 + tid] = s_q[tid * S_DU];
-  }
-  if (lead && tid < 2) {
-    float sq = 0.f, sth = 0.f;
-    for (int r = 4 * tid; r < 4 * tid + 4; ++r) {
-      sq += s_q[r * S_DU];
-      for (int j = 0; j < d.dimu; ++j) sth += s_th[r * S_DU + j] * s_th[r * S_DU + j];
-    }
-    float* lp = P.loss_part + ((row0 >> 2) + tid) * 4;
-    lp[1] = sq; lp[2] = sth; lp[3] = 0.f;
-  }
-  X.sync();
-  consumer_sync();
-  // ===== backward through main.Q, actor-through-critic chain =====
-  {
-    {
-      const float wq = __ldg(P.WoutQ + gcol);
-      float v[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r)
-        v[r] = relu_mask(s_dq[4 * rh + r] * wq, __ldcg(P.hqp[L - 1] + (row0 + 4 * rh + r) * S_H + gcol));
-      X.put(xa, gcol, rh, v);
-      consumer_sync();
-    }
-    float* xin = pair_backward_net(P, rg, X, L, gc0, xa, xb, red, P.hqp, nullptr, row0);
-    X.wait();
-    // gradient wrt the action inputs of main.Q, then through tanh and the action penalty (ddpg.py:440-441):
-    // d pi_loss/d(pre-tanh) = (dL/d(pi/max_u) + action_l2*2/(B*dimu)*th) * (1 - th^2)
-    small_out<S_H>(xin, PR_ROWS, 0, PR_ROWS, P.W0Q_act, 1, S_H, d.dimu, nullptr, s_dy);
-    consumer_sync();
-    if (tid < PR_ROWS * S_DU) {
-      const int r = tid >> 3, j = tid & (S_DU - 1);
-      float v = 0.f;
-      if (j < d.dimu) {
-        const float coef = P.action_l2 * 2.0f / (float)(P.grad_rows * d.dimu);
-        const float th = s_th[tid];
-        v = (s_dy[tid] + coef * th) * (1.f - th * th);
-      }
-      s_dy[tid] = v;
-      if (lead && j < P.lddy) P.dy[(row0 + r) * P.lddy + j] = v;
-    }
-    X.sync();
-    consumer_sync();
-  }
-  PR_TL(6);
-  // ===== backward through main.pi =====
-  {
-    {
-      float v[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) v[r] = 0.f;
-      for (int j = 0; j < d.dimu; ++j) {
-        const float wj = __ldg(P.WoutP + (int64_t)gcol * d.dimu + j);
-#pragma unroll
-        for (int r = 0; r < 4; ++r) v[r] = fmaf(s_dy[(4 * rh + r) * S_DU + j], wj, v[r]);
-      }
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        v[r] = relu_mask(v[r], __ldcg(P.hp[L - 1] + (row0 + 4 * rh + r) * S_H + gcol));
-        P.dp[L - 1][(row0 + 4 * rh + r) * S_H + gcol] = v[r];
-      }
-      X.put(xa, gcol, rh, v);
-      consumer_sync();
-    }
-    pair_backward_net(P, rg, X, L, gc0, xa, xb, red, P.hp, P.dp, row0);
-    X.wait();
-  }
-  PR_TL(7);
-#undef PR_TL
-}
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(S_THREADS, 1)
-ddpg_stream_pair_kernel(const __grid_constant__ PairParams PP) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  float* ringf = reinterpret_cast<float*>(smem_raw);
-  float* xa = ringf + S_NSLOT * S_SLOT;
-  float* xb = xa + S_XT;
-  float* red = xb + S_XT;
-  float* misc = red + S_RED;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(misc + PR_MISC);      // full[4], empty[4], xchg[2]
-  const int tid = threadIdx.x;
-  const uint32_t full = smem_addr(bars), empty = smem_addr(bars + S_NSLOT), xbar = smem_addr(bars + 2 * S_NSLOT);
-  if (tid == 0) {
-    for (int i = 0; i < S_NSLOT; ++i) {
-      mbar_init(full + 8 * i, 1);
-      mbar_init(empty + 8 * i, S_CONSUMERS / 32);
-    }
-    mbar_init(xbar, 1);
-    mbar_init(xbar + 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  pdl_launch_dependents();
-  pdl_wait();               // everything below reads what the previous kernel (weight gradients + Adam of the last update) wrote
-  cluster_sync_all();       // both CTAs' barriers are initialised before anybody arrives on them (locally or remotely)
-
-  if (tid >= S_CONSUMERS) {
-    // ------------------------------------------------------------ producer warp: stream this CTA's half of every chunk
-    if (tid == S_CONSUMERS) {
-      const uint32_t rank = cluster_ctarank(), role = (blockIdx.x >> 1) & 1;
-      const PairChunk* my = PP.ch[role][rank];
-      const int total = PP.nch[role][rank];
-      const uint32_t ring_s = smem_addr(ringf);
-      for (int i = 0; i < total; ++i) {
-        const int slot = i % S_NSLOT, round = i / S_NSLOT;
-        if (round > 0) mbar_wait(empty + 8 * slot, (round - 1) & 1);
-        mbar_expect_tx(full + 8 * slot, (uint32_t)S_SLOT * 4);          // a box always counts in full (zero-filled rows too)
-        tc_tma_2d(ring_s + slot * S_SLOT * 4, &PP.maps[my[i].map], (int)rank * PR_NC, my[i].krow, full + 8 * slot);
-      }
-    }
-  } else {
-    pair_consumer(PP, ringf, xa, xb, red, misc, full, empty, xbar);
-  }
-  cluster_sync_all();       // neither CTA leaves while the partner may still store into it / arrive on its barriers
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1244,7 +731,6 @@ constexpr int A_MAXCHUNK = 64;          // pi + Q forward chunks (L = 4: 2 * 27)
 struct ActParams {
   cur_net_desc d;
   int in_sp, in_g, KP, L, nchunks;
-  int dbg_skip_math;         // (read by the shared GEMV core)
   int ch0[2];                // chunks of the first layer: [0] pi, [1] Q
   int64_t n;
   const float *o, *g, *td;
@@ -1396,7 +882,6 @@ struct ActExpert {
 struct ActGroupParams {
   cur_net_desc d;
   int in_sp, in_g, KP, L, nchunks;
-  int dbg_skip_math;         // (read by the shared GEMV core)
   int ch0[2];
   const float *o, *g, *td, *ag;
   float clip;
@@ -1543,8 +1028,6 @@ __device__ __noinline__ void xchg_timeout_check(unsigned long long t0, int* erro
 }
 
 struct DwTail {
-  int dbg_skip_stage;              // debug (CUR_DW_SKIP_STAGE=1): tiles run on whatever their shared memory holds
-  int pdl_late;                    // trigger the dependent launch when the tile is done (not at the start)
   AdamCtx ax;                      // ax.theta == NULL: gradients only
   const float* neg_a_table;
   int table_len;
@@ -1965,7 +1448,6 @@ rows_dw_kernel(const __grid_constant__ GemmBatch G, const __grid_constant__ DwTa
   // fenced and took a ticket AFTER its tile and the last one to finish did the fold - ~3 us behind the slowest tile.)
   const unsigned int n_tile_ctas = gridDim.x - (T.last_chunk ? 1u : 0u);
   if (blockIdx.x >= n_tile_ctas) {
-    pdl_wait();
     const long long st = T.step_counter ? *T.step_counter : 0;   // value BEFORE this update's bump
     float* lp = As;                                              // the partials travel in parallel (one round trip) ...
     for (int i = threadIdx.x; i < 4 * T.n_clusters; i += GEMM_THREADS) lp[i] = __ldcg(T.loss_part + i);
@@ -1992,7 +1474,6 @@ rows_dw_kernel(const __grid_constant__ GemmBatch G, const __grid_constant__ DwTa
       *T.ticket = 0u;
       __threadfence();
     }
-    pdl_launch_dependents();
     return;
   }
   long long* tl = nullptr;
@@ -2003,8 +1484,6 @@ rows_dw_kernel(const __grid_constant__ GemmBatch G, const __grid_constant__ DwTa
   }
   if (tl) tl[0] = clock64();
   if (T.tl != nullptr && threadIdx.x == 0 && blockIdx.x < 512) T.tl[1088 + 2 * blockIdx.x] = (long long)globaltimer_ns();
-  if (!T.pdl_late) pdl_launch_dependents();
-  pdl_wait();                                                    // activations / deltas of the stream kernel, the step counter
   int pi = 0;
   {
     // the problem of this tile: last p with tile_begin[p] <= blockIdx.x (bisection: a linear walk over the ~30 problems
@@ -2027,8 +1506,7 @@ rows_dw_kernel(const __grid_constant__ GemmBatch G, const __grid_constant__ DwTa
   const int tile = blockIdx.x - P.tile_begin;
   const int tm = (P.variant == DW_FULLK) ? tile / P.tiles_n : 0, tn = tile - tm * P.tiles_n;
   // ---- the operands first (one round trip) ...
-  if (T.dbg_skip_stage) {                                        // debug: what the launch costs without its operand traffic
-  } else if (P.variant == DW_FULLK) dw_stage_fullk(P, As, Bs, tm * GT, tn * GT);
+  if (P.variant == DW_FULLK) dw_stage_fullk(P, As, Bs, tm * GT, tn * GT);
   else if (P.variant == DW_SKINNY) dw_stage_skinny(P, As, Bs, tile * GT);
   // ---- ... and what depends on the device step counter (two dependent round trips of thread 0) while they travel
   long long st = 0;
@@ -2070,7 +1548,6 @@ rows_dw_kernel(const __grid_constant__ GemmBatch G, const __grid_constant__ DwTa
     if (blockIdx.x < 512) T.tl[1089 + 2 * blockIdx.x] = (long long)globaltimer_ns();
     tl_mark_max(T.tl + TL_MARKS + 4 * (int)(st & 7) + 3);
   }
-  pdl_launch_dependents();
   if (tl) tl[3] = clock64();
 }
 
@@ -2145,7 +1622,7 @@ constexpr int64_t ROWS_MAX_BATCH = 1024;
 
 static bool rows_supported(const cur_net_desc* d, int64_t n) {
   if (check_desc(d) != CUR_OK) return false;
-  // hidden 256, and 64 / 128 for networks run at their true width (pad_hidden='native'; the CTA-pair kernel is 256 only)
+  // hidden 256, and 64 / 128 for networks run at their true width (pad_hidden='native')
   if ((d->hidden != 64 && d->hidden != 128 && d->hidden != S_H) || d->layers < 1 || d->layers > S_MAXL) return false;
   if (d->dimu > S_DU || n <= 0 || (n % S_ROWS) != 0 || n > ROWS_MAX_BATCH) return false;
   const NetLayout q = net_layout(*d, 0), p = net_layout(*d, 1);
@@ -2181,14 +1658,14 @@ static void build_dw_batch(GemmBatch& G, const NetLayout& LQ, const NetLayout& L
 }
 
 template <int H>
-static int launch_stream(cudaLaunchConfig_t& cfg, const StreamParams& P) {
+static int launch_stream(unsigned grid, cudaStream_t s, const StreamParams& P) {
   static bool configured = false;
   if (!configured) {
     CUR_CUDA_TRY(cudaFuncSetAttribute(ddpg_stream_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)S_SMEM_BYTES));
     configured = true;
   }
-  CUR_CUDA_TRY(cudaLaunchKernelEx(&cfg, ddpg_stream_kernel<H>, P));
+  ddpg_stream_kernel<H><<<grid, S_THREADS, S_SMEM_BYTES, s>>>(P);
   return CUR_OK;
 }
 
@@ -2207,25 +1684,6 @@ static int launch_actions(unsigned blocks, cudaStream_t s, const PT& P) {
   }
   kernel<<<blocks, S_THREADS, S_SMEM_BYTES, s>>>(P);
   return CUR_OK;
-}
-
-// launch configuration; CUR_PDL=1 adds programmatic stream serialisation (measured: batch 256 60.2 us with, 58.3 us
-// without - the early-scheduled CTAs of the next kernel do not pay for what they displace - so it is off by default)
-static void pdl_config(cudaLaunchConfig_t& cfg, cudaLaunchAttribute* at, unsigned grid, unsigned block, size_t smem,
-                       cudaStream_t s, int which = 0 /* 0: stream kernel, 1: weight-gradient launch */) {
-  // CUR_PDL: 1 both launches may start early (trigger at the start of the previous kernel), 2 both with the trigger at the
-  // END of the previous kernel's CTAs, 3 only the weight-gradient launch, 4 only the stream kernel
-  static const char mode = getenv("CUR_PDL") != nullptr ? getenv("CUR_PDL")[0] : '0';
-  const bool on = mode == '1' || mode == '2' || (mode == '3' && which == 1) || (mode == '4' && which == 0);
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(block, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = on ? 1 : 0;
-  cfg.attrs = at;
-  cfg.numAttrs = on ? 1 : 0;
 }
 
 }  // namespace cur
@@ -2428,107 +1886,11 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
   }
   P.tl = tl_on ? tl_dev : nullptr;
   P.tl_step = h->step_counter;
-  P.dbg_skip_math = getenv("CUR_ROWS_SKIP_MATH") != nullptr;
-  static const int pdl_late = (getenv("CUR_PDL") != nullptr && getenv("CUR_PDL")[0] == '2') ? 1 : 0;
-  P.pdl_late = pdl_late;
 
   const unsigned int n_ctas = (unsigned int)(n / S_ROWS);
-  // CTA-pair form (column split over a 2-CTA cluster, 8 rows per pair): half the weight bytes per SM
-  static const int pair_mode = getenv("CUR_ROWS_PAIR") ? atoi(getenv("CUR_ROWS_PAIR")) : 0;   // measured slower, see profiles/README.md
-  const bool use_pair = pair_mode != 0 && H == S_H && (n % PR_ROWS) == 0 && d->dimu <= 4 &&
-                        (her == nullptr || PR_ROWS * P.plan.stage_stride <= PR_MISC - PR_STAGE_OFF);
-  if (use_pair) {
-    static bool pair_configured = false;
-    if (!pair_configured) {
-      CUR_CUDA_TRY(cudaFuncSetAttribute(ddpg_stream_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                        (int)PR_SMEM_BYTES));
-      pair_configured = true;
-    }
-    static thread_local PairParams PP;                       // ~20 KB: kept off the stack; rebuilt on every call
-    PP.S = P;
-    // one tensor map per weight block (encoded once per address: the arenas and the workspace do not move)
-    struct MapKey { const float* ptr; int rows; };
-    static thread_local MapKey cache_key[256];
-    static thread_local CUtensorMap cache_map[256];
-    static thread_local int cache_n = 0;
-    int n_maps = 0;
-    MapKey used[PR_MAXMAPS];
-    auto map_of = [&](const float* ptr, int rows, int* out) -> int {
-      for (int i = 0; i < n_maps; ++i)
-        if (used[i].ptr == ptr && used[i].rows == rows) { *out = i; return CUR_OK; }
-      CUR_REQUIRE(n_maps < PR_MAXMAPS, "too many weight blocks for the CTA-pair rows schedule");
-      int hit = -1;
-      for (int i = 0; i < cache_n; ++i)
-        if (cache_key[i].ptr == ptr && cache_key[i].rows == rows) { hit = i; break; }
-      if (hit < 0) {
-        hit = cache_n < 256 ? cache_n++ : 0;
-        CUR_TRY(tc_make_plain_map(&cache_map[hit], ptr, rows, H, H, PR_NC, PR_CK));
-        cache_key[hit].ptr = ptr; cache_key[hit].rows = rows;
-      }
-      PP.maps[n_maps] = cache_map[hit];
-      used[n_maps].ptr = ptr; used[n_maps].rows = rows;
-      *out = n_maps++;
-      return CUR_OK;
-    };
-    for (int rank = 0; rank < 2; ++rank) {
-      int m = 0;
-      PairChunk* pl = nullptr;
-      // a row block [nrows][256] as chunks of <= 64 rows of this rank's 128 columns; `exchanged`: the k rows are the
-      // columns of the previous layer's output, so the rank's own half comes first and the partner's half waits
-      auto rows_of = [&](const float* src, int nrows, int k0, bool exchanged) -> int {
-        int mi = 0;
-        CUR_TRY(map_of(src, nrows, &mi));
-        if (!exchanged) {
-          for (int r = 0; r < nrows; r += PR_CK) {
-            CUR_REQUIRE(m < PR_MAXCHUNK, "too many weight chunks for the CTA-pair rows schedule");
-            PairChunk& C = pl[m++];
-            C.map = mi; C.krow = r; C.nrows = (short)((nrows - r < PR_CK) ? nrows - r : PR_CK); C.wait = 0; C.k0 = k0 + r;
-          }
-          return CUR_OK;
-        }
-        for (int half = 0; half < 2; ++half) {
-          const int hk = (half == 0 ? rank : 1 - rank) * PR_NC;          // first k row of this half
-          for (int r = 0; r < PR_NC; r += PR_CK) {
-            CUR_REQUIRE(m < PR_MAXCHUNK, "too many weight chunks for the CTA-pair rows schedule");
-            PairChunk& C = pl[m++];
-            C.map = mi; C.krow = hk + r; C.nrows = PR_CK; C.wait = (short)((half == 1 && r == 0) ? 1 : 0); C.k0 = k0 + hk + r;
-          }
-        }
-        return CUR_OK;
-      };
-      auto forward_net = [&](const float* th, const NetLayout& NL, int* first) -> int {
-        const int before = m;
-        CUR_TRY(rows_of(th + NL.off_W0, NL.in_s, 0, false));
-        if (NL.in_g > 0) CUR_TRY(rows_of(th + NL.off_W0g, NL.in_g, NL.in_s, false));
-        if (first) *first = m - before;
-        for (int l = 1; l < L; ++l) CUR_TRY(rows_of(th + NL.off_W[l], H, 0, true));
-        return CUR_OK;
-      };
-      pl = PP.ch[0][rank]; m = 0;
-      CUR_TRY(forward_net(mP, LP, &PP.pch0[0]));
-      CUR_TRY(forward_net(mQ, LQ, &PP.pch0[1]));
-      for (int l = L - 1; l >= 1; --l) CUR_TRY(rows_of(w.TQ[l], H, 0, true));
-      for (int l = L - 1; l >= 1; --l) CUR_TRY(rows_of(w.TP[l], H, 0, true));
-      PP.nch[0][rank] = m;
-      pl = PP.ch[1][rank]; m = 0;
-      CUR_TRY(forward_net(tP, LP, nullptr));
-      CUR_TRY(forward_net(tQ, LQ, nullptr));
-      CUR_TRY(forward_net(mQ, LQ, nullptr));                                      // critic pair: main.Q(o,g,u) ...
-      for (int l = L - 1; l >= 1; --l) CUR_TRY(rows_of(w.TQ[l], H, 0, true));     // ... and its backward chain
-      PP.nch[1][rank] = m;
-    }
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute at[1];
-    pdl_config(cfg, at, (unsigned)(n / PR_ROWS) * 4u, S_THREADS, PR_SMEM_BYTES, s);   // (actor, critic) x (rank 0, rank 1)
-    CUR_CUDA_TRY(cudaLaunchKernelEx(&cfg, ddpg_stream_pair_kernel, PP));
-  } else {
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute at[1];
-    pdl_config(cfg, at, 2 * n_ctas, S_THREADS, S_SMEM_BYTES, s);
-    if (H == 64) CUR_TRY(launch_stream<64>(cfg, P));                     // (actor, critic) CTA pairs
-    else if (H == 128) CUR_TRY(launch_stream<128>(cfg, P));
-    else CUR_TRY(launch_stream<256>(cfg, P));
-  }
+  if (H == 64) CUR_TRY(launch_stream<64>(2 * n_ctas, s, P));                     // (actor, critic) CTA pairs
+  else if (H == 128) CUR_TRY(launch_stream<128>(2 * n_ctas, s, P));
+  else CUR_TRY(launch_stream<256>(2 * n_ctas, s, P));
   CUR_CHECK_LAUNCH();
   if (tl_on && ++tl_calls == 40) {          // debug only: one warmed-up timeline of CTA 0
     long long t[64];
@@ -2537,11 +1899,6 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
     fprintf(stderr, "[rows timeline] build %lld | main.pi %lld | main.Q x2 %lld | wait target.Q %lld | "
                     "loss+bwd Q %lld | bwd pi %lld | total %lld cycles\n",
             t[1] - t[0], t[2] - t[1], t[4] - t[3], t[5] - t[4], t[6] - t[5], t[7] - t[6], t[7] - t[0]);
-    if (use_pair) {
-      fprintf(stderr, "[pair main.pi stamps, cycles after build]");
-      for (int i = 8; i < 32 && t[i] != 0; ++i) fprintf(stderr, " %lld", t[i] - t[1]);
-      fprintf(stderr, "\n");
-    }
   }
 
   // ---- launch 2: weight gradients, one launch per 256-row chunk of the batch (K of the tiles)
@@ -2589,8 +1946,6 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
     T.xc.res_mc = x->mc_region ? reinterpret_cast<unsigned long long*>(x->mc_region) + x->arena : nullptr;
   }
   T.tl = tl_on ? tl_dev : nullptr;
-  T.pdl_late = pdl_late;
-  T.dbg_skip_stage = getenv("CUR_DW_SKIP_STAGE") != nullptr;
   const AdamCtx ax_full = T.ax;
   const int n_chunks = (int)((n + DW_KMAX - 1) / DW_KMAX);
   for (int c = 0; c < n_chunks; ++c) {
@@ -2609,12 +1964,7 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
     T.tl_skinny_block = 0;
     for (int i = 0; i < G.n; ++i)
       if (G.p[i].variant == DW_FULLK) { T.tl_skinny_block = G.p[i].tile_begin; break; }
-    {
-      cudaLaunchConfig_t cfg;
-      cudaLaunchAttribute at[1];
-      pdl_config(cfg, at, (unsigned)tiles + (last ? 1u : 0u), GEMM_THREADS, DW_SMEM_BYTES, s, 1);   // + the bookkeeping CTA
-      CUR_CUDA_TRY(cudaLaunchKernelEx(&cfg, rows_dw_kernel, G, T));
-    }
+    rows_dw_kernel<<<(unsigned)tiles + (last ? 1u : 0u), GEMM_THREADS, DW_SMEM_BYTES, s>>>(G, T);   // + the bookkeeping CTA
     CUR_CHECK_LAUNCH();
   }
   if (tl_on && tl_calls == 40) {
@@ -2716,7 +2066,6 @@ static int act_common(PT& P, const cur_net_desc* d, const float* theta, const fl
   P.d = *d;
   P.in_sp = LP.in_s; P.in_g = LQ.in_g; P.L = L;
   P.KP = (LQ.in_s + LQ.in_g + 3) / 4 * 4;
-  P.dbg_skip_math = 0;
   P.o = o; P.g = g; P.td = td; P.ag = ag; P.clip = clip_obs; P.seq = seq;
   P.pi = out_pi; P.q = out_q;
   int nc = 0;

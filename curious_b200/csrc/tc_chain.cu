@@ -96,7 +96,6 @@ struct __align__(64) ChainParams {
   int clip_pos;
   float* loss_part;               // [tiles][4]: ssq (critic), sum Q_pi, sum th^2 (actor)
   long long* tl;                  // debug timeline (clock64 stamps of CTA 0 / 1), normally NULL
-  int dbg;                        // measurement switches (CUR_CHAIN_DBG): 1 no transposed copies, 2 masks all ones
 };
 
 // ---------------------------------------------------------------------------------------------------- feeder
@@ -109,7 +108,6 @@ struct Feeder {
   int64_t row;                    // batch row
   int a_cnt;                      // k-blocks of the A operand so far (both parities count all of them)
   long long* tl;                  // debug stamps (first feeder warp, lane 0) or NULL
-  int dbg;
   int n_stamp;
   __device__ __forceinline__ void stamp() { if (tl && n_stamp < 100) tl[400 + n_stamp++] = clock64(); }
 
@@ -229,7 +227,7 @@ __device__ __forceinline__ void ch_feed_relu(Feeder& F, int g, const float* bias
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i] + b[i], 0.f);
     if (mask) mask[(int64_t)c * n + F.row] = ch_mask_word(v);
-    if (HT && !(F.dbg & 1)) ch_store_t(HT, n, F.row, c, v);
+    if (HT) ch_store_t(HT, n, F.row, c, v);
     F.push_A(v);
   }
 }
@@ -250,7 +248,7 @@ __device__ __forceinline__ void ch_out_layer(Feeder& F, int g, const float* bias
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i] + b[i], 0.f);
     if (mask) mask[(int64_t)c * n + F.row] = ch_mask_word(v);
-    if (HT && !(F.dbg & 1)) ch_store_t(HT, n, F.row, c, v);
+    if (HT) ch_store_t(HT, n, F.row, c, v);
     if (NJMAX == 1) {
       float w[32];
       ch_load32(Wout + 32 * c, w);
@@ -284,7 +282,7 @@ __device__ __forceinline__ void ch_seed(Feeder& F, const float (&dout)[NJMAX], i
   for (int c = 0; c < ChW<H>::NCH; ++c) {
     if (!F.mine()) { ++F.a_cnt; continue; }
     float v[32];
-    const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : mask[(int64_t)c * n + F.row];
+    const uint32_t mw = mask[(int64_t)c * n + F.row];
     if (NJMAX == 1) {
       float w[32];
       ch_load32(Wout + 32 * c, w);
@@ -307,7 +305,7 @@ __device__ __forceinline__ void ch_seed(Feeder& F, const float (&dout)[NJMAX], i
         v[i] = ((mw >> i) & 1u) ? s : 0.f;
       }
     }
-    if (DT && !(F.dbg & 1)) ch_store_t(DT, n, F.row, c, v);
+    if (DT) ch_store_t(DT, n, F.row, c, v);
     F.push_A(v);
   }
 }
@@ -324,11 +322,11 @@ __device__ __forceinline__ void ch_feed_mask(Feeder& F, int g, const uint32_t* m
       continue;
     }
     float v[32];
-    const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : mask[(int64_t)c * n + F.row];
+    const uint32_t mw = mask[(int64_t)c * n + F.row];
     F.ld_chunk<H>(g, c, v);
 #pragma unroll
     for (int i = 0; i < 32; ++i) v[i] = ((mw >> i) & 1u) ? v[i] : 0.f;
-    if (DT && !(F.dbg & 1)) ch_store_t(DT, n, F.row, c, v);
+    if (DT) ch_store_t(DT, n, F.row, c, v);
     if (push) F.push_A(v);
   }
 }
@@ -460,7 +458,6 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
     F.tmem_lane = tmem + ((uint32_t)(32 * q) << 16);
     F.row = (int64_t)tile * CH_BM + F.r;
     F.a_cnt = 0;
-    F.dbg = P.dbg;
     F.n_stamp = 0;
     F.tl = (tl && warp == CH_WARP_FEED0) ? tl : nullptr;
     const int64_t row = F.row, n = P.n;
@@ -527,7 +524,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
 #pragma unroll 1
       for (int c = F.par; c < ChW<H>::NCH; c += 2) {
         float v[32];
-        const uint32_t mw = (F.dbg & 2) ? 0xFFFFFFFFu : P.mqp[(int64_t)c * n + row];
+        const uint32_t mw = P.mqp[(int64_t)c * n + row];
         F.ld_chunk<H>(g, c, v);
 #pragma unroll
         for (int i = 0; i < 32; ++i) v[i] = ((mw >> i) & 1u) ? v[i] : 0.f;
@@ -936,8 +933,6 @@ int tc_chain_launch(cudaStream_t s, const cur_net_desc& d, const TcChainIO& io) 
   P.gamma = io.gamma; P.clip_return = io.clip_return; P.action_l2 = io.action_l2; P.clip_pos = io.clip_pos;
   P.loss_part = io.loss_part;
   P.tl = g_chain_timeline;
-  static const int dbg = getenv("CUR_CHAIN_DBG") ? atoi(getenv("CUR_CHAIN_DBG")) : 0;
-  P.dbg = dbg;
 
   // ---- the weights as 3xTF32 halves, once per call (the weights change with every update)
   const int64_t arena = r4(LQ.total) + r4(LP.total);

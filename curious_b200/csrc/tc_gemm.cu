@@ -82,7 +82,6 @@ struct __align__(64) TcBatch {
   TcProb p[TC_MAX_PROBS];
   int n, total_tiles;
   long long* tl;                     // debug timeline of CTA 0 (cur_tc_gemm_timeline), normally NULL
-  int raw_hi;                        // experiment: see tc_lo_of_raw
 };
 
 // Epilogue of one warp: 4 column chunks of 32 for its 32 accumulator rows.  Per chunk: both accumulators TMEM ->
@@ -292,8 +291,8 @@ __device__ __forceinline__ void tc_gemm_body(const TcBatch& G) {
       tc_bar_wait(full + 8 * s, round & 1);
       if (tl && warp == TC_SPLIT_WARP0 && kb < 16) tl[24 + 2 * kb] = clock64();
       float* st = reinterpret_cast<float*>(gen_base + s * STAGE_BYTES);
-      tc_split_tile(st, TC_A_BYTES / 4, TC_A_BYTES / 16, t, TC_SPLIT_GROUP_WARPS * 32, G.raw_hi != 0);
-      tc_split_tile(st + 2 * TC_A_BYTES / 4, B_BYTES_OWN / 4, B_BYTES_OWN / 16, t, TC_SPLIT_GROUP_WARPS * 32, G.raw_hi != 0);
+      tc_split_tile(st, TC_A_BYTES / 4, TC_A_BYTES / 16, t, TC_SPLIT_GROUP_WARPS * 32);
+      tc_split_tile(st + 2 * TC_A_BYTES / 4, B_BYTES_OWN / 4, B_BYTES_OWN / 16, t, TC_SPLIT_GROUP_WARPS * 32);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       __syncwarp();
       if (tl && warp == TC_SPLIT_WARP0 && kb < 16) tl[25 + 2 * kb] = clock64();
@@ -606,26 +605,6 @@ static int make_map(CUtensorMap* m, const float* ptr, int64_t rows, int64_t cols
   return CUR_OK;
 }
 
-// row-major [rows][cols] fp32 block, box_cols x box_rows tiles delivered dense (no swizzle) - the weight chunks of the
-// CTA-pair rows kernel (ddpg_rows.cu); rows beyond `rows` are zero-filled by the TMA unit
-int tc_make_plain_map(void* map, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows) {
-  EncodeTiledFn fn = encode_fn();
-  CUR_REQUIRE(fn != nullptr, "cuTensorMapEncodeTiled is not available");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1u, 1u};
-  CUresult rc = fn(reinterpret_cast<CUtensorMap*>(map), CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(ptr), dims,
-                   strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (rc != CUDA_SUCCESS) {
-    snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled (plain) failed (%d): rows %lld cols %lld ld %lld",
-             (int)rc, (long long)rows, (long long)cols, (long long)ld);
-    return CUR_ERR_CUDA;
-  }
-  return CUR_OK;
-}
-
 int tc_make_map(void* map, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool mn_major) {
   return make_map(reinterpret_cast<CUtensorMap*>(map), ptr, rows, cols, ld, box_rows, mn_major);
 }
@@ -803,8 +782,6 @@ int TcLauncher::flush(cudaStream_t s_main) {
   }
   if (G.n > 0) {
     B.n = G.n; B.total_tiles = G.total_tiles; B.tl = g_tc_timeline;
-    static const int raw_hi = (getenv("CUR_TC_RAW_HI") != nullptr && getenv("CUR_TC_RAW_HI")[0] == '1') ? 1 : 0;
-    B.raw_hi = raw_hi;
     if (pair) tc_gemm_pair_kernel<<<2 * G.total_tiles, TC_THREADS, TC_SMEM_BYTES, s_main>>>(B);
     else tc_gemm_kernel<<<G.total_tiles, TC_THREADS, TC_SMEM_BYTES, s_main>>>(B);
     CUR_CHECK_LAUNCH();

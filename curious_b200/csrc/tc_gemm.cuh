@@ -103,7 +103,4 @@ void tc_chain_set_timeline(long long* dev);             // 128 x int64 debug sta
 int tc_make_map(void* map /* CUtensorMap */, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows,
                 bool mn_major);
 
-int tc_make_plain_map(void* map /* CUtensorMap */, const float* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols,
-                      int box_rows);                    // dense (unswizzled) tiles, zero-filled beyond `rows`
-
 }  // namespace cur

@@ -134,23 +134,9 @@ __device__ __forceinline__ void tc_split1(float x, float& h, float& l) {
   h = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u);
   l = __uint_as_float(__float_as_uint(x - h) & 0xFFFFE000u);
 }
-__device__ __forceinline__ float tc_lo_of_raw(float x) {
-  // experiment (CUR_TC_RAW_HI=1): leave the raw fp32 in place as `hi` (valid only if the tensor core TRUNCATES fp32 to
-  // TF32 when it reads kind::tf32 operands) and write lo = x - trunc(x)
-  const float h = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-  return __uint_as_float(__float_as_uint(x - h) & 0xFFFFE000u);
-}
-__device__ __forceinline__ void tc_split_tile(float* hi, int lo_off_floats, int n4, int t, int nthreads, bool raw_hi) {
+__device__ __forceinline__ void tc_split_tile(float* hi, int lo_off_floats, int n4, int t, int nthreads) {
   float4* h4 = reinterpret_cast<float4*>(hi);
   float4* l4 = reinterpret_cast<float4*>(hi + lo_off_floats);
-  if (raw_hi) {
-#pragma unroll 4
-    for (int i = t; i < n4; i += nthreads) {
-      const float4 x = h4[i];
-      l4[i] = make_float4(tc_lo_of_raw(x.x), tc_lo_of_raw(x.y), tc_lo_of_raw(x.z), tc_lo_of_raw(x.w));
-    }
-    return;
-  }
 #pragma unroll 4
   for (int i = t; i < n4; i += nthreads) {
     const float4 x = h4[i];

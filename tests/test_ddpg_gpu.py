@@ -880,24 +880,6 @@ def test_store_episode_issues_one_packed_statistics_collective(monkeypatch):
         assert torch.equal(a.mean, b.mean) and torch.equal(a.std, b.std) and torch.equal(a.count, b.count)
 
 
-def test_pair_form_of_the_stream_kernel_in_a_subprocess():
-    """The CTA-pair form of the stream kernel (2-CTA cluster, columns of every layer split over the pair, st.async exchange
-    through distributed shared memory; opt-in with CUR_ROWS_PAIR=1 because it measured slower than the 4-row form) walks the
-    same oracle and reference-fixture checks as the default kernel.  The switch is read once per process, hence the subprocess."""
-    import subprocess
-    import sys
-    env = dict(os.environ, CUR_ROWS_PAIR='1')
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, '-m', 'pytest', '-x', '-q', '-p', 'no:cacheprovider',
-                          'tests/test_ddpg_gpu.py::test_store_sample_train_against_oracle',
-                          'tests/test_ddpg_gpu.py::test_rows_schedule_trajectory',
-                          'tests/test_ddpg_gpu.py::test_cuda_graph_path_equals_eager_path',
-                          'tests/test_reference_graph_gpu.py', '-k', 'not levels'],
-                         cwd=root, env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-    assert ' passed' in out.stdout
-
-
 def test_zz_gradient_escape_frequency():
     """Runs last in this file: how many of the per-step gradient comparisons above needed the ReLU-kink fallback (5e-4)
     because the strict bound (2e-5 of max|grad|) failed.  Printed (pytest -rP), written next to the other run records
