@@ -726,7 +726,7 @@ ddpg_stream_kernel(const __grid_constant__ StreamParams P) {
 // live in mapped pinned HOST memory (zero-copy over PCIe: a rollout step is n = 2 rows, 0.5 KB) and so may the outputs;
 // the last CTA to finish then stores the call's sequence number into a host-visible word the caller polls - no
 // memcpy calls, no stream synchronisation on the critical path of a rollout step (rollout.py:217,226).
-constexpr int A_MAXCHUNK = 64;          // pi + Q forward chunks (L = 4: 2 * 27)
+constexpr int A_MAXCHUNK = 66;          // pi + Q forward chunks (L = 4, first-layer fan-in 256: 2 * (8 + 1 + 3 * 8))
 
 struct ActParams {
   cur_net_desc d;
@@ -2084,7 +2084,11 @@ static int act_common(PT& P, const cur_net_desc* d, const float* theta, const fl
     for (int l = 1; l < L; ++l) rows_of(th + NL.off_W[l], H, 0);
     return first;
   };
-  CUR_REQUIRE((out_q ? 2 : 1) * (4 + (L - 1) * (H / CK)) <= A_MAXCHUNK, "too many weight chunks");
+  // the chunks forward_net appends: the state and goal blocks of the first layer, then the hidden layers
+  auto net_chunks = [&](const NetLayout& NL) {
+    return (NL.in_s + CK - 1) / CK + (NL.in_g + CK - 1) / CK + (L - 1) * ((H + CK - 1) / CK);
+  };
+  CUR_REQUIRE(net_chunks(LP) + (out_q ? net_chunks(LQ) : 0) <= A_MAXCHUNK, "too many weight chunks");
   P.ch0[0] = forward_net(thP, LP);
   P.ch0[1] = out_q != nullptr ? forward_net(thQ, LQ) : 0;
   P.nchunks = nc;
