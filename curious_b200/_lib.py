@@ -192,6 +192,7 @@ SIGNATURES = {
                                  C.POINTER(NormStats), C.POINTER(Batch), C.POINTER(DdpgHyper), C.c_void_p,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     'cur_ddpg_rows_supported': (C.c_int, [C.POINTER(NetDesc), C.c_int64]),
+    'cur_ddpg_rows_her_supported': (C.c_int, [C.POINTER(NetDesc), C.POINTER(HerArgs)]),
     'cur_ddpg_rows_workspace_floats': (C.c_int64, [C.POINTER(NetDesc), C.c_int64]),
     'cur_ddpg_rows_step': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_void_p, C.c_void_p,
                                      C.POINTER(NormStats), C.POINTER(Batch), C.POINTER(DdpgHyper), C.c_void_p,

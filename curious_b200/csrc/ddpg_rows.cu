@@ -1757,6 +1757,33 @@ extern "C" int cur_ddpg_rows_owner_map(const cur_net_desc* d, int64_t batch, int
 
 extern "C" int cur_ddpg_rows_supported(const cur_net_desc* d, int64_t batch) { return rows_supported(d, batch) ? 1 : 0; }
 
+// What cur_ddpg_rows_step requires of `her` for a batch of n rows (host only, no CUDA call): the batch, the layout against
+// the nets, relative goals, and the staged image of a transition against the 4-row HER stage of the update kernel (the
+// image holds ag(t+1), the future achieved goal and, for relative goals or an INFO reward, the cold row - none of which
+// the net's fan-in bounds).  Fills the prologue's copy of the args and its plan.
+static int fused_her_plan(const cur_net_desc* d, const cur_her_args* her, int64_t n, cur_her_args* a, HerPlan* plan) {
+  CUR_REQUIRE(her->batch == n, "HER args must describe exactly this batch");
+  CUR_REQUIRE(her->L.dimo == d->dimo && her->L.dimg == d->dimg && her->L.dimu == d->dimu &&
+              her->L.dimtd == (d->modular ? d->dimtd : her->L.dimtd), "HER layout does not match the networks");
+  CUR_REQUIRE(!her->relative_goals || her->L.dimag == her->L.dimg, "relative goals need dimg == dimag");
+  *a = *her;
+  a->change = nullptr; a->info = nullptr;                // cold rows travel only for an INFO reward (make_plan)
+  a->ag = nullptr;                                       // (ag_t is staged iff relative_goals)
+  make_plan(*a, plan);
+  CUR_REQUIRE(S_ROWS * plan->stage_stride <= S_MISC - S_STAGE_OFF, "transition too wide for the fused HER stage");
+  if (plan->cold4 > 0)
+    for (int i = 0; i < her->n_segments; ++i)
+      CUR_REQUIRE(her->seg[i].cold != nullptr, "an INFO reward needs the cold rows of every segment");
+  return CUR_OK;
+}
+
+extern "C" int cur_ddpg_rows_her_supported(const cur_net_desc* d, const cur_her_args* her) {
+  if (her == nullptr || !rows_supported(d, her->batch)) return 0;
+  cur_her_args a;
+  HerPlan plan;
+  return fused_her_plan(d, her, her->batch, &a, &plan) == CUR_OK ? 1 : 0;
+}
+
 extern "C" int64_t cur_ddpg_rows_workspace_floats(const cur_net_desc* d, int64_t batch) {
   if (!rows_supported(d, batch)) return -1;
   return carve_rows(*d, batch, nullptr).total;
@@ -1826,18 +1853,7 @@ extern "C" int cur_ddpg_rows_step(void* stream, const cur_net_desc* d, float* th
   P.loss_part = w.loss_part; P.q_pi = q_pi;
   if (her != nullptr) {
     // fused sampling: the rows of the batch are drawn, gathered and relabelled in the kernel's prologue
-    CUR_REQUIRE(her->batch == n, "HER args must describe exactly this batch");
-    CUR_REQUIRE(her->L.dimo == d->dimo && her->L.dimg == d->dimg && her->L.dimu == d->dimu &&
-                her->L.dimtd == (d->modular ? d->dimtd : her->L.dimtd), "HER layout does not match the networks");
-    CUR_REQUIRE(!her->relative_goals || her->L.dimag == her->L.dimg, "relative goals need dimg == dimag");
-    P.her = *her;
-    P.her.change = nullptr; P.her.info = nullptr;         // cold rows travel only for an INFO reward (make_plan)
-    P.her.ag = nullptr;                                    // (ag_t is staged iff relative_goals)
-    make_plan(P.her, &P.plan);
-    CUR_REQUIRE(S_ROWS * P.plan.stage_stride <= S_MISC - S_STAGE_OFF, "transition too wide for the fused HER stage");
-    if (P.plan.cold4 > 0)
-      for (int i = 0; i < her->n_segments; ++i)
-        CUR_REQUIRE(her->seg[i].cold != nullptr, "an INFO reward needs the cold rows of every segment");
+    CUR_TRY(fused_her_plan(d, her, n, &P.her, &P.plan));
     P.fused_her = 1;
   }
 

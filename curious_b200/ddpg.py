@@ -1091,15 +1091,12 @@ class DDPG(object):
             # the workers' batches: one standalone sampler launch (not fused into the rows prologue)
             self._sample_workers(self._gwant, rng='philox', out=self._gbatch, dyn=self._wdyn_dev.data_ptr(),
                                  step=self._step.data_ptr(), call_offset=self.GRAPH_STREAM_OFFSET)
-        elif self._use_rows(self._graph_rows) and self.fuse_her:
-            # rows schedule: every CTA of the update kernel samples its own rows (no separate HER launch)
-            her_args, self._her_keep = sampler.sample_device(
-                segs, self._graph_rows, clip_obs=self.clip_obs, relative_goals=self.relative_goals, want=(),
-                dyn=self._dyn_dev.data_ptr(), call_offset=self.GRAPH_STREAM_OFFSET, args_only=True)
         else:
-            sampler.sample_device(segs, self._graph_rows, clip_obs=self.clip_obs, relative_goals=self.relative_goals,
-                                  want=self._gwant, out=self._gbatch, dyn=self._dyn_dev.data_ptr(),
-                                  call_offset=self.GRAPH_STREAM_OFFSET)
+            her_args = self._fused_her_args(segs)
+            if her_args is None:
+                sampler.sample_device(segs, self._graph_rows, clip_obs=self.clip_obs,
+                                      relative_goals=self.relative_goals, want=self._gwant, out=self._gbatch,
+                                      dyn=self._dyn_dev.data_ptr(), call_offset=self.GRAPH_STREAM_OFFSET)
         b = self._gbatch
         n = self._graph_rows
         g2 = b['g_2'] if self.relative_goals else b['g']       # g_2 == g without relative goals (ddpg.py:353)
@@ -1149,6 +1146,20 @@ class DDPG(object):
             self.grads.data_ptr(), self._q_ring.data_ptr(), self._pi_ring.data_ptr(), self._q_pi.data_ptr()),
             'cur_ddpg_grads')
         return False
+
+    def _fused_her_args(self, segs):
+        """The sampler's cur_her_args for the rows update kernel to sample its own rows in its prologue (no separate HER
+        launch), or None: the rows schedule does not run, fusing is off, or a transition does not fit that kernel's HER
+        stage (cur_ddpg_rows_her_supported) - the batch is then sampled into _gbatch by the standalone kernel."""
+        if not (self._use_rows(self._graph_rows) and self.fuse_her):
+            return None
+        her_args, keep = self.sample_transitions.sample_device(
+            segs, self._graph_rows, clip_obs=self.clip_obs, relative_goals=self.relative_goals, want=(),
+            dyn=self._dyn_dev.data_ptr(), call_offset=self.GRAPH_STREAM_OFFSET, args_only=True)
+        if not _lib.load().cur_ddpg_rows_her_supported(C.byref(self.net.desc), C.byref(her_args)):
+            return None
+        self._her_keep = keep
+        return her_args
 
     def _launch_adam(self, warmup=False):
         """Adam on the (already all-reduced) gradient arena; the step scale is read from the device table with

@@ -91,7 +91,7 @@ typedef struct cur_episode_src {
 
 int cur_store_episodes(void* stream, const cur_layout* L, const cur_episode_src* src, int n_ep,
                        int n_copies, const int32_t* copy_src, float* const* copy_hot,
-                       float* const* copy_cold /* entries may be NULL when cold_stride == 0 */,
+                       float* const* copy_cold /* required, no NULL entries: every layout has cold rows (ag(t)) */,
                        const int64_t* copy_slot);
 
 /* ------------------------------------------------------------------------------------------
@@ -441,7 +441,7 @@ int cur_ddpg_grads_group(void* stream, const cur_net_desc* d, int n_experts, con
  * With `her` != NULL the batch is not read from `batch` (only batch->n is used): every CTA draws,
  * gathers and relabels its own rows in the kernel prologue with the code of cur_her_sample (same
  * Philox counters / injected draws / control block, bit-identical transitions); output pointers
- * inside `her` are ignored.
+ * inside `her` are ignored.  Which `her` it takes: cur_ddpg_rows_her_supported.
  * ------------------------------------------------------------------------------------------ */
 /* Tile-level gradient exchange INSIDE the weight-gradient launch (csrc/ddpg_rows.cu, several ranks; replaces the
  * Allreduce(SUM) of mpi_adam.py:24-28 between _grads and _update, scale_grad_by_procs=False).  Every rank runs the same
@@ -495,6 +495,12 @@ typedef struct cur_adam_fused {
 } cur_adam_fused;
 
 int cur_ddpg_rows_supported(const cur_net_desc* d, int64_t batch);
+/* 1 exactly when cur_ddpg_rows_step takes `her` (fused sampling) for this net: cur_ddpg_rows_supported(d, her->batch), a
+ * layout whose dims match the net, dimag == dimg for relative goals, cold rows in every segment when the stage needs
+ * them, and a transition image (transition row, future achieved goal, and the cold row for relative goals or an INFO
+ * reward) that fits the update kernel's 4-row HER stage.  A wider transition has to be sampled by cur_her_sample into
+ * `batch`.  Host only: no CUDA call. */
+int cur_ddpg_rows_her_supported(const cur_net_desc* d, const cur_her_args* her);
 /* (Re)build the transposed hidden-layer weights of main.Q / main.pi in a rows-schedule workspace (see
  * cur_adam_fused.transposes_valid). */
 int cur_ddpg_rows_refresh(void* stream, const cur_net_desc* d, const float* theta_main, float* workspace,

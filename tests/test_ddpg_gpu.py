@@ -552,6 +552,38 @@ def test_cuda_graph_path_equals_eager_path(task_replay, schedule):
     assert np.array_equal(g.get_flat('Q', True), e.get_flat('Q', True))
 
 
+@pytest.mark.parametrize('n_modules,dimo,fused', [(8, 220, False), (4, 204, False), (4, 200, True)])
+def test_graph_path_when_a_transition_does_not_fit_the_fused_stage(n_modules, dimo, fused):
+    """Default options (Philox draws, CUDA graph, rows schedule at batch 256).  Arm8 at dimo 220 (Q fan-in exactly 256)
+    and Arm4 at dimo 204 are nets the rows kernel takes whose transitions do not fit its 4-row HER stage: the graph
+    samples them with the standalone kernel.  Arm4 at dimo 200 is the widest that fits and samples in the prologue.
+    Either way the graph path equals the launch-by-launch path bit for bit."""
+    import torch
+    from curious_b200.ddpg import DDPG
+    kw, dims, ag_ids, g_ids = ddpg_kwargs(n_modules, dimo=dimo)
+    episodes = episode_stream(dims, kw['T'], 6)
+    cp = np.resize([0.05, 0.2, 0.1, 0.0], n_modules)
+    agents = []
+    for use_graph in (True, False):
+        ag = make_gpu_agent(kw, dims, ag_ids, g_ids, her_rng='philox', use_cuda_graph=use_graph)
+        np.random.seed(4)
+        _fill(ag, episodes, cp)
+        agents.append(ag)
+    g, e = agents
+    e.sample_transitions.calls = DDPG.GRAPH_STREAM_OFFSET
+    for step in range(5):
+        lg, qg = g.train()
+        le, qe = e.train()
+        assert float(lg) == float(le), step
+        assert np.array_equal(np.asarray(qg), np.asarray(qe)), step
+    for which in ('Q', 'pi'):
+        assert np.array_equal(g.get_flat(which), e.get_flat(which)), which
+    for adam in ('Q_adam', 'pi_adam'):
+        assert torch.equal(getattr(g, adam).m, getattr(e, adam).m) and torch.equal(getattr(g, adam).v, getattr(e, adam).v)
+    segs = [(buf.device_view(), 0, ttr) for buf, ttr in g._all_segments()]
+    assert (g._fused_her_args(segs) is not None) == fused
+
+
 @pytest.mark.parametrize('batch_size', [512, 1024, 1280, 2560, 4096, 4864])
 def test_large_batch_tensor_core_update_against_oracle(batch_size):
     """BASELINE configs 4 / 5 (19 workers x 256 = 4864 rows; batch sweep): at large batch the update runs on tcgen05
