@@ -95,6 +95,13 @@ class ActionsExpert(C.Structure):
     _fields_ = [('theta', C.c_void_p), ('stats', NormStats)]
 
 
+class NoiseRow(C.Structure):
+    _fields_ = [('seed', C.c_uint64), ('call', C.c_uint64), ('ctr', C.c_uint32), ('noisy', C.c_uint32)]
+
+
+CUR_ACTIONS_NOISY_MAX_ROWS = 512
+
+
 class Batch(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ('o', 'g', 'u', 'td', 'o_2', 'g_2', 'r')] + [('n', C.c_int64)]
 
@@ -170,6 +177,9 @@ SIGNATURES = {
     'cur_ddpg_actions_rows': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_void_p, C.POINTER(NormStats), C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_void_p,
                                         C.c_uint32]),
+    'cur_ddpg_actions_rows_noisy': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_void_p, C.POINTER(NormStats),
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
+                                              C.c_double, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]),
     'cur_ddpg_actions_rows_group': (C.c_int, [C.c_void_p, C.POINTER(NetDesc), C.c_int, C.POINTER(ActionsExpert),
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                               C.c_float, C.c_void_p, C.c_void_p, C.c_uint32]),

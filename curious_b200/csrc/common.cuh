@@ -72,6 +72,45 @@ __host__ __device__ inline double u01_from_u32(uint32_t x) {
   return ((double)x + 0.5) * (1.0 / 4294967296.0);
 }
 
+// ---------------------------------------------------------------- exploration noise (device-side option)
+// ddpg.py:147-152 on the action matrix u [n, dimu] in place, with counter-based draws instead of the host's MT19937:
+//   u += noise_eps * max_u * randn(*u.shape); u = clip(u, -max_u, max_u)
+//   u += binomial(1, random_eps, n)[:, None] * (uniform(-max_u, max_u, (n, dimu)) - u)
+// Per (row, pair of action components): x = philox(counter = (row, pair, call_lo, call_hi ^ TAG), key = seed):
+// (x0, x1) -> one Box-Muller pair, (x2, x3) -> the two uniform random-action components; the row's eps-greedy draw
+// comes from the block with pair = 0xFFFFFFFF.  Arithmetic in float64 like NumPy's (the float32 action array is updated
+// in place by float64 operands), rounded to float32 where the reference's `+=` rounds.  Used by cur_action_noise(_rows)
+// and by the noise epilogue of the action kernel (cur_ddpg_actions_rows_noisy), which must give the same bits.
+constexpr uint32_t ACTION_NOISE_TAG = 0x40000000u;
+
+// components 2p, 2p + 1 of row r of u; `ctr` is the row's counter word (its row number in the call)
+__device__ __forceinline__ void action_noise_pair(float* __restrict__ u, int64_t r, uint32_t ctr, int p, int dimu,
+                                                  float max_u, double noise_eps, double random_eps, uint64_t seed,
+                                                  uint64_t call) {
+  const uint32_t c2 = (uint32_t)call, c3 = (uint32_t)(call >> 32) ^ ACTION_NOISE_TAG;
+  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+  const Philox x = philox4x32_10(ctr, (uint32_t)p, c2, c3, k0, k1);
+  const Philox b = philox4x32_10(ctr, 0xFFFFFFFFu, c2, c3, k0, k1);
+  const bool explore = u01_from_u32(b.x[0]) < random_eps;                       // binomial(1, random_eps)
+  const double rad = sqrt(-2.0 * log(u01_from_u32(x.x[0])));
+  const double ang = 6.283185307179586 * u01_from_u32(x.x[1]);
+  const double z[2] = {__dmul_rn(rad, cos(ang)), __dmul_rn(rad, sin(ang))};
+  const double mu = (double)max_u;
+#pragma unroll
+  for (int e = 0; e < 2; ++e) {
+    const int k = 2 * p + e;
+    if (k >= dimu) break;
+    float v = u[r * dimu + k];
+    v = (float)__dadd_rn((double)v, __dmul_rn(noise_eps * mu, z[e]));           // ddpg.py:148-149 (no fma contraction)
+    v = fminf(fmaxf(v, -max_u), max_u);                                         // ddpg.py:150
+    if (explore) {
+      const double ra = __dadd_rn(-mu, __dmul_rn(mu - (-mu), u01_from_u32(x.x[2 + e])));   // _random_action, ddpg.py:114-116
+      v = (float)__dadd_rn((double)v, __dsub_rn(ra, (double)v));                // ddpg.py:151
+    }
+    u[r * dimu + k] = v;
+  }
+}
+
 // Adam on one element: unfused IEEE float32 operations in NumPy's order (mpi_adam.py:32-35)
 __device__ __forceinline__ void adam_elem(float& th, float g, float& m, float& v, float neg_a, float b1,
                                           float omb1, float b2, float omb2, float eps) {

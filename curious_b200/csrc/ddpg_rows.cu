@@ -35,6 +35,8 @@
 // The stream and action kernels are instantiated for hidden 64, 128 and 256 (Width<H>); the numbers above are for 256.
 #include <stdlib.h>
 
+#include <type_traits>
+
 #include "her_device.cuh"
 #include "net_layout.cuh"
 #include "tc_gemm.cuh"
@@ -777,6 +779,13 @@ __device__ __forceinline__ float act_x_elem(const PT& P, const float* o_mean, co
   return v;
 }
 
+// cur_ddpg_actions_rows_noisy: the device-side exploration noise as an epilogue of the pi output, row by row with the
+// row's own key / call / counter row (cur_noise_row)
+struct ActNoiseParams : ActParams {
+  double noise_eps, random_eps;
+  const cur_noise_row* rows;   // [n]
+};
+
 // an output element: plain float32, or - seq != 0 - one naturally aligned 8-byte word {value | seq << 32}: a 64-bit
 // store is single-copy atomic (also across PCIe), so the host polls the data words themselves and the kernel needs
 // neither a system fence nor a completion ticket
@@ -785,9 +794,12 @@ __device__ __forceinline__ void put_out(void* base, int64_t i, float v, uint32_t
   else st_ll(reinterpret_cast<unsigned long long*>(base) + i, v, seq);
 }
 
-template <int H>
+// PT = ActParams: the plain launch; PT = ActNoiseParams: with the noise epilogue (one kernel body, so the noise-free
+// instantiations compile as before)
+template <int H, class PT>
 __global__ void __launch_bounds__(S_THREADS, 1)
-actions_stream_kernel(const __grid_constant__ ActParams P) {
+actions_stream_kernel(const __grid_constant__ PT P) {
+  constexpr bool kNoise = std::is_same<PT, ActNoiseParams>::value;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float* ringf = reinterpret_cast<float*>(smem_raw);
   float* xa = ringf + S_NSLOT * S_SLOT;
@@ -797,6 +809,8 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
   uint64_t* bars = reinterpret_cast<uint64_t*>(misc + S_MISC);
   float* s_th = misc;                 // [4][8] tanh output
   float* s_q = misc + 64;             // [4][8]
+  float* s_u = misc + 128;            // [4][8] noisy actions (kNoise)
+  cur_noise_row* s_rows = reinterpret_cast<cur_noise_row*>(misc + 160);   // [4] (kNoise)
   const int tid = threadIdx.x;
   const int64_t row0 = (int64_t)blockIdx.x * S_ROWS;
   const cur_net_desc& d = P.d;
@@ -830,6 +844,9 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
     if (P.tl != nullptr && tid == 0 && blockIdx.x == 0) P.tl[i] = (long long)globaltimer_ns(); \
   } while (0)
   A_TL(0);
+  if constexpr (kNoise) {
+    if (tid < nr) s_rows[tid] = P.rows[row0 + tid];     // (read early: the table may sit in host memory)
+  }
   auto build = [&](int act_kind) {
     for (int idx = tid; idx < S_ROWS * P.KP; idx += S_CONSUMERS) {
       const int k = idx >> 2, r = idx & 3;
@@ -848,9 +865,25 @@ actions_stream_kernel(const __grid_constant__ ActParams P) {
     const float th = tanhf(s_th[tid]);                                  // actor_critic.py:89
     s_th[tid] = th;
     const int r = tid >> 3, j = tid & (S_DU - 1);
-    if (r < nr) put_out(P.pi, (row0 + r) * d.dimu + j, d.max_u * th, P.seq);
+    if constexpr (kNoise) s_u[tid] = d.max_u * th;
+    else if (r < nr) put_out(P.pi, (row0 + r) * d.dimu + j, d.max_u * th, P.seq);
   }
   consumer_sync();
+  if constexpr (kNoise) {
+    // the noise of cur_action_noise on the row's action (the float32 the plain launch writes), keyed per row
+    const int pairs = (d.dimu + 1) / 2;
+    if (tid < S_ROWS * pairs) {
+      const int r = tid / pairs, p = tid - r * pairs;
+      if (r < nr && s_rows[r].noisy)
+        action_noise_pair(s_u + r * S_DU, 0, s_rows[r].ctr, p, d.dimu, d.max_u, P.noise_eps, P.random_eps, s_rows[r].seed,
+                          s_rows[r].call);
+    }
+    consumer_sync();
+    if (tid < S_ROWS * S_DU && (tid & (S_DU - 1)) < d.dimu) {
+      const int r = tid >> 3, j = tid & (S_DU - 1);
+      if (r < nr) put_out(P.pi, (row0 + r) * d.dimu + j, s_u[tid], P.seq);
+    }
+  }
   if (P.q != nullptr) {
     build(2);                                                          // Q(o, g, pi / max_u): the noise-free action
     consumer_sync();
@@ -1670,7 +1703,9 @@ static int launch_stream(unsigned grid, cudaStream_t s, const StreamParams& P) {
 }
 
 template <int H>
-static auto act_kernel(const ActParams*) { return actions_stream_kernel<H>; }
+static auto act_kernel(const ActParams*) { return actions_stream_kernel<H, ActParams>; }
+template <int H>
+static auto act_kernel(const ActNoiseParams*) { return actions_stream_kernel<H, ActNoiseParams>; }
 template <int H>
 static auto act_kernel(const ActGroupParams*) { return actions_group_kernel<H>; }
 
@@ -2113,24 +2148,33 @@ static int act_common(PT& P, const cur_net_desc* d, const float* theta, const fl
 
 // One launch for DDPG.get_actions (see actions_stream_kernel).  o / ag / g / td / out_pi / out_q may be device
 // pointers of mapped pinned host memory.  seq != 0: the outputs are 8-byte words {float32 bits | seq << 32}.
-extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
-                                     const float* o, const float* ag, const float* g, const float* td, int64_t n,
-                                     float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
+// The checks and the ActParams of one cur_ddpg_actions_rows launch over n rows (n <= max_rows)
+static int act_params(ActParams& P, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
+                      const float* o, const float* ag, const float* g, const float* td, int64_t n, int64_t max_rows,
+                      float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
   CUR_TRY(check_desc(d));
   CUR_REQUIRE(theta && o && g && out_pi, "NULL argument");
   CUR_REQUIRE(!d->modular || td, "task_descr required for a modular net");
-  CUR_REQUIRE(n > 0 && n <= 4096, "bad row count (the one-launch action path covers up to 4096 rows)");
+  CUR_REQUIRE(n > 0 && n <= max_rows, "bad row count (beyond the rows the one-launch action path covers)");
   CUR_REQUIRE(rows_supported(d, S_ROWS), "shape not supported by the rows schedule (see cur_ddpg_rows_supported)");
   if (d->normalize_obs)
     CUR_REQUIRE(stats && stats->o_mean && stats->o_std && stats->g_mean && stats->g_std, "normalizer stats required");
-  const int H = d->hidden;
-  static const bool tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
-  ActParams P;
   CUR_TRY(act_common(P, d, theta, o, ag, g, td, clip_obs, out_pi, out_q, seq));
   P.n = n;
   P.o_mean = P.o_std = P.g_mean = P.g_std = nullptr;
   if (stats) { P.o_mean = stats->o_mean; P.o_std = stats->o_std; P.g_mean = stats->g_mean; P.g_std = stats->g_std; }
   act_net_ptrs(P, *d, theta);
+  P.tl = nullptr;
+  return CUR_OK;
+}
+
+extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
+                                     const float* o, const float* ag, const float* g, const float* td, int64_t n,
+                                     float clip_obs, void* out_pi, void* out_q, uint32_t seq) {
+  ActParams P;
+  CUR_TRY(act_params(P, d, theta, stats, o, ag, g, td, n, 4096, clip_obs, out_pi, out_q, seq));
+  const int H = d->hidden;
+  static const bool tl_on = getenv("CUR_ACTIONS_TIMELINE") != nullptr;
   static long long* tl_dev = nullptr;
   static int tl_calls = 0;
   if (tl_on && tl_dev == nullptr) {
@@ -2150,6 +2194,34 @@ extern "C" int cur_ddpg_actions_rows(void* stream, const cur_net_desc* d, const 
     fprintf(stderr, "[actions timeline] inputs %lld | pi forward %lld | outputs (+ Q) %lld | total %lld ns\n", t[1] - t[0],
             t[2] - t[1], t[3] - t[2], t[3] - t[0]);
   }
+  return CUR_OK;
+}
+
+// cur_ddpg_actions_rows + cur_action_noise with per-row keys in one launch (the kNoise epilogue of actions_stream_kernel)
+extern "C" int cur_ddpg_actions_rows_noisy(void* stream, const cur_net_desc* d, const float* theta,
+                                           const cur_norm_stats* stats, const float* o, const float* ag, const float* g,
+                                           const float* td, int64_t n, float clip_obs, double noise_eps,
+                                           double random_eps, const cur_noise_row* rows, void* out_pi, void* out_q,
+                                           uint32_t seq) {
+  ActNoiseParams P;
+  CUR_TRY(act_params(P, d, theta, stats, o, ag, g, td, n, CUR_ACTIONS_NOISY_MAX_ROWS, clip_obs, out_pi, out_q, seq));
+  CUR_REQUIRE(d->dimu <= CUR_ACTIONS_MAX_DIMU && CUR_ACTIONS_MAX_DIMU <= S_DU, "dimu above the action kernel's bound");
+  CUR_REQUIRE(noise_eps >= 0.0 && random_eps >= 0.0 && random_eps <= 1.0, "bad noise parameters");
+  CUR_REQUIRE(rows != nullptr, "NULL argument");
+  const unsigned blocks = (unsigned)((n + S_ROWS - 1) / S_ROWS);
+  const int H = d->hidden;
+  if (noise_eps == 0.0 && random_eps == 0.0) {             // what a caller does without noise: the plain launch
+    const ActParams& A = P;
+    if (H == 64) CUR_TRY(launch_actions<64>(blocks, (cudaStream_t)stream, A));
+    else if (H == 128) CUR_TRY(launch_actions<128>(blocks, (cudaStream_t)stream, A));
+    else CUR_TRY(launch_actions<256>(blocks, (cudaStream_t)stream, A));
+  } else {
+    P.noise_eps = noise_eps; P.random_eps = random_eps; P.rows = rows;
+    if (H == 64) CUR_TRY(launch_actions<64>(blocks, (cudaStream_t)stream, P));
+    else if (H == 128) CUR_TRY(launch_actions<128>(blocks, (cudaStream_t)stream, P));
+    else CUR_TRY(launch_actions<256>(blocks, (cudaStream_t)stream, P));
+  }
+  CUR_CHECK_LAUNCH();
   return CUR_OK;
 }
 

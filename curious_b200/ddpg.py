@@ -552,6 +552,113 @@ class DDPG(object):
             self._action_calls += 1
         return self._finish_actions(out.cpu().numpy(), n, compute_Q, device_noise, noise_eps, random_eps)
 
+    def get_actions_workers(self, o, ag, g, task_descr=None, noise_eps=(), random_eps=(), streams=None,
+                            use_target_net=False, compute_Q=False):
+        """get_actions for the k reference workers this rank hosts, as ONE action launch over their k * B rows: rows
+        [j * B, (j + 1) * B) are worker j's, acting with noise_eps[j] / random_eps[j] (0 for a worker that exploits).
+        Worker j's exploration noise is what a lone agent of its reference rank gets (ddpg.py:147-152): host noise drawn
+        from streams.rng(j) in reference order (randn, binomial, uniform; also when its eps are 0), taken while the
+        launch is in flight; device noise (action_noise='device') keyed by streams.philox_key(j) at counter rows 0..B-1
+        and this agent's call number, applied inside the launch (cur_ddpg_actions_rows_noisy).  Up to
+        ACTION_ZERO_COPY_MAX rows zero-copy, up to ACTION_ROWS_MAX through device memory; anything the one-launch
+        action kernel does not take raises ValueError.  Returns (u [k * B, dimu] float32, q [k * B, 1] or None)."""
+        k = len(noise_eps)
+        o = np.asarray(o, np.float32).reshape(-1, self.dimo)
+        g = np.asarray(g, np.float32).reshape(-1, self.dimg)
+        n = o.shape[0]
+        if k == 0 or len(random_eps) != k or streams is None or len(streams) != k or n % k:
+            raise ValueError('get_actions_workers takes k * B rows, k noise_eps / random_eps and the k workers\' streams')
+        if n > self.ACTION_ROWS_MAX or not self._action_rows_ok():
+            raise ValueError('get_actions_workers runs the one-launch action kernel (up to %d rows of a shape '
+                             'cur_ddpg_rows_supported takes)' % self.ACTION_ROWS_MAX)
+        B = n // k
+        device_noise = self.action_noise == 'device'
+        noisy = [float(ne) != 0. or float(re) != 0. for ne, re in zip(noise_eps, random_eps)]
+        eps = {(float(ne), float(re)) for ne, re, on in zip(noise_eps, random_eps, noisy) if on}
+        if device_noise and len(eps) > 1:
+            raise ValueError('device noise: the workers that explore share one noise_eps / random_eps')
+        lib = _lib.load()
+        slot = self._action_slot(n)
+        np.copyto(slot['o'], o.reshape(-1))
+        np.copyto(slot['g'], g.reshape(-1))
+        if self.relative_goals:
+            np.copyto(slot['ag'], np.asarray(ag, np.float32).reshape(-1))
+        if self.modular:
+            np.copyto(slot['td'], np.asarray(task_descr, np.float32).reshape(-1))
+        zero_copy = n <= self.ACTION_ZERO_COPY_MAX
+        if zero_copy:
+            slot['seq'] = seq = slot['seq'] % 0xFFFFFFF0 + 1
+            base, out_pi, out_q = slot['d_o'], slot['d_out'], slot['d_q'] if compute_Q else None
+        else:
+            # above a few dozen rows: inputs and float32 outputs through device memory (as get_actions does)
+            seq, out = 0, torch.empty(n * (self.dimu + 1), dtype=torch.float32, device=self.device)
+            if 'dev_in' not in slot:
+                slot['n_in'] = (slot['d_out'] - slot['d_o']) // 4
+                slot['dev_in'] = torch.empty(slot['n_in'], dtype=torch.float32, device=self.device)
+            _lib.check(lib.cur_copy_h2d(_lib.stream_ptr(), slot['dev_in'].data_ptr(), slot['d_o'], 4 * slot['n_in']),
+                       'cur_copy_h2d')
+            base = slot['dev_in'].data_ptr()
+            out_pi, out_q = out.data_ptr(), out.data_ptr() + 4 * n * self.dimu if compute_Q else None
+        rel = lambda name: base + (slot[name] - slot['d_o'])
+        theta = self.theta_target if use_target_net else self.theta_main
+        args = (_lib.stream_ptr(), C.byref(self.net.desc), theta.data_ptr(), C.byref(self._stats), base,
+                rel('d_ag') if self.relative_goals else None, rel('d_g'), rel('d_td') if self.modular else None, n,
+                float(self.clip_obs))
+        if device_noise and eps:
+            rows = self._noise_rows(slot, n)
+            rows['seed'] = np.repeat(np.array([streams.philox_key(j) for j in range(k)], np.uint64), B)
+            rows['call'] = self._action_calls
+            rows['ctr'] = np.tile(np.arange(B, dtype=np.uint32), k)
+            rows['noisy'] = np.repeat(np.array(noisy, np.uint32), B)
+            ne, re = eps.pop()
+            _lib.check(lib.cur_ddpg_actions_rows_noisy(*args, ne, re, slot['d_noise_rows'], out_pi, out_q, seq),
+                       'cur_ddpg_actions_rows_noisy')
+        else:
+            _lib.check(lib.cur_ddpg_actions_rows(*args, out_pi, out_q, seq), 'cur_ddpg_actions_rows')
+        if device_noise:
+            self._action_calls += 1
+        else:
+            # every worker's draws from its own stream, in reference order, while the launch is in flight; the noise is
+            # scaled here (noise_eps * max_u * randn, ddpg.py:148) because the workers' scales differ
+            randn, explore, u_rand = slot['randn'], slot['explore'], slot['u_rand']
+            for j in range(k):
+                rng, s = streams.rng(j), slice(j * B, (j + 1) * B)
+                np.multiply(float(noise_eps[j]) * self.max_u, rng.randn(B, self.dimu), out=randn[s])
+                explore[s] = rng.binomial(1, random_eps[j], B)
+                u_rand[s] = rng.uniform(low=-self.max_u, high=self.max_u, size=(B, self.dimu))
+        if not zero_copy:
+            res = out[:n * (self.dimu + (1 if compute_Q else 0))].cpu().numpy()
+            u = res[:n * self.dimu].reshape(n, self.dimu)
+            if not device_noise:
+                u += slot['randn']                                                          # ddpg.py:148-149
+                np.minimum(np.maximum(u, -self.max_u, out=u), self.max_u, out=u)            # ddpg.py:150
+                u += slot['explore'].reshape(-1, 1) * (slot['u_rand'] - u)                  # ddpg.py:151
+            return u.copy(), (res[n * self.dimu:].reshape(n, 1).copy() if compute_Q else None)
+        draws = (None,) * 3 if device_noise else (slot['p_randn'], slot['p_explore'], slot['p_u_rand'])
+        finish = (slot['h_out'], n, self.dimu, 1 if compute_Q else 0, seq, *draws, 1.0, float(self.max_u), slot['p_fin'],
+                  slot['p_fin_q'] if compute_Q else None, 20000000)
+        status = lib.cur_actions_finish_host(*finish)
+        if status == 3:                     # no answer: let a launch failure surface, then give up
+            torch.cuda.current_stream().synchronize()
+            status = lib.cur_actions_finish_host(*finish)
+            if status == 3:
+                raise RuntimeError('the action launch did not complete')
+        _lib.check(status, 'cur_actions_finish_host')
+        return slot['fin_u'].copy(), (slot['fin_q'].copy() if compute_Q else None)
+
+    def _noise_rows(self, slot, n):
+        """The per-row {seed, call, ctr, noisy} table of cur_ddpg_actions_rows_noisy, in mapped pinned memory of the slot."""
+        if 'noise_rows' not in slot:
+            hp, dp = C.c_void_p(), C.c_void_p()
+            size = C.sizeof(_lib.NoiseRow)
+            _lib.check(_lib.load().cur_host_alloc(size * n, C.byref(hp), C.byref(dp)), 'cur_host_alloc')
+            dt = np.dtype({'names': ['seed', 'call', 'ctr', 'noisy'], 'formats': ['<u8', '<u8', '<u4', '<u4'],
+                           'offsets': [_lib.NoiseRow.seed.offset, _lib.NoiseRow.call.offset, _lib.NoiseRow.ctr.offset,
+                                       _lib.NoiseRow.noisy.offset], 'itemsize': size})
+            slot['noise_rows'] = np.ctypeslib.as_array((C.c_uint8 * (size * n)).from_address(hp.value)).view(dt)
+            slot['d_noise_rows'] = dp.value
+        return slot['noise_rows']
+
     def _action_rows_ok(self):
         if self._action_rows is None:
             self._action_rows = bool(self.action_path != 'levels' and self._rows_shape_ok(4))

@@ -22,7 +22,7 @@ from .ddpg import DDPG
 from .envs import ModularPointEnv
 from .replay_buffer import ReplayBuffer
 from .rollout import RolloutWorker
-from .parallel import assert_rank_streams_differ, bcast_object, rank as _rank, rank_seed
+from .parallel import assert_rank_streams_differ, bcast_object, rank as _rank, rank_seed, world as _world
 from .runlog import RunLog, mpi_average
 
 MULTI_TASK_PARAMS = {            # config.py:56-90
@@ -71,9 +71,16 @@ def configure_buffer(dims, T, sampler, buffer_size, structure, task_replay, nb_t
 
 def make_experiment(nb_tasks=4, n_controllable=None, structure='curious', task_selection='active_competence_progress',
                     goal_replay='her', task_replay='replay_task_cp_buffer', seed=0, device=None, normalize_obs=False,
-                    make_env=None, policy_kwargs=None, **overrides):
+                    make_env=None, policy_kwargs=None, workers_per_rank=1, **overrides):
     """config.prepare_params + configure_* + the RolloutWorker pair of train.py:268-337.  Returns the keyword
-    arguments of train()."""
+    arguments of train().  workers_per_rank=k > 1: the rank hosts k reference workers (worker j = reference rank j, one
+    rank only): DDPG(workers_per_rank=k, worker_buffers='own') with k-worker exploration and evaluation RolloutWorkers on
+    the policy's worker streams; the run parameters record num_cpu = k."""
+    if workers_per_rank != 1:
+        if structure == 'task_experts':
+            raise ValueError("workers_per_rank > 1 does not take structure='task_experts'")
+        if _world((policy_kwargs or {}).get('comm'))[1] > 1:
+            raise ValueError('workers_per_rank > 1 runs on one rank')
     params = dict(FLAT_PARAMS if structure == 'flat' else MULTI_TASK_PARAMS)
     params.update(overrides)
     # train.py:241-243: every rank seeds everything with rank_seed = seed + 1000000 * rank (set_global_seeds: np.random
@@ -110,6 +117,8 @@ def make_experiment(nb_tasks=4, n_controllable=None, structure='curious', task_s
                    seed=seed, device=device)
     ddpg_kw['noise_seed'] = rs                      # key of the device-side exploration noise (action_noise='device')
     ddpg_kw.update(policy_kwargs or {})             # this implementation's extras: action_noise, update_schedule, comm, ...
+    if workers_per_rank != 1:
+        ddpg_kw.update(workers_per_rank=workers_per_rank, worker_buffers='own')
     sampler.seed = rs                               # Philox key of the HER draws
     buffer_size = (params['buffer_size'] // params['rollout_batch_size']) * params['rollout_batch_size']    # config.py:204
     buffers = configure_buffer({k: v for k, v in dims.items() if structure != 'flat' or k != 'task_descr'}, T, sampler,
@@ -130,6 +139,12 @@ def make_experiment(nb_tasks=4, n_controllable=None, structure='curious', task_s
             w.seed(rs + i)                                          # train.py:328-329
     else:
         policy = DDPG(buffers=buffers, **ddpg_kw)
+        if workers_per_rank != 1:               # every worker acts, stores and samples on its own stream
+            if not policy._action_rows_ok():
+                raise ValueError('workers_per_rank > 1 acts through the one-launch action kernel, which does not take this '
+                                 'network shape (see cur_ddpg_rows_supported)')
+            explore = dict(explore, workers=workers_per_rank, streams=policy.worker_streams)
+            test = dict(test, workers=workers_per_rank, streams=policy.worker_streams)
         rollout_worker = RolloutWorker(make_env, policy, **explore)
         rollout_worker.seed(rs)                                     # train.py:332
     evaluator = RolloutWorker(make_env, policy, **test)
@@ -220,7 +235,10 @@ class _EpochRecords(object):
         log.dump_tabular()
         rollout_worker.save_goal_task_history(log.get_dir())
         success = mpi_average(self.evaluator.current_success_rate(), comm)
-        assert_rank_streams_differ(comm)                                       # train.py:207-212
+        if getattr(self.evaluator, 'streams', None) is None:
+            assert_rank_streams_differ(comm)                                   # train.py:207-212
+        else:
+            self.evaluator.streams.assert_differ()                             # ... on every virtual worker's stream
         if log.active and self.save_policies:
             if success >= self.best:
                 self.best = success
@@ -245,6 +263,15 @@ def train(policy, rollout_worker, evaluator, n_epochs, n_test_rollouts, n_cycles
     Like the reference, a fresh run starts with one evaluation of the untrained policy, recorded as epoch -1
     (train.py:62-75,125-135; `initial_evaluation=False` skips it), and the evaluator's competence queues run over all epochs
     (`clear_eval_competence=True` restarts them at every evaluation instead)."""
+    hosted = getattr(evaluator, 'streams', None) is not None or getattr(policy, 'worker_buffers', 'shared') == 'own'
+    if hosted:
+        # what the learner refuses for worker_buffers='own' (DDPG), refused before the first rollout instead of mid-run
+        if checkpoint_interval > 0 or resume:
+            raise ValueError('checkpoints do not cover virtual workers (worker_buffers=\'own\')')
+        if structure == 'task_experts' or isinstance(policy, list):
+            raise ValueError("virtual workers do not take structure='task_experts'")
+        if _world(evaluator.comm)[1] > 1:
+            raise ValueError('virtual workers run on one rank')
     history = []
     records = None
     resumed_run = None

@@ -329,6 +329,28 @@ int cur_ddpg_actions_rows_group(void* stream, const cur_net_desc* d, int n_exper
                                 const int32_t* row_expert, const float* o, const float* ag /* or NULL */, const float* g,
                                 const float* td, int64_t n, float clip_obs, void* out_pi, void* out_q /* or NULL */,
                                 uint32_t seq);
+/* cur_ddpg_actions_rows with the device-side exploration noise (cur_action_noise) applied in the same launch, row by row
+ * with the row's own key: rows[i] = {seed, call, ctr, noisy}.  A noisy row i gets exactly the bits that
+ * cur_action_noise(u, m, ..., seed, call) gives row `ctr` of a call over m > ctr rows (the action of a lone agent whose key
+ * is `seed`, at that agent's call number `call`); a row with noisy == 0 gets the noise-free action.  One launch thus
+ * acts for several agents that share a network, e.g. the reference workers one rank hosts (worker j's rows carry its
+ * key, its call number and counter rows 0..B-1).  Q (out_q) is evaluated on the noise-free action, as in
+ * cur_ddpg_actions_rows.  noise_eps == random_eps == 0: the plain launch.  `rows`: n entries readable by the device
+ * (device memory or mapped pinned host memory).  Outputs as cur_ddpg_actions_rows (seq == 0: float32; seq != 0: words).
+ * Refused before any launch: a shape cur_ddpg_rows_supported(d, 4) refuses, dimu > CUR_ACTIONS_MAX_DIMU, n outside
+ * 1..CUR_ACTIONS_NOISY_MAX_ROWS, noise parameters outside noise_eps >= 0, 0 <= random_eps <= 1. */
+#define CUR_ACTIONS_NOISY_MAX_ROWS 512
+#define CUR_ACTIONS_MAX_DIMU 8
+typedef struct cur_noise_row {
+  uint64_t seed;                   /* Philox key (the lone agent's noise seed) */
+  uint64_t call;                   /* that agent's call number */
+  uint32_t ctr;                    /* counter row: the row's index in that agent's call */
+  uint32_t noisy;                  /* 0: no noise on this row */
+} cur_noise_row;
+int cur_ddpg_actions_rows_noisy(void* stream, const cur_net_desc* d, const float* theta, const cur_norm_stats* stats,
+                                const float* o, const float* ag /* or NULL */, const float* g, const float* td, int64_t n,
+                                float clip_obs, double noise_eps, double random_eps, const cur_noise_row* rows,
+                                void* out_pi, void* out_q /* or NULL */, uint32_t seq);
 /* Host-side tail of a seq != 0 call of cur_ddpg_actions_rows (ddpg.py:147-155): polls the n * dimu (+ n with_q) output
  * words in the mapped buffer until all carry `seq`, then applies the reference's exploration post-processing with the
  * caller's np.random draws (randn [n, dimu] float64, explore [n] int64 = binomial(1, random_eps), u_rand [n, dimu] float64 =
